@@ -362,7 +362,9 @@ int pm_host_orientation(const PMOrientationModel *model, double et, double *rmat
  * ulp error on the device.  kind: 0 rcp(a), 1 rsqrt(a), 2 sqrt(a), 3 sin(a) and
  * 4 cos(a) for |a| <= pi/4, 5 atan2(a, b), 6 acos(a), 7 a / b, 8 sin(a), 9 cos(a)
  * for any |a| < 1e5, 10 atan2(|a|, b) and 11 atan2(a, |b|) (the half-plane variants used
- * for vector separations and latitudes).  `b` may be NULL for the one-argument kinds. */
+ * for vector separations and latitudes), 12 sin(a) and 13 cos(a) as the pixel-offset path
+ * evaluates them (a tiny-angle series for |a| <= 2^-8, else as 3 / 4).  `b` may be NULL for the
+ * one-argument kinds. */
 int pm_math_probe(int kind, const double *a, const double *b, int64_t n, double *out,
                   void *stream);
 

@@ -281,7 +281,8 @@ __global__ void __launch_bounds__(256) fp64_probe_kernel(double *out, const doub
 
 // Device self-test of the pm_math.cuh primitives (tests/test_gpu_math.py):
 // kind 0 rcp, 1 rsqrt, 2 sqrt, 3 sin(quarter), 4 cos(quarter), 5 atan2(a, b),
-// 6 acos, 7 div(a, b), 8 sin(full), 9 cos(full), 10 atan2(|a|, b), 11 atan2(a, |b|)
+// 6 acos, 7 div(a, b), 8 sin(full), 9 cos(full), 10 atan2(|a|, b), 11 atan2(a, |b|),
+// 12 sin, 13 cos of the pixel-offset path (sincos_small2: the tiny-angle tier for |a| <= 2^-8)
 __global__ void math_probe_kernel(int kind, const double *__restrict__ a, const double *__restrict__ b,
                                   int64_t n, double *__restrict__ out) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -301,6 +302,8 @@ __global__ void math_probe_kernel(int kind, const double *__restrict__ a, const 
         case 9: sincos_full(x, s, c); r = c; break;
         case 10: r = fast_atan2_ypos(fabs(x), y); break;
         case 11: r = fast_atan2_xpos(x, fabs(y)); break;
+        case 12: sincos_small2(x, 0.0, s, c, r, r); r = s; break;
+        case 13: sincos_small2(x, 0.0, s, c, r, r); r = c; break;
         default: break;
     }
     out[i] = r;

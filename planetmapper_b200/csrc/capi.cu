@@ -288,7 +288,7 @@ int pm_fits_stage(const double *const *src, const int64_t *n_elems, const int64_
 }
 
 int pm_math_probe(int kind, const double *a, const double *b, int64_t n, double *out, void *stream) {
-    if (!a || !out || n < 0 || kind < 0 || kind > 11) return PM_ERR_BAD_ARG;
+    if (!a || !out || n < 0 || kind < 0 || kind > 13) return PM_ERR_BAD_ARG;
     if ((kind == 5 || kind == 7 || kind == 10 || kind == 11) && !b) return PM_ERR_BAD_ARG;
     if (n == 0) return PM_OK;
     return check(launch_math_probe(kind, a, b, n, out, (cudaStream_t)stream));

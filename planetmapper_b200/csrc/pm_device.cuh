@@ -79,6 +79,8 @@ struct FrameD {
     // J2000 vectors of the frame rotated into the body frame at t_ref (R0 v)
     double P0b[3], VTb[3], ATb[3], VOb[3], S0b[3], VSb[3];
     double G[9];       // R0 M^T: radrec(1, -ax, ay) vector -> ray in the body frame at t_ref
+    double y0[3];      // -P0b / radii: the observer at t_ref in the scaled (unit-sphere) space of surfpt
+    double y0m2;       // |y0|^2, associated as surfpt's dot(y, y)
     double As[6];      // xy -> (-ax, ay) in radians: A scaled by rpd / 3600 (first row negated)
     double inv_kmpa;   // 1 / km_per_arcsec
     int biaxial;       // intercept ellipsoid == recpgr spheroid -> closed-form geodetic
@@ -133,6 +135,12 @@ PM_HD void derive_frame_item(FrameD &s, int item) {
         double *dst = item == 3 ? s.P0b : item == 4 ? s.VTb : item == 5 ? s.ATb : item == 6 ? s.VOb : item == 7 ? s.S0b : s.VSb;
         for (int r = 0; r < 3; r++)
             dst[r] = ex_dot3(f.R0[3 * r], src[0], f.R0[3 * r + 1], src[1], f.R0[3 * r + 2], src[2]);
+        if (item == 3) {
+            // the first light-time pass of sincpt starts every pixel's ray at this observer: its scaled
+            // position and |.|^2 with the same roundings as surfpt's mul3(o, inv_r) and dot(y, y)
+            for (int r = 0; r < 3; r++) s.y0[r] = ex_mul(-dst[r], ex_div(1.0, f.radii[r]));
+            s.y0m2 = fma(s.y0[0], s.y0[0], fma(s.y0[1], s.y0[1], ex_mul(s.y0[2], s.y0[2])));
+        }
     } else if (item >= 9 && item <= 11) {
         const int r = item - 9;  // row r of R0 M^T
         for (int c = 0; c < 3; c++)
@@ -206,6 +214,27 @@ inline void load_frame_host(FrameD &s, const PMFrame *g) {
     for (int i = 0; i < kDeriveItems; i++) derive_frame_item(s, i);
 }
 
+// cos^2 (scaled-space emission) below which sincpt iterates to convergence: emission > ~86.9 deg.
+// Above it the fixed-point step's own error (the light time is not linear in the epoch:
+// V^3 de^2 / (2 r c^2 cos^4 e) km) stays below the target motion in one epoch quantum ulp(et) ~ 3e-8 s
+// (V ulp(et) / cos e), which is the resolution of CSPICE's own result.
+#ifndef PM_GRAZING_COS2
+#define PM_GRAZING_COS2 3.0e-3
+#endif
+constexpr double kGrazingCos2 = PM_GRAZING_COS2;
+
+// Per-pixel literals that are not exact in a DADD / DFMA immediate, in pairs used together (one 16-byte
+// constant load each instead of two 32-bit moves per literal); the spin series reads kTinyC (pm_math.cuh)
+enum PixC {
+    kPixDt1Min = 0,   // sincpt: |dt1| above which the two-pass fixed point is used
+    kPixGrazing = 1,  // sincpt: kGrazingCos2
+    kPixInv60 = 2,    // local_solar_time: 1/60, 1/3600
+    kPixInv3600 = 3,
+    kPixRpd = 4,      // local_solar_time: rad per deg
+    kPixBetaMax = 5,  // doppler_factor / radial_velocity: |v| / c bound of the series
+};
+PM_DEV_TABLE(kPixC, 6, 1.0e-6, kGrazingCos2, 1.0 / 60.0, 1.0 / 3600.0, kRpd, 1.0e-3)
+
 // ---------------------------------------------------------------------------------
 // Frame spin: body frame at t_ref  <->  body frame at t_ref + dt
 // ---------------------------------------------------------------------------------
@@ -218,8 +247,8 @@ PM_HD Rot make_rot(const FrameD &fs, double dt) {
     Rot r;
     if (fabs(th) < 0.001953125) {  // 2^-9: series exact to < 1e-20 relative
         const double z = th * th;
-        r.s = th * fma(z, fma(z, 1.0 / 120.0, -1.0 / 6.0), 1.0);
-        r.omc = z * fma(z, fma(z, 1.0 / 720.0, -1.0 / 24.0), 0.5);
+        r.s = th * fma(z, fma(z, PM_T(kTinyC)[0], PM_T(kTinyC)[2]), 1.0);  // 1/120, -1/6
+        r.omc = z * fma(z, fma(z, -PM_T(kTinyC)[1], -PM_T(kTinyC)[3]), 0.5);  // 1/720, -1/24
     } else {
         double sh, ch;
         sincos_lib(0.5 * th, &sh, &ch);
@@ -284,13 +313,13 @@ struct RayHit {
     double t;     // ray parameter of the intercept, t = a - h with the half-chord h = sqrt((1 - |pp|^2) ixx)
     double cos2;  // 1 - |pp|^2: squared half-chord in the unit-sphere space, -> 0 at tangency
 };
-PM_HD bool surfpt(const FrameD &fs, V3 o, V3 u, V3 &p, RayHit &hit) {
+// y: the ray's origin in the scaled (unit-sphere) space, ym2 = |y|^2 (surfpt below, or per frame)
+PM_HD bool surfpt_y(const FrameD &fs, V3 y, double ym2, V3 u, V3 &p, RayHit &hit) {
     // scaled space (unit sphere); the direction x is deliberately NOT normalised: the
     // three dot products are independent and a single reciprocal serves both the
     // projection and the half-chord
     const V3 x = mul3(u, fs.inv_r);
-    const V3 y = mul3(o, fs.inv_r);
-    const double xx = dot(x, x), yx = dot(y, x), ym2 = dot(y, y);
+    const double xx = dot(x, x), yx = dot(y, x);
     if (!(xx > 0.0)) return false;
     const double ixx = fast_rcp(xx);
     const double a = -(yx * ixx);
@@ -315,6 +344,10 @@ PM_HD bool surfpt(const FrameD &fs, V3 o, V3 u, V3 &p, RayHit &hit) {
     p = mul3(axpy(h, x, pp), fs.f.radii);
     return true;
 }
+PM_HD bool surfpt(const FrameD &fs, V3 o, V3 u, V3 &p, RayHit &hit) {
+    const V3 y = mul3(o, fs.inv_r);
+    return surfpt_y(fs, y, dot(y, y), u, p, hit);
+}
 
 // Result of the converged intercept, everything in the body frame at the intercept
 // epoch t_ref + dt unless stated.
@@ -327,15 +360,6 @@ struct Intercept {
     double L;    // observer -> point range (km)
     double lt;   // L / c
 };
-
-// cos^2 (scaled-space emission) below which sincpt iterates to convergence: emission > ~86.9 deg.
-// Above it the fixed-point step's own error (the light time is not linear in the epoch:
-// V^3 de^2 / (2 r c^2 cos^4 e) km) stays below the target motion in one epoch quantum ulp(et) ~ 3e-8 s
-// (V ulp(et) / cos e), which is the resolution of CSPICE's own result.
-#ifndef PM_GRAZING_COS2
-#define PM_GRAZING_COS2 3.0e-3
-#endif
-constexpr double kGrazingCos2 = PM_GRAZING_COS2;
 
 // Slow path of sincpt for grazing rays and for frames whose first two passes coincide in
 // epoch: CSPICE's loop as written - full intercepts until the FP64 epoch et - lt stops
@@ -376,7 +400,7 @@ PM_HD bool sincpt(const FrameD &fs, V3 u0, Intercept &it) {
     const PMFrame &f = fs.f;
     V3 p1, p2;
     RayHit h1, h2;
-    if (!surfpt(fs, -ld3(fs.P0b), u0, p1, h1)) return false;
+    if (!surfpt_y(fs, ld3(fs.y0), fs.y0m2, u0, p1, h1)) return false;  // observer at t_ref: -P0b
     const double lt1 = h1.t * fs.inv_c;  // u0 is a unit vector: the ray parameter is the range
 
     const double dt1 = (f.et - lt1) - f.t_ref;
@@ -389,7 +413,7 @@ PM_HD bool sincpt(const FrameD &fs, V3 u0, Intercept &it) {
     double dt = (f.et - lt2) - f.t_ref;
     V3 p;
     double L;
-    if (fabs(dt1) > 1.0e-6 && h2.cos2 > kGrazingCos2) {
+    if (fabs(dt1) > PM_T(kPixC)[kPixDt1Min] && h2.cos2 > PM_T(kPixC)[kPixGrazing]) {
         // The epochs e_0 = t_ref, e_1, e_2 of CSPICE's loop contract geometrically (ratio (e_2 - e_1) /
         // (e_1 - e_0)); the loop's fixed point is e_1 + lam (e_1 - e_0), lam = (e_2 - e_1) / (e_1 - e_2 + e_1 - e_0).
         // The intercept there comes from the two solves without a third one: the foot pp of the
@@ -438,7 +462,7 @@ PM_HD void geodetic_general(const FrameD &fs, double rho, double z, double &lat,
     }
     // reduced latitude beta: tan(beta) = re z / (rp rho)
     double sb = f.re * z, cb = fs.rp * rho;
-    double n = fast_rsqrt(fma(sb, sb, cb * cb) + 1.0e-300);
+    double n = fast_rsqrt(fma(sb, sb, cb * cb) + sqrt_guard());
     sb *= n;
     cb *= n;
     double num = z, den = rho;
@@ -447,7 +471,7 @@ PM_HD void geodetic_general(const FrameD &fs, double rho, double z, double &lat,
         num = fma(fs.ep2 * fs.rp, sb * sb * sb, z);
         den = fma(-fs.e2 * f.re, cb * cb * cb, rho);
         double nsb = fs.omf * num, ncb = den;
-        n = fast_rsqrt(fma(nsb, nsb, ncb * ncb) + 1.0e-300);
+        n = fast_rsqrt(fma(nsb, nsb, ncb * ncb) + sqrt_guard());
         nsb *= n;
         ncb *= n;
         const double change = fabs(nsb - sb) + fabs(ncb - cb);
@@ -456,7 +480,7 @@ PM_HD void geodetic_general(const FrameD &fs, double rho, double z, double &lat,
         if (change <= 4.0e-16) break;
     }
     lat = fast_atan2(num, den);
-    n = fast_rsqrt(fma(num, num, den * den) + 1.0e-300);
+    n = fast_rsqrt(fma(num, num, den * den) + sqrt_guard());
     const double sp = num * n, cp = den * n;
     alt = fma(rho, cp, z * sp) - f.re * fast_sqrt(fma(-fs.e2 * sp, sp, 1.0));
 }
@@ -469,7 +493,7 @@ PM_HD double geodetic_lat_spheroid(double re, double rp, double rho, double z) {
     const double q = fast_div(rp, re), qi = fast_div(re, rp);
     const double e2 = fma(-q, q, 1.0), ep2 = fma(qi, qi, -1.0);
     double sb = re * z, cb = rp * rho;
-    double n = fast_rsqrt(fma(sb, sb, cb * cb) + 1.0e-300);
+    double n = fast_rsqrt(fma(sb, sb, cb * cb) + sqrt_guard());
     sb *= n;
     cb *= n;
     double num = z, den = rho;
@@ -478,7 +502,7 @@ PM_HD double geodetic_lat_spheroid(double re, double rp, double rho, double z) {
         num = fma(ep2 * rp, sb * sb * sb, z);
         den = fma(-e2 * re, cb * cb * cb, rho);
         double nsb = q * num, ncb = den;
-        n = fast_rsqrt(fma(nsb, nsb, ncb * ncb) + 1.0e-300);
+        n = fast_rsqrt(fma(nsb, nsb, ncb * ncb) + sqrt_guard());
         nsb *= n;
         ncb *= n;
         const double change = fabs(nsb - sb) + fabs(ncb - cb);
@@ -511,7 +535,7 @@ PM_HD V3 pgrrec0(const FrameD &fs, double lon, double lat) {
     sincos_full(lat, slat, clat);
     sincos_full(f.lon_sign * lon, slon, clon);
     const double x = f.re * clat, y = fs.rp * slat;
-    const double scale = fast_rsqrt(fma(x, x, y * y) + 1.0e-300);
+    const double scale = fast_rsqrt(fma(x, x, y * y) + sqrt_guard());
     return mk(scale * clon * x * f.re, scale * slon * x * f.re, scale * y * fs.rp);
 }
 
@@ -525,7 +549,7 @@ PM_HD void reclat_angles(V3 v, double &lon, double &lat) {
 // lon_deg finite.  Whole seconds are split with integer arithmetic; the two divisions
 // of the reference's `hr + mn / 60 + sc / 3600` are reproduced correctly rounded.
 PM_HD double local_solar_time(const PMFrame &f, double lon_deg) {
-    double ang = f.lon_sign * (lon_deg * kRpd) - f.sun_lon_lst;
+    double ang = f.lon_sign * (lon_deg * PM_T(kPixC)[kPixRpd]) - f.sun_lon_lst;
     if (f.prograde == 0.0) ang = -ang;
     // fmod(ang, 2 pi) folded into [0, 2 pi): ang - k 2pi is exact for the small k here
     const double k = floor(ang * PM_T(kMisc)[8]);
@@ -539,10 +563,10 @@ PM_HD double local_solar_time(const PMFrame &f, double lon_deg) {
     const int mn = rem / 60, sc = rem - mn * 60;
     // correctly rounded mn / 60 and sc / 3600 (Markstein: r = RN(1/b), one FMA correction)
     const double dm = (double)mn, ds = (double)sc;
-    double qm = dm * (1.0 / 60.0);
-    qm = fma(fma(-60.0, qm, dm), 1.0 / 60.0, qm);
-    double qs = ds * (1.0 / 3600.0);
-    qs = fma(fma(-3600.0, qs, ds), 1.0 / 3600.0, qs);
+    double qm = dm * PM_T(kPixC)[kPixInv60];
+    qm = fma(fma(-60.0, qm, dm), PM_T(kPixC)[kPixInv60], qm);
+    double qs = ds * PM_T(kPixC)[kPixInv3600];
+    qs = fma(fma(-3600.0, qs, ds), PM_T(kPixC)[kPixInv3600], qs);
     return ((double)hr + qm) + qs;
 }
 
@@ -555,7 +579,7 @@ PM_HD double doppler_factor(const FrameD &fs, double rv) {
     // sqrt((1 + b) / (1 - b)) = (1 + b) (1 - b^2)^(-1/2) = 1 + b + b^2/2 + b^3/2 + 3 b^4/8 + 3 b^5/8 + 5 b^6/16 + ...
     // For |b| < 1e-3 (300 km/s; solar-system radial velocities are < 1e-4 c) the first omitted term is
     // < 3.2e-19: the sum is within one ulp of the correctly rounded quotient and root, without either.
-    if (fabs(beta) < 1.0e-3)
+    if (fabs(beta) < PM_T(kPixC)[kPixBetaMax])
         return fma(beta, fma(beta, fma(beta, fma(beta, fma(beta, 0.375, 0.375), 0.5), 0.5), 1.0), 1.0);
     return doppler_factor_closed(beta);
 }
@@ -568,7 +592,7 @@ PM_HD double radial_velocity(const FrameD &fs, double a, double b) {
     // of the correction for |a| < 300 km/s)
     const double ac = a * fs.inv_c;
     double dlt = (a - b) * fs.inv_c * fma(ac, ac - 1.0, 1.0);
-    if (!(fabs(ac) < 1.0e-3)) dlt = light_time_rate_closed(a, b, fs.f.clight);
+    if (!(fabs(ac) < PM_T(kPixC)[kPixBetaMax])) dlt = light_time_rate_closed(a, b, fs.f.clight);
     return fma(-dlt, a, a) - b;
 }
 
@@ -586,10 +610,13 @@ PM_HD void illum_angles(V3 n, V3 s, V3 e, bool want_az, Illum &out) {
     out.incdnc = fast_atan2_ypos(mns, dns);
     out.emissn = fast_atan2_ypos(mne, dne);
     if (want_az) {
-        // (cos g - cos e cos i) / (sin e sin i) with the common factor |n|^2 |s| |e|
-        // cancelled: ((s.e)(n.n) - (n.e)(n.s)) / (|n x e| |n x s|)
-        const double a = fma(dse, dot(n, n), -dne * dns);
-        out.azimuth = kPi - fast_acos(fast_div_lite(a, mne * mns));
+        // pi - acos of (cos g - cos e cos i) / (sin e sin i), i.e. of the cosine of the angle between
+        // n x e and n x s, written as the atan2 of that angle's sine and cosine: by Lagrange's identity
+        // (n x e).(n x s) = (s.e)(n.n) - (n.e)(n.s) and |(n x e) x (n x s)| = |n| |n.(s x e)|.  No division
+        // or acos, and well conditioned where sin e or sin i -> 0 (acos of a 0 / 0 quotient there)
+        const double nn = dot(n, n);
+        const double a = fma(dse, nn, -dne * dns);
+        out.azimuth = fast_atan2_ypos(fast_sqrt_pos(nn) * fabs(dot(n, cse)), -a);  // pi - atan2(y, a)
     }
 }
 
@@ -608,7 +635,7 @@ PM_HD void illum_at(const FrameD &fs, V3 p, V3 p0 /* spin_bwd(p) */, V3 e, Rot r
                        fs.S0b[2] - fma(fs.ATb[2], h, fma(fs.VTb[2], dt, p0.z)));
     const V3 VSb = ld3(fs.VSb);
     V3 sv = axpy(dt, VSb, base);
-    const double lts = norm(sv) * fs.inv_c;
+    const double lts = fast_sqrt_pos(dot(sv, sv)) * fs.inv_c;  // the Sun is never at the point
     sv = axpy(dt - (lts - f.lts0), VSb, base);
     const V3 s_b = spin_fwd(fs, r, sv);
     const V3 n = mul3(p, fs.nw);  // spice.surfnm direction

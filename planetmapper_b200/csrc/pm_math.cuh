@@ -32,7 +32,7 @@
 #define PM_HD __host__ __device__ __forceinline__
 #define PM_HD_NOINLINE static __host__ __device__ __noinline__
 #define PM_DEV_TABLE(name, n, ...)                        \
-    static __constant__ double name##_dev[n] = {__VA_ARGS__}; \
+    static __constant__ __align__(16) double name##_dev[n] = {__VA_ARGS__}; \
     static const double name##_host[n] = {__VA_ARGS__};
 #else
 #define PM_HD inline
@@ -67,11 +67,15 @@ PM_DEV_TABLE(kSinC, 6, -0.16666666666666664621, 0.008333333333330946103, -0.0001
 PM_DEV_TABLE(kCosC, 6, 0.041666666666666665387, -0.0013888888888887395746, 0.000024801587298763433277,
              -2.7557317270560382548e-7, 2.0876146024701932874e-9, -1.1382614869434128293e-11)
 // misc constants read as constant-bank operands: tan(pi/12), pi/4, pi/2, pi, 2/pi,
-// pi/2 split (hi, lo), 2 pi, 1/(2 pi), sqrt(3), pi/6
-PM_DEV_TABLE(kMisc, 11, 0.2679491924311227064725537, 0.78539816339744830961566, 1.5707963267948966192313,
+// pi/2 split (hi, lo), 2 pi, 1/(2 pi), sqrt(3), pi/6, the zero guard of the square roots
+PM_DEV_TABLE(kMisc, 12, 0.2679491924311227064725537, 0.78539816339744830961566, 1.5707963267948966192313,
              3.1415926535897932384626, 0.6366197723675813430755351, 1.570796326794896619231322,
              6.12323399573676588613033e-17, 6.283185307179586476925287, 0.1591549430918953357688838,
-             1.732050807568877293527446, 0.5235987755982988730771072)
+             1.732050807568877293527446, 0.5235987755982988730771072, 1.0e-300)
+
+// x + sqrt_guard() keeps an rsqrt seed finite at x == 0 (1e-300, read from the table like the other
+// full-mantissa literals instead of being rebuilt by two 32-bit moves at every use)
+PM_HD double sqrt_guard() { return PM_T(kMisc)[11]; }
 
 // ---- MUFU seeds ----------------------------------------------------------------
 PM_HD double rcp_seed(double b) {
@@ -135,14 +139,16 @@ PM_HD double fast_rsqrt(double x) {
 }
 // sqrt(x) for x >= 0 (x == 0 -> 0).  Not for negative x (see fast_sqrt_nan).
 PM_HD double fast_sqrt(double x) {
-    double y = fast_rsqrt(x + 1.0e-300);  // keeps the seed finite at x == 0
+    double y = fast_rsqrt(x + sqrt_guard());
     double s = x * y;
     double rem = fma(-s, s, x);
     return fma(rem, 0.5 * y, s);
 }
 // Two-instruction-cheaper variants (<= 1.5 ulp instead of <= 0.5) for values that feed light
 // times, angle arguments and normalisations, where the last half ulp is immaterial
-PM_HD double fast_sqrt_lite(double x) { return x * fast_rsqrt(x + 1.0e-300); }
+PM_HD double fast_sqrt_lite(double x) { return x * fast_rsqrt(x + sqrt_guard()); }
+// ... for x known to be finite, normal and > 0 (lengths of vectors that cannot vanish): no zero guard
+PM_HD double fast_sqrt_pos(double x) { return x * fast_rsqrt(x); }
 PM_HD double fast_div_lite(double a, double b) { return a * fast_rcp(b); }
 // sqrt that keeps IEEE's NaN for negative input
 PM_HD double fast_sqrt_nan(double x) { return (x < 0.0) ? NAN : fast_sqrt_lite(x); }
@@ -178,10 +184,24 @@ PM_HD void sincos_small(double x, double &s, double &c) {
         sincos_lib(x, &s, &c);
     }
 }
+// sin, cos for |x| <= 2^-8: x + x z (-1/6 + z/120), 1 - z/2 + z^2 (1/24 - z/720); the first omitted terms
+// are < 1e-18 relative.  Pixel offsets from the optical axis of a telescope image (an arcminute field is
+// 3e-4 rad) stay far inside this range.
+// [0] 1/120, [1] -1/720, [2] -1/6, [3] 1/24 (also the spin series of pm_device.cuh's make_rot)
+PM_DEV_TABLE(kTinyC, 4, 1.0 / 120.0, -1.0 / 720.0, -1.0 / 6.0, 1.0 / 24.0)
+PM_HD void sincos_tiny(double x, double &s, double &c) {
+    const double z = x * x;
+    s = fma(x * z, fma(z, PM_T(kTinyC)[0], PM_T(kTinyC)[2]), x);
+    c = fma(z * z, fma(z, PM_T(kTinyC)[1], PM_T(kTinyC)[3]), fma(-0.5, z, 1.0));
+}
 // sin, cos of two small angles with ONE range test, so that the four polynomial
 // chains share a basic block (cold library fallback for anything above pi/4)
 PM_HD void sincos_small2(double a, double b, double &sa, double &ca, double &sb, double &cb) {
-    if (fmax(fabs(a), fabs(b)) <= PM_T(kMisc)[1]) {
+    const double m = fmax(fabs(a), fabs(b));
+    if (m <= 0.00390625) {  // 2^-8
+        sincos_tiny(a, sa, ca);
+        sincos_tiny(b, sb, cb);
+    } else if (m <= PM_T(kMisc)[1]) {
         sincos_quarter(a, sa, ca);
         sincos_quarter(b, sb, cb);
     } else {
@@ -215,11 +235,11 @@ PM_HD void sincos_full(double x, double &s, double &c) {
 }
 
 // Bit-level helpers: keep sign / magnitude bookkeeping off the FP64 pipe
-PM_HD bool abs_gt(double a, double b) {  // |a| > |b| for non-NaN inputs (IEEE ordering == integer ordering)
+PM_HD bool pos_gt(double a, double b) {  // a > b for non-NaN a, b >= 0 (IEEE ordering == integer ordering)
 #ifdef __CUDA_ARCH__
-    return (__double_as_longlong(a) & 0x7fffffffffffffffll) > (__double_as_longlong(b) & 0x7fffffffffffffffll);
+    return __double_as_longlong(a) > __double_as_longlong(b);
 #else
-    return fabs(a) > fabs(b);
+    return a > b;
 #endif
 }
 PM_HD double with_sign_of(double r, double y) {  // r >= 0: copysign(r, y)
@@ -228,6 +248,13 @@ PM_HD double with_sign_of(double r, double y) {  // r >= 0: copysign(r, y)
     return __hiloint2double(hi, __double2loint(r));
 #else
     return copysign(r, y);
+#endif
+}
+PM_HD double abs_bits(double x) {  // fabs(x) as one integer AND of the high word instead of an FP64 DADD
+#ifdef __CUDA_ARCH__
+    return __hiloint2double(__double2hiint(x) & 0x7fffffff, __double2loint(x));
+#else
+    return fabs(x);
 #endif
 }
 PM_HD bool sign_bit(double x) {
@@ -258,8 +285,8 @@ PM_HD double atan_ratio(double mn, double mx) {
 // atan2(y, x), full quadrant, atan2(0, 0) = 0 (the convention recrad / reclat / recgeo
 // apply explicitly).  NaN in -> NaN out.
 PM_HD double fast_atan2(double y, double x) {
-    const double ax = fabs(x), ay = fabs(y);
-    const bool sw = abs_gt(y, x);
+    const double ax = abs_bits(x), ay = abs_bits(y);
+    const bool sw = pos_gt(ay, ax);
     const double mx = sw ? ay : ax, mn = sw ? ax : ay;
     double r = atan_ratio(mn, mx);  // 0 / 0 -> NaN, replaced below
     if (sw) r = PM_T(kMisc)[2] - r;
@@ -269,8 +296,8 @@ PM_HD double fast_atan2(double y, double x) {
 }
 // atan2(y, x) for y >= 0 and (x, y) != (0, 0): angle in [0, pi] (vector separations)
 PM_HD double fast_atan2_ypos(double y, double x) {
-    const double ax = fabs(x);
-    const bool sw = abs_gt(y, x);
+    const double ax = abs_bits(x);
+    const bool sw = pos_gt(abs_bits(y), ax);
     const double mx = sw ? y : ax, mn = sw ? ax : y;
     double r = atan_ratio(mn, mx);
     if (sw) r = PM_T(kMisc)[2] - r;
@@ -279,8 +306,8 @@ PM_HD double fast_atan2_ypos(double y, double x) {
 }
 // atan2(y, x) for x >= 0 and (x, y) != (0, 0): angle in [-pi/2, pi/2] (latitudes)
 PM_HD double fast_atan2_xpos(double y, double x) {
-    const double ay = fabs(y);
-    const bool sw = abs_gt(y, x);
+    const double ay = abs_bits(y);
+    const bool sw = pos_gt(ay, abs_bits(x));
     const double mx = sw ? ay : x, mn = sw ? x : ay;
     double r = atan_ratio(mn, mx);
     if (sw) r = PM_T(kMisc)[2] - r;
