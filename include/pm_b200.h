@@ -111,6 +111,7 @@ enum PMPlane {
 #define PM_FLAG_NOT_VISIBLE_NAN 1u /* lonlat2xy(not_visible_nan=True)               */
 #define PM_FLAG_PROPAGATE_NAN 2u   /* map_img(propagate_nan=True)                   */
 #define PM_FLAG_PLANETOCENTRIC 4u   /* lonlat2xy(planetocentric=True) inputs         */
+#define PM_FLAG_RING_ALL 8u         /* ring_plane_coordinates(only_visible=False)    */
 
 /* coordinate systems of pm_transform (the five systems of Body / BodyXY, planetmapper/body.py:1083-1900,
  * planetmapper/body_xy.py:385-676; CENTRIC = planetocentric lon / lat as a destination) */
@@ -146,6 +147,17 @@ int pm_backplanes_img(const PMFrame *frames, int n_frames, int nx, int ny,
  * `out` is a DEVICE pointer: [popcount(mask)][ny][nx]. */
 int pm_backplanes_img_host(const PMFrame *frame_host, int nx, int ny, uint64_t plane_mask,
                            double *out, void *stream);
+/* Image-direction backplanes at n arbitrary image positions (x[i], y[i]) - fractional, outside the
+ * image, in any order - of ONE frame given in HOST memory (constants as a kernel parameter, like
+ * pm_backplanes_img_host): the per-point geometry queries of Body (illumination / limb / ring-plane
+ * coordinates at a direction, planetmapper/body.py:2081-2110, :2577-2615).  `x`, `y`, `out` are
+ * DEVICE pointers; out: [popcount(mask)][n].  At integer (x, y) every plane equals
+ * pm_backplanes_img_host's pixel bit for bit.  A point whose x or y is not finite gets NaN in every
+ * plane but PIXEL-X / PIXEL-Y, which echo the input.  flags: 0 or PM_FLAG_RING_ALL = ring-plane
+ * coordinates without the "hidden behind the body" test (Body.ring_plane_coordinates with
+ * only_visible=False).  n = 0 is valid with NULL pointers. */
+int pm_backplanes_points_host(const PMFrame *frame_host, const double *x, const double *y, int64_t n,
+                              uint64_t plane_mask, uint32_t flags, double *out, void *stream);
 
 /*
  * Map-direction backplanes on arbitrary lon/lat cells (degrees, planetographic):

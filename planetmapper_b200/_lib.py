@@ -25,6 +25,7 @@ PROJ_ORTHOGRAPHIC, PROJ_AZIMUTHAL, PROJ_AZIMUTHAL_EQUAL_AREA = 1, 2, 3
 FLAG_NOT_VISIBLE_NAN = 1
 FLAG_PROPAGATE_NAN = 2
 FLAG_PLANETOCENTRIC = 4
+FLAG_RING_ALL = 8
 
 PLANE_NAMES = [
     'LON-GRAPHIC', 'LAT-GRAPHIC', 'LON-CENTRIC', 'LAT-CENTRIC', 'RA', 'DEC', 'PIXEL-X',
@@ -44,6 +45,7 @@ EXPORTED_SYMBOLS = [
     'pm_nan_minmax', 'pm_pchip_work_bytes', 'pm_pchip_resample', 'pm_gather_grid_linear',
     'pm_fits_data_unit_bytes', 'pm_fits_stage', 'pm_backplanes_map_batch', 'pm_gather_paired',
     'pm_host_ssb_state', 'pm_host_orientation', 'pm_backplanes_img_host', 'pm_transform', 'pm_fp64_probe', 'pm_proj_forward',
+    'pm_backplanes_points_host',
 ]
 
 
@@ -76,6 +78,8 @@ def load_library() -> ctypes.CDLL:
     lib.pm_backplanes_map_host.argtypes = [c_p, c_p, c_p, c_i64, c_u64, c_p, c_p]
     lib.pm_backplanes_img_host.argtypes = [c_p, c_i, c_i, c_u64, c_p, c_p]
     lib.pm_backplanes_img_host.restype = c_i
+    lib.pm_backplanes_points_host.argtypes = [c_p, c_p, c_p, c_i64, c_u64, c_u32, c_p, c_p]
+    lib.pm_backplanes_points_host.restype = c_i
     lib.pm_transform.argtypes = [c_p, c_i, c_i, c_p, c_p, c_i64, ctypes.c_double, c_u32, c_p, c_p, c_p, c_p, c_p]
     lib.pm_transform.restype = c_i
     lib.pm_xy2lonlat.argtypes = [c_p, c_p, c_p, c_i64, c_p, c_p, c_p, c_p]
@@ -311,6 +315,26 @@ def backplanes_map_host(frame_host, lon_dev, lat_dev, mask: int = ALL_PLANES, ou
     rc = lib.pm_backplanes_map_host(fr.ctypes.data_as(ctypes.c_void_p), lon_dev.data_ptr(), lat_dev.data_ptr(),
                                     lon_dev.numel(), mask, out.data_ptr(), _stream_ptr(torch))
     _check(rc, 'pm_backplanes_map_host')
+    return out
+
+
+def backplanes_points_host(frame_host, x_dev, y_dev, mask: int = ALL_PLANES, *, ring_all: bool = False, out=None):
+    """Image-direction planes at arbitrary (fractional, out-of-image) positions ``(x_dev, y_dev)`` of one frame whose
+    92 constants are a HOST float64 array (pm_backplanes_points_host).  ``ring_all``: ring-plane coordinates
+    without the hidden-behind-the-body test.  Returns a CUDA tensor (popcount(mask),) + x_dev.shape."""
+    torch = _torch()
+    lib = load_library()
+    fr = np.ascontiguousarray(frame_host, dtype=np.float64).reshape(-1)
+    if fr.size != 92:
+        raise ValueError('frame_host must hold the 92 PMFrame doubles')
+    assert x_dev.is_cuda and y_dev.is_cuda and x_dev.is_contiguous() and y_dev.is_contiguous()
+    assert x_dev.dtype == torch.float64 and y_dev.dtype == torch.float64 and x_dev.shape == y_dev.shape
+    if out is None:
+        out = torch.empty((popcount(mask),) + tuple(x_dev.shape), dtype=torch.float64, device=x_dev.device)
+    rc = lib.pm_backplanes_points_host(fr.ctypes.data_as(ctypes.c_void_p), x_dev.data_ptr(), y_dev.data_ptr(),
+                                       x_dev.numel(), mask, FLAG_RING_ALL if ring_all else 0, out.data_ptr(),
+                                       _stream_ptr(torch))
+    _check(rc, 'pm_backplanes_points_host')
     return out
 
 

@@ -613,6 +613,112 @@ class BodyXY(ProgressMixin):
         alt = self._check_alt(alt)
         return self._transform('lonlat', 'lonlat', lon_centric, lat_centric, alt=alt, planetocentric=True)
 
+    # ---- per-point geometry (body.py:2081-2110, :2152-2615) ------------------------------
+    # Vectorised forms of the reference's scalar queries: scalars give floats, arrays give float64
+    # arrays of the broadcast shape, and each call is a fixed number of launches whatever the number of
+    # points.  Nothing here is cached (the reference caches none of them) and no image size is needed.
+    @staticmethod
+    def _refuse_point_alt(alt) -> None:
+        if float(alt) != 0.0:
+            # the reference's meaning of a point above the ellipsoid (illumf's normal, spkcpt at an
+            # off-surface point) is not pinned by any test here: refuse rather than guess
+            raise NotImplementedError('alt != 0 is not supported by the lon / lat point methods')
+
+    def _lonlat_point_planes(self, lon, lat, names):
+        """The map-direction planes ``names`` at the cells (lon, lat): one pm_backplanes_map_host launch, the
+        values get_backplane_map gives for those cells."""
+        scalar, lo, la = self._broadcast(lon, lat)
+        mask = L.mask_from_names(names)
+        planes = L.to_host(L.backplanes_map_host(self._frame_host(), L.to_device(lo), L.to_device(la), mask))
+        return scalar, [planes[L.popcount(mask & ((1 << L.PLANE_ID[n]) - 1))] for n in names]
+
+    def _radec_point_planes(self, ra, dec, names, *, ring_all: bool = False):
+        """The image-direction planes ``names`` along the directions (ra, dec): pm_transform radec -> xy, then
+        pm_backplanes_points_host at those (fractional) pixel positions - two launches."""
+        scalar, a, b = self._broadcast(ra, dec)
+        mask = L.mask_from_names(names)
+        x, y, _ = L.transform(self._frame_dev(), 'radec', 'xy', L.to_device(a), L.to_device(b))
+        planes = L.to_host(L.backplanes_points_host(self._frame_host(), x, y, mask, ring_all=ring_all))
+        return scalar, [planes[L.popcount(mask & ((1 << L.PLANE_ID[n]) - 1))] for n in names]
+
+    @staticmethod
+    def _point_result(scalar, arrays):
+        if scalar:
+            values = tuple(float(a.reshape(())) for a in arrays)
+        else:
+            values = tuple(arrays)
+        return values if len(values) > 1 else values[0]
+
+    def illumination_angles_from_lonlat(self, lon, lat, *, alt: float = 0.0):
+        """Body.illumination_angles_from_lonlat: (phase, incidence, emission) in degrees at a surface point;
+        angles of points on the far side are returned too (emission > 90)."""
+        self._refuse_point_alt(alt)
+        scalar, planes = self._lonlat_point_planes(lon, lat, ['PHASE', 'INCIDENCE', 'EMISSION'])
+        return self._point_result(scalar, planes)
+
+    def azimuth_angle_from_lonlat(self, lon, lat, *, alt: float = 0.0):
+        """Body.azimuth_angle_from_lonlat: azimuth angle in degrees at a surface point."""
+        self._refuse_point_alt(alt)
+        scalar, planes = self._lonlat_point_planes(lon, lat, ['AZIMUTH'])
+        return self._point_result(scalar, planes)
+
+    def local_solar_time_from_lon(self, lon):
+        """Body.local_solar_time_from_lon: local solar time in decimal local hours (et2lst's whole seconds)."""
+        scalar, planes = self._lonlat_point_planes(lon, 0.0, ['LOCAL-SOLAR-TIME'])
+        return self._point_result(scalar, planes)
+
+    @staticmethod
+    def _lst_string(hours) -> str:
+        if not math.isfinite(hours):
+            return 'nan'
+        total = round(hours * 3600)   # the decimal hours are h + m / 60 + s / 3600 of et2lst's integers
+        return '%02d:%02d:%02d' % (total // 3600, (total % 3600) // 60, total % 60)
+
+    def local_solar_time_string_from_lon(self, lon):
+        """Body.local_solar_time_string_from_lon: local solar time as 'HH:MM:SS' (an array of '<U8' strings for
+        array input; 'nan' where lon is not finite)."""
+        hours = self.local_solar_time_from_lon(lon)
+        if np.ndim(hours) == 0:
+            return self._lst_string(float(hours))
+        out = np.empty(np.shape(hours), dtype='<U8')
+        flat = out.reshape(-1)
+        for i, h in enumerate(np.asarray(hours).reshape(-1).tolist()):
+            flat[i] = self._lst_string(h)
+        return out
+
+    def distance_from_lonlat(self, lon, lat, *, alt: float = 0.0):
+        """Body.distance_from_lonlat: distance from the observer to a surface point, km."""
+        self._refuse_point_alt(alt)
+        scalar, planes = self._lonlat_point_planes(lon, lat, ['DISTANCE'])
+        return self._point_result(scalar, planes)
+
+    def radial_velocity_from_lonlat(self, lon, lat, *, alt: float = 0.0):
+        """Body.radial_velocity_from_lonlat: radial velocity of a surface point away from the observer, km/s."""
+        self._refuse_point_alt(alt)
+        scalar, planes = self._lonlat_point_planes(lon, lat, ['RADIAL-VELOCITY'])
+        return self._point_result(scalar, planes)
+
+    def test_if_lonlat_visible(self, lon, lat, alt: float = 0.0):
+        """Body.test_if_lonlat_visible: True where the point (at altitude ``alt`` above the surface) faces the
+        observer and nothing of the body hides it; a bool array for array input."""
+        ra, dec = self.lonlat2radec(lon, lat, alt=alt, not_visible_nan=True)
+        visible = np.isfinite(ra) & np.isfinite(dec)
+        return bool(visible) if np.ndim(visible) == 0 else visible
+
+    def limb_coordinates_from_radec(self, ra, dec):
+        """Body.limb_coordinates_from_radec: (lon, lat, distance) of the limb point nearest to the direction
+        (ra, dec); distance is km above the limb (negative inside the disc)."""
+        scalar, planes = self._radec_point_planes(ra, dec, ['LIMB-LON-GRAPHIC', 'LIMB-LAT-GRAPHIC', 'LIMB-DISTANCE'])
+        return self._point_result(scalar, planes)
+
+    def ring_plane_coordinates(self, ra, dec, only_visible: bool = True):
+        """Body.ring_plane_coordinates: (radius km, planetographic longitude deg, distance km) where the direction
+        (ra, dec) meets the equatorial (ring) plane; NaN where it does not, and with ``only_visible`` also where
+        the body hides that point."""
+        scalar, planes = self._radec_point_planes(ra, dec, ['RING-RADIUS', 'RING-LON-GRAPHIC', 'RING-DISTANCE'],
+                                                  ring_all=not only_visible)
+        return self._point_result(scalar, planes)
+
     # ---- projections (body_xy.py:2755-3012) -------------------------------------------
     def generate_map_coordinates(self, projection: str = 'rectangular', *,
                                  degree_interval: float = 1, lon: float = 0, lat: float = 0,

@@ -113,6 +113,27 @@ __global__ void __launch_bounds__(kBlock, kImgParamCtas) backplanes_img_param_ke
 }
 
 // ---------------------------------------------------------------------------------
+// Image direction at arbitrary positions (pm_backplanes_points_host): the per-pixel code of the
+// single-frame image kernel on a list of (x, y), tiled like map_tile; output plane stride = n
+// ---------------------------------------------------------------------------------
+template <bool kSky, bool kRingAll>
+__global__ void __launch_bounds__(kBlock, 4) backplanes_points_param_kernel(const __grid_constant__ FrameD fs,
+                                                                            const double *__restrict__ x_in,
+                                                                            const double *__restrict__ y_in,
+                                                                            int64_t n, uint64_t mask,
+                                                                            const __grid_constant__ PlaneOffsets po,
+                                                                            double *__restrict__ out) {
+    const int64_t first = (int64_t)blockIdx.x * (kBlock * kPerThread) + threadIdx.x;
+#pragma unroll 1
+    for (int r = 0; r < kPerThread; r++) {
+        const int64_t idx = first + r * kBlock;
+        if (idx >= n) break;
+        PlaneSink sink{reinterpret_cast<char *>(out + idx), po};
+        image_point<kSky, kRingAll>(fs, __ldg(x_in + idx), __ldg(y_in + idx), mask, sink);
+    }
+}
+
+// ---------------------------------------------------------------------------------
 // Map direction
 // ---------------------------------------------------------------------------------
 // x_map / y_map of BodyXY.map_img (body_xy.py:3482): the plane set of every reprojection
@@ -382,6 +403,23 @@ cudaError_t launch_backplanes_img_host(const PMFrame *frame_host, int nx, int ny
     else
         backplanes_img_param_kernel<false, 0><<<grid, kBlock, 0, st>>>(fs, (uint32_t)nx, (uint32_t)npx, per, centre, mask,
                                                                         po, out);
+    count_launches(1);
+    return cudaGetLastError();
+}
+// n arbitrary image positions of ONE frame given on the HOST (constants derived here, as above)
+cudaError_t launch_backplanes_points_host(const PMFrame *frame_host, const double *x, const double *y, int64_t n,
+                                          uint64_t mask, uint32_t flags, double *out, cudaStream_t st) {
+    FrameD fs;
+    load_frame_host(fs, frame_host);
+    const PlaneOffsets po = make_plane_offsets(mask, n);
+    const unsigned grid = chunks_for(n);
+    // the ring planes are sky planes: without a sky plane PM_FLAG_RING_ALL has nothing to change
+    if (!(mask & kSkyMask))
+        backplanes_points_param_kernel<false, false><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
+    else if (flags & PM_FLAG_RING_ALL)
+        backplanes_points_param_kernel<true, true><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
+    else
+        backplanes_points_param_kernel<true, false><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
     count_launches(1);
     return cudaGetLastError();
 }

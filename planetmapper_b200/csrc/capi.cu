@@ -64,6 +64,17 @@ int pm_backplanes_img_host(const PMFrame *frame_host, int nx, int ny, uint64_t p
     return check(launch_backplanes_img_host(frame_host, nx, ny, plane_mask, out, sms, (cudaStream_t)stream));
 }
 
+int pm_backplanes_points_host(const PMFrame *frame_host, const double *x, const double *y, int64_t n,
+                              uint64_t plane_mask, uint32_t flags, double *out, void *stream) {
+    if (!frame_host || n < 0 || (flags & ~PM_FLAG_RING_ALL)) return PM_ERR_BAD_ARG;
+    plane_mask &= PM_ALL_PLANES;
+    if (!plane_mask) return PM_ERR_BAD_ARG;
+    if (n == 0) return PM_OK;  // empty inputs are valid (and carry null pointers)
+    if (!x || !y || !out) return PM_ERR_BAD_ARG;
+    if (sm_count() <= 0) return PM_ERR_NO_DEVICE;
+    return check(launch_backplanes_points_host(frame_host, x, y, n, plane_mask, flags, out, (cudaStream_t)stream));
+}
+
 int pm_backplanes_map(const PMFrame *frame, const double *lon, const double *lat, int64_t n_cells,
                       uint64_t plane_mask, double *out, void *stream) {
     if (!frame || n_cells < 0) return PM_ERR_BAD_ARG;

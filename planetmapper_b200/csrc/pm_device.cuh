@@ -791,7 +791,9 @@ constexpr uint64_t kSkyMask = bit(PM_RA) | bit(PM_DEC) | kKmMask | kLimbMask | k
 // kFixedMask != 0 fixes the plane set at compile time (the launcher uses it for the
 // default surface stack): every `mask & bit` test folds away and the per-pixel code
 // becomes a handful of large basic blocks the scheduler can interleave freely.
-template <bool kSky, uint64_t kFixedMask = 0, class Sink>
+// kRingAll = true keeps ring-plane points hidden behind the body
+// (Body.ring_plane_coordinates(only_visible=False), body.py:2577-2615); the backplanes hide them.
+template <bool kSky, uint64_t kFixedMask = 0, bool kRingAll = false, class Sink>
 PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, Sink &out) {
     const PMFrame &f = fs.f;
     const double nan = NAN;
@@ -902,11 +904,26 @@ PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, S
     if (kSky && (mask & kRingMask)) {  // _get_ring_plane_coordinate_imgs (body_xy.py:4061-4085)
         double rad, rl, rd;
         ring_coordinates(fs, d2, rad, rl, rd);
-        if (rd > v_dist) rad = rl = rd = nan;  // NaN distance compares false (quirk kept)
+        if (!kRingAll && rd > v_dist) rad = rl = rd = nan;  // NaN distance compares false (quirk kept)
         if (mask & bit(PM_RING_RADIUS)) out.put(PM_RING_RADIUS, rad);
         if (mask & bit(PM_RING_LON_GRAPHIC)) out.put(PM_RING_LON_GRAPHIC, rl);
         if (mask & bit(PM_RING_DISTANCE)) out.put(PM_RING_DISTANCE, rd);
     }
+}
+
+// The image-direction planes at one arbitrary image position (pm_backplanes_points_host): a
+// fractional pixel, or one outside the image.  A non-finite x or y never reaches image_pixel -
+// a NaN ray would drive sincpt's light-time iteration, which runs until the epoch stops
+// changing - so it writes NaN to every plane, with PIXEL-X / PIXEL-Y echoing the input.
+template <bool kSky, bool kRingAll, class Sink>
+PM_HD void image_point(const FrameD &fs, double x, double y, uint64_t mask_in, Sink &out) {
+    if (fabs(x) < INFINITY && fabs(y) < INFINITY) {
+        image_pixel<kSky, 0, kRingAll>(fs, x, y, mask_in, out);
+        return;
+    }
+#pragma unroll 1
+    for (int k = 0; k < PM_N_PLANES; k++)
+        if (mask_in & bit(k)) out.put(k, k == PM_PIXEL_X ? x : (k == PM_PIXEL_Y ? y : (double)NAN));
 }
 
 // ---------------------------------------------------------------------------------

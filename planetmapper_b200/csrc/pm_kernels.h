@@ -30,6 +30,8 @@ cudaError_t launch_backplanes_img(const PMFrame *frames, int n_frames, int nx, i
                                   double *out, int sm_count, cudaStream_t st);
 cudaError_t launch_backplanes_img_host(const PMFrame *frame_host, int nx, int ny, uint64_t mask, double *out,
                                        int sm_count, cudaStream_t st);
+cudaError_t launch_backplanes_points_host(const PMFrame *frame_host, const double *x, const double *y, int64_t n,
+                                          uint64_t mask, uint32_t flags, double *out, cudaStream_t st);
 cudaError_t launch_backplanes_map(const PMFrame *frames, int n_frames, const double *lon, const double *lat,
                                   int64_t n, uint64_t mask, double *out, int sm_count, cudaStream_t st);
 cudaError_t launch_backplanes_map_host(const PMFrame *frame_host, const double *lon, const double *lat, int64_t n,
