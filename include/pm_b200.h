@@ -288,6 +288,34 @@ int pm_spline_prepare(const double *cube, int n_planes, int ny, int nx, int degr
                       void *stream);
 
 /*
+ * Smoothing splines, map_img(spline_smoothing = s > 0): per plane, FITPACK's regrid (iopt 0, maxit as
+ * given, tol 0.001, nxest = ny + k_rows + 1, nyest = nx + k_cols + 1), i.e. RectBivariateSpline(
+ * arange(ny), arange(nx), plane, kx = k_rows, ky = k_cols, s) (body_xy.py:1651-1702), one CTA per plane
+ * and one launch for any number of planes.  `coef` / `plane_bits` are pm_spline_prepare's outputs for
+ * degree PM_INTERP_LINEAR (the NaN-repaired planes); all-NaN planes are not fitted (nx = ny = 0,
+ * ier 0, fp NaN).  Per plane l, in fixed-size slots:
+ *   tx [n_planes][ny + k_rows + 1], ty [n_planes][nx + k_cols + 1], c [n_planes][ny * nx]
+ *   (c[l][i * (ny_l - k_cols - 1) + j] multiplies B_i(row) B_j(column)), nxy [n_planes][2] = knot
+ *   counts (nx_l along rows, ny_l along columns), fp [n_planes], ier [n_planes] = FITPACK's ier
+ *   (0, -1, -2 accepted by RectBivariateSpline; 1, 2, 3 are its ValueErrors).
+ * `work` must hold pm_regrid_work_bytes(...) bytes of device scratch.  k_rows, k_cols: 1..3.
+ */
+int64_t pm_regrid_work_bytes(int n_planes, int ny, int nx, int k_rows, int k_cols);
+int pm_regrid_fit(const double *coef, const uint32_t *plane_bits, int n_planes, int ny, int nx, int k_rows,
+                  int k_cols, double s, int maxit, double *tx, double *ty, double *c, int *nxy, double *fp,
+                  int *ier, void *work, void *stream);
+/*
+ * Evaluation of pm_regrid_fit's splines at map cells (RectBivariateSpline.ev(y, x), bispeu): planes
+ * [plane_begin, plane_begin + plane_count), any plane_begin; out [plane_count][n_cells].  NaN cells,
+ * all-NaN planes and (flags PM_FLAG_PROPAGATE_NAN) the cells of _should_propagate_nan_to_map are NaN,
+ * as in pm_gather; nanbits / plane_bits are pm_spline_prepare's.
+ */
+int pm_gather_regrid(const double *tx, const double *ty, const double *c, const int *nxy,
+                     const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes, int ny, int nx,
+                     int k_rows, int k_cols, int plane_begin, int plane_count, const double *xmap,
+                     const double *ymap, int64_t n_cells, uint32_t flags, double *out, void *stream);
+
+/*
  * map_img(interpolation='smooth') (BodyXY._do_smooth_interpolation, body_xy.py:1704-1790):
  *   pm_nan_minmax         np.nanmin / np.nanmax of a device array -> out2[2] (device), the x / y
  *                         map limits the host needs to size the oversampled grid (:1720-1721);

@@ -45,7 +45,7 @@ EXPORTED_SYMBOLS = [
     'pm_nan_minmax', 'pm_pchip_work_bytes', 'pm_pchip_resample', 'pm_gather_grid_linear',
     'pm_fits_data_unit_bytes', 'pm_fits_stage', 'pm_backplanes_map_batch', 'pm_gather_paired',
     'pm_host_ssb_state', 'pm_host_orientation', 'pm_backplanes_img_host', 'pm_transform', 'pm_fp64_probe', 'pm_proj_forward',
-    'pm_backplanes_points_host',
+    'pm_backplanes_points_host', 'pm_regrid_work_bytes', 'pm_regrid_fit', 'pm_gather_regrid',
 ]
 
 
@@ -98,6 +98,14 @@ def load_library() -> ctypes.CDLL:
     lib.pm_spline_planebits_bytes.argtypes = [c_i]
     lib.pm_spline_work_bytes.argtypes = [c_i, c_i, c_i, c_i]
     lib.pm_spline_prepare.argtypes = [c_p, c_i, c_i, c_i, c_i, c_p, c_p, c_p, c_p, c_p]
+    lib.pm_regrid_work_bytes.restype = c_i64
+    lib.pm_regrid_work_bytes.argtypes = [c_i, c_i, c_i, c_i, c_i]
+    lib.pm_regrid_fit.restype = c_i
+    lib.pm_regrid_fit.argtypes = [c_p, c_p, c_i, c_i, c_i, c_i, c_i, ctypes.c_double, c_i, c_p, c_p, c_p, c_p, c_p,
+                                  c_p, c_p, c_p]
+    lib.pm_gather_regrid.restype = c_i
+    lib.pm_gather_regrid.argtypes = [c_p, c_p, c_p, c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_i, c_p, c_p, c_i64,
+                                     c_u32, c_p, c_p]
     lib.pm_fp64_peak_probe.argtypes = [c_i, c_p, c_p]
     lib.pm_fp64_probe.argtypes = [c_i, c_i, c_p, c_p]
     lib.pm_fp64_probe.restype = c_i
@@ -538,6 +546,62 @@ def gather(src, xmap_dev, ymap_dev, mode: int, *, plane_begin: int = 0, plane_co
                        xmap_dev.data_ptr(), ymap_dev.data_ptr(), n_cells, cells_per_row, mode, flags,
                        out.data_ptr(), _stream_ptr(torch))
     _check(rc, 'pm_gather')
+    return out
+
+
+class RegridFit:
+    """Per-plane smoothing splines of :func:`regrid_fit`: device tensors in fixed-size slots (tx (n, ny +
+    k_rows + 1), ty (n, nx + k_cols + 1), c (n, ny * nx), nxy (n, 2) knot counts, fp (n,)), the FITPACK
+    ier of every plane as a host array, and the prepared cube (repaired planes, NaN bit planes)."""
+
+    def __init__(self, spline, tx, ty, c, nxy, fp, ier, k_rows, k_cols):
+        self.spline, self.tx, self.ty, self.c, self.nxy, self.fp, self.ier = spline, tx, ty, c, nxy, fp, ier
+        self.k_rows, self.k_cols = k_rows, k_cols
+
+
+def regrid_fit(cube_dev, k_rows: int, k_cols: int, s: float, maxit: int = 20) -> RegridFit:
+    """RectBivariateSpline(arange(ny), arange(nx), plane, kx=k_rows, ky=k_cols, s=s, maxit=maxit) for every
+    plane of a (n, ny, nx) CUDA cube after map_img's NaN repair: one fit launch, then one copy of the ier
+    array to the host (the only synchronisation)."""
+    torch = _torch()
+    lib = load_library()
+    nl, ny, nx = cube_dev.shape
+    dev = cube_dev.device
+    spline = spline_prepare(cube_dev, INTERP_LINEAR)
+    tx = torch.empty((nl, ny + k_rows + 1), dtype=torch.float64, device=dev)
+    ty = torch.empty((nl, nx + k_cols + 1), dtype=torch.float64, device=dev)
+    c = torch.empty((nl, ny * nx), dtype=torch.float64, device=dev)
+    nxy = torch.empty((nl, 2), dtype=torch.int32, device=dev)
+    fp = torch.empty((nl,), dtype=torch.float64, device=dev)
+    ier = torch.empty((nl,), dtype=torch.int32, device=dev)
+    nbytes = lib.pm_regrid_work_bytes(nl, ny, nx, k_rows, k_cols)
+    if nbytes < 0:
+        _check(int(nbytes), 'pm_regrid_work_bytes')
+    work = torch.empty((max(int(nbytes), 256),), dtype=torch.uint8, device=dev)
+    rc = lib.pm_regrid_fit(spline.coef.data_ptr(), spline.plane_bits.data_ptr(), nl, ny, nx, k_rows, k_cols,
+                           float(s), int(maxit), tx.data_ptr(), ty.data_ptr(), c.data_ptr(), nxy.data_ptr(),
+                           fp.data_ptr(), ier.data_ptr(), work.data_ptr(), _stream_ptr(torch))
+    _check(rc, 'pm_regrid_fit')
+    return RegridFit(spline, tx, ty, c, nxy, fp, ier.cpu().numpy(), k_rows, k_cols)
+
+
+def gather_regrid(fit: RegridFit, xmap_dev, ymap_dev, *, plane_begin: int = 0, plane_count=None,
+                  propagate_nan: bool = True, out=None):
+    """Evaluate the splines of planes [plane_begin, plane_begin + plane_count) of :func:`regrid_fit` at the
+    map cells (RectBivariateSpline.ev(y, x)).  Returns (plane_count,) + xmap.shape."""
+    torch = _torch()
+    lib = load_library()
+    sp = fit.spline
+    if plane_count is None:
+        plane_count = sp.n_planes - plane_begin
+    if out is None:
+        out = torch.empty((plane_count,) + tuple(xmap_dev.shape), dtype=torch.float64, device=xmap_dev.device)
+    flags = FLAG_PROPAGATE_NAN if propagate_nan else 0
+    rc = lib.pm_gather_regrid(fit.tx.data_ptr(), fit.ty.data_ptr(), fit.c.data_ptr(), fit.nxy.data_ptr(),
+                              sp.nanbits.data_ptr(), sp.plane_bits.data_ptr(), sp.n_planes, sp.ny, sp.nx, fit.k_rows,
+                              fit.k_cols, plane_begin, plane_count, xmap_dev.data_ptr(), ymap_dev.data_ptr(),
+                              xmap_dev.numel(), flags, out.data_ptr(), _stream_ptr(torch))
+    _check(rc, 'pm_gather_regrid')
     return out
 
 

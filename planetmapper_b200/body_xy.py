@@ -1207,8 +1207,9 @@ class BodyXY(ProgressMixin):
         maps of the requested projection and, for the spline modes, the repaired / prefiltered coefficient
         planes.  The result maps any range of planes on demand (one gather launch per call), which is how
         Observation walks a cube whose mapped output is larger than device or host memory."""
+        smoothing = _smoothing_degrees(interpolation, spline_smoothing)
         torch = L._torch()
-        mode = _interpolation_mode(interpolation, spline_smoothing)
+        mode = INTERP_REGRID if smoothing else _interpolation_mode(interpolation, spline_smoothing)
         if isinstance(img, torch.Tensor):
             cube = img if img.dim() == 3 else img[None]
             cube = cube.to(device='cuda', dtype=torch.float64).contiguous()
@@ -1227,14 +1228,17 @@ class BodyXY(ProgressMixin):
         if mode not in (L.INTERP_NEAREST, INTERP_SMOOTH):
             if warn_nan and bool(torch.isfinite(cube).logical_not().any()):
                 print('Warning, image contains NaN values which will be corrected')
-            spline = L.spline_prepare(cube, mode)
+            if mode == INTERP_REGRID:
+                spline = _fit_smoothing_splines(cube, *smoothing, spline_smoothing)
+            else:
+                spline = L.spline_prepare(cube, mode)
         return _MapSource(mode, cube, spline, xy[0], xy[1], propagate_nan, smooth_oversample_by,
                           smooth_max_oversampled_img_size)
 
 
 class _MapSource:
     """A cube prepared for mapping onto one x / y map; ``gather(begin, count)`` maps planes
-    [begin, begin + count) (``begin`` a multiple of 4 for the spline modes)."""
+    [begin, begin + count) (``begin`` a multiple of 4 for the interpolating spline modes)."""
 
     def __init__(self, mode, cube, spline, xmap, ymap, propagate_nan, smooth_oversample_by, smooth_max_size):
         self.mode, self.cube, self.spline, self.xmap, self.ymap = mode, cube, spline, xmap, ymap
@@ -1250,11 +1254,74 @@ class _MapSource:
             return L.map_smooth(self.cube[begin:begin + count], self.xmap, self.ymap, propagate_nan=self.propagate_nan,
                                 oversample_by=self.smooth_oversample_by,
                                 max_oversampled_img_size=self.smooth_max_size, out=out)
+        if self.mode == INTERP_REGRID:
+            return L.gather_regrid(self.spline, self.xmap, self.ymap, plane_begin=begin, plane_count=count,
+                                   propagate_nan=self.propagate_nan, out=out)
         return L.gather(self.spline, self.xmap, self.ymap, self.mode, plane_begin=begin, plane_count=count,
                         propagate_nan=self.propagate_nan, out=out)
 
 
 INTERP_SMOOTH = -1   # host-side marker: PCHIP oversampling + linear (its own entry points)
+INTERP_REGRID = -2   # host-side marker: smoothing splines, spline_smoothing > 0 (pm_regrid_fit / pm_gather_regrid)
+
+# scipy.interpolate._fitpack2._surfit_messages: RectBivariateSpline's ValueError text for each FITPACK ier
+_SURFIT_MESSAGES = {1: """
+The required storage space exceeds the available storage space: nxest
+or nyest too small, or s too small.
+The weighted least-squares spline corresponds to the current set of
+knots.""",
+                    2: """
+A theoretically impossible result was found during the iteration
+process for finding a smoothing spline with fp = s: s too small or
+badly chosen eps.
+Weighted sum of squared residuals does not satisfy abs(fp-s)/s < tol.""",
+                    3: """
+the maximal number of iterations maxit (set to 20 by the program)
+allowed for finding a smoothing spline with fp=s has been reached:
+s too small.
+Weighted sum of squared residuals does not satisfy abs(fp-s)/s < tol.
+Try increasing maxit by passing it as a keyword argument."""}
+
+
+def _smoothing_degrees(interpolation, spline_smoothing):
+    """(k_rows, k_cols) when map_img must fit smoothing splines (spline_smoothing != 0 with a spline degree),
+    else None (every other call goes through _interpolation_mode unchanged)."""
+    if spline_smoothing == 0:
+        return None
+    spline_k = {'linear': 1, 'quadratic': 2, 'cubic': 3}
+    if isinstance(interpolation, str):
+        if interpolation not in spline_k:
+            return None
+        k = spline_k[interpolation]
+        degrees = (k, k)
+    elif isinstance(interpolation, (int, np.integer)) and not isinstance(interpolation, bool):
+        degrees = (int(interpolation), int(interpolation))
+    elif isinstance(interpolation, tuple) and len(interpolation) == 2:
+        degrees = tuple(int(k) for k in interpolation)
+    else:
+        return None
+    if not all(1 <= k <= 3 for k in degrees):
+        raise NotImplementedError(f'spline degrees {interpolation!r} with spline_smoothing != 0 are not '
+                                  'accelerated (1..3 are)')
+    if not spline_smoothing >= 0.0:   # RectBivariateSpline's own check
+        raise ValueError('s should be s >= 0.0')
+    return degrees
+
+
+def _fit_smoothing_splines(cube, k_rows: int, k_cols: int, s: float):
+    """RectBivariateSpline(arange(ny), arange(nx), plane, kx=k_rows, ky=k_cols, s=s) per plane on the device
+    (body_xy.py:1651-1702); raises its ValueError for the first plane, in plane order, whose fit fails."""
+    _, ny, nx = cube.shape
+    if ny <= k_rows:
+        raise ValueError('mx must be > kx')
+    if nx <= k_cols:
+        raise ValueError('my must be > ky')
+    fit = L.regrid_fit(cube, k_rows, k_cols, float(s))
+    bad = np.flatnonzero(~np.isin(fit.ier, (0, -1, -2)))
+    if bad.size:
+        ier = int(fit.ier[bad[0]])
+        raise ValueError(_SURFIT_MESSAGES.get(ier, f'ier={ier}'))
+    return fit
 
 
 def _interpolation_mode(interpolation, spline_smoothing) -> int:

@@ -270,6 +270,46 @@ int pm_pchip_resample(const double *cube, int n_planes, int ny, int nx, int x_fi
                                        (cudaStream_t)stream));
 }
 
+static bool regrid_degrees_ok(int k_rows, int k_cols) { return k_rows >= 1 && k_rows <= 3 && k_cols >= 1 && k_cols <= 3; }
+
+int64_t pm_regrid_work_bytes(int n_planes, int ny, int nx, int k_rows, int k_cols) {
+    if (n_planes < 0 || ny <= 0 || nx <= 0) return PM_ERR_BAD_ARG;
+    if (!regrid_degrees_ok(k_rows, k_cols)) return PM_ERR_UNSUPPORTED;
+    return regrid_work_bytes(n_planes, ny, nx, k_rows, k_cols);
+}
+
+int pm_regrid_fit(const double *coef, const uint32_t *plane_bits, int n_planes, int ny, int nx, int k_rows,
+                  int k_cols, double s, int maxit, double *tx, double *ty, double *c, int *nxy, double *fp, int *ier,
+                  void *work, void *stream) {
+    if (n_planes < 0 || ny <= 0 || nx <= 0 || !(s > 0.0) || !(s <= 1.79769313486231570e308) || maxit < 1)
+        return PM_ERR_BAD_ARG;
+    if (!regrid_degrees_ok(k_rows, k_cols)) return PM_ERR_UNSUPPORTED;
+    if (ny <= k_rows || nx <= k_cols) return PM_ERR_BAD_ARG;
+    if (n_planes == 0) return PM_OK;
+    if (!coef || !plane_bits || !tx || !ty || !c || !nxy || !fp || !ier || !work) return PM_ERR_BAD_ARG;
+    int sms = sm_count();
+    if (sms <= 0) return PM_ERR_NO_DEVICE;
+    return check(launch_regrid_fit(coef, plane_bits, n_planes, ny, nx, k_rows, k_cols, s, maxit, tx, ty, c, nxy, fp,
+                                   ier, work, (cudaStream_t)stream));
+}
+
+int pm_gather_regrid(const double *tx, const double *ty, const double *c, const int *nxy, const uint32_t *nanbits,
+                     const uint32_t *plane_bits, int n_planes, int ny, int nx, int k_rows, int k_cols, int plane_begin,
+                     int plane_count, const double *xmap, const double *ymap, int64_t n_cells, uint32_t flags,
+                     double *out, void *stream) {
+    if (n_planes < 0 || ny <= 0 || nx <= 0 || n_cells < 0 || plane_begin < 0 || plane_count < 0 ||
+        plane_begin > n_planes - plane_count || (flags & ~PM_FLAG_PROPAGATE_NAN))
+        return PM_ERR_BAD_ARG;
+    if (!regrid_degrees_ok(k_rows, k_cols)) return PM_ERR_UNSUPPORTED;
+    if (ny <= k_rows || nx <= k_cols) return PM_ERR_BAD_ARG;
+    if (n_cells == 0 || plane_count == 0) return PM_OK;  // the empty arrays may carry null pointers
+    if (!tx || !ty || !c || !nxy || !nanbits || !plane_bits || !xmap || !ymap || !out) return PM_ERR_BAD_ARG;
+    int sms = sm_count();
+    if (sms <= 0) return PM_ERR_NO_DEVICE;
+    return check(launch_gather_regrid(tx, ty, c, nxy, nanbits, plane_bits, n_planes, ny, nx, k_rows, k_cols,
+                                      plane_begin, plane_count, xmap, ymap, n_cells, flags, out, (cudaStream_t)stream));
+}
+
 int pm_gather_grid_linear(const double *fine, int n_planes, int n_ys, int n_xs, int x_first, int x_last, int y_first,
                           int y_last, const double *cube, int ny, int nx, const double *xmap, const double *ymap,
                           int64_t n_cells, uint32_t flags, double *out, void *stream) {

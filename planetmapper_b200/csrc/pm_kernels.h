@@ -70,6 +70,15 @@ cudaError_t launch_spline_prepare(const double *cube, int n_planes, int ny, int 
                                   uint32_t *nanbits, uint32_t *plane_bits, void *work, int sm_count,
                                   cudaStream_t st);
 
+// map_img with spline_smoothing > 0 (regrid_kernels.cu)
+int64_t regrid_work_bytes(int n_planes, int ny, int nx, int k_rows, int k_cols);
+cudaError_t launch_regrid_fit(const double *coefq, const uint32_t *plane_bits, int n_planes, int ny, int nx,
+                              int k_rows, int k_cols, double s, int maxit, double *tx, double *ty, double *c, int *nxy,
+                              double *fp, int *ier, void *work, cudaStream_t st);
+cudaError_t launch_gather_regrid(const double *tx, const double *ty, const double *c, const int *nxy,
+                                 const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes, int ny, int nx,
+                                 int k_rows, int k_cols, int plane_begin, int plane_count, const double *xmap,
+                                 const double *ymap, int64_t n_cells, uint32_t flags, double *out, cudaStream_t st);
 
 // map_img(interpolation='smooth') (smooth_kernels.cu)
 cudaError_t launch_nan_minmax(const double *x, int64_t n, double *out2, cudaStream_t st);
