@@ -59,7 +59,7 @@ struct PlaneSink {
 // Image direction: all requested backplanes for every pixel of every frame.
 // ---------------------------------------------------------------------------------
 // Pixels idx, idx + 128, ... of this CTA's tile, every requested plane of each
-template <bool kSky, uint64_t kFixedMask>
+template <bool kSky, uint64_t kFixedMask, bool kSpinSym>
 __device__ __forceinline__ void img_tile(const FrameD &fs, uint32_t tile, uint32_t nx, uint32_t npx, int per_thread,
                                          uint64_t mask, const PlaneOffsets &po, double *__restrict__ out) {
     uint32_t idx = tile * (uint32_t)(kBlock * per_thread) + threadIdx.x;
@@ -67,7 +67,7 @@ __device__ __forceinline__ void img_tile(const FrameD &fs, uint32_t tile, uint32
 #pragma unroll 1
     for (int r = 0; r < per_thread && idx < npx; r++) {
         PlaneSink sink{reinterpret_cast<char *>(out + idx), po};
-        image_pixel<kSky, kFixedMask>(fs, (double)xi, (double)yi, mask, sink);
+        image_pixel<kSky, kFixedMask, false, kSpinSym>(fs, (double)xi, (double)yi, mask, sink);
         idx += kBlock;
         xi += kBlock;
         while (xi >= nx) {
@@ -77,7 +77,8 @@ __device__ __forceinline__ void img_tile(const FrameD &fs, uint32_t tile, uint32
     }
 }
 
-// Batched launch (time series): frame blockIdx.y is staged in shared memory by the CTA
+// Batched launch (time series): frame blockIdx.y is staged in shared memory by the CTA.  The frame's
+// spin_sym flag is uniform over the CTA, so the branch on it does not diverge.
 template <bool kSky, uint64_t kFixedMask>
 __global__ void __launch_bounds__(kBlock, 4) backplanes_img_kernel(const PMFrame *__restrict__ frames, uint32_t nx,
                                                                    uint32_t npx, int per_thread, uint64_t mask,
@@ -85,8 +86,11 @@ __global__ void __launch_bounds__(kBlock, 4) backplanes_img_kernel(const PMFrame
                                                                    double *__restrict__ out_all) {
     __shared__ FrameD fs;
     load_frame(fs, frames + blockIdx.y);
-    img_tile<kSky, kFixedMask>(fs, blockIdx.x, nx, npx, per_thread, mask, po,
-                               out_all + (int64_t)blockIdx.y * __popcll(mask) * npx);
+    double *out = out_all + (int64_t)blockIdx.y * __popcll(mask) * npx;
+    if (fs.spin_sym)
+        img_tile<kSky, kFixedMask, true>(fs, blockIdx.x, nx, npx, per_thread, mask, po, out);
+    else
+        img_tile<kSky, kFixedMask, false>(fs, blockIdx.x, nx, npx, per_thread, mask, po, out);
 }
 
 // Single frame: the finished constants (derived on the host with the same exactly rounded
@@ -104,19 +108,19 @@ __device__ __forceinline__ uint32_t centre_out_tile(uint32_t k, uint32_t n_tiles
     if (j <= min(lo, hi)) return (k & 1u) ? centre + j : centre - j;
     return lo < hi ? k : n_tiles - 1u - k;  // one side exhausted: the rest in order, moving away
 }
-template <bool kSky, uint64_t kFixedMask>
+template <bool kSky, uint64_t kFixedMask, bool kSpinSym>
 __global__ void __launch_bounds__(kBlock, kImgParamCtas) backplanes_img_param_kernel(
     const __grid_constant__ FrameD fs, uint32_t nx, uint32_t npx, int per_thread, uint32_t centre_tile, uint64_t mask,
     const __grid_constant__ PlaneOffsets po, double *__restrict__ out) {
-    img_tile<kSky, kFixedMask>(fs, centre_out_tile(blockIdx.x, gridDim.x, centre_tile), nx, npx, per_thread, mask,
-                               po, out);
+    img_tile<kSky, kFixedMask, kSpinSym>(fs, centre_out_tile(blockIdx.x, gridDim.x, centre_tile), nx, npx, per_thread,
+                                         mask, po, out);
 }
 
 // ---------------------------------------------------------------------------------
 // Image direction at arbitrary positions (pm_backplanes_points_host): the per-pixel code of the
 // single-frame image kernel on a list of (x, y), tiled like map_tile; output plane stride = n
 // ---------------------------------------------------------------------------------
-template <bool kSky, bool kRingAll>
+template <bool kSky, bool kRingAll, bool kSpinSym>
 __global__ void __launch_bounds__(kBlock, 4) backplanes_points_param_kernel(const __grid_constant__ FrameD fs,
                                                                             const double *__restrict__ x_in,
                                                                             const double *__restrict__ y_in,
@@ -129,7 +133,7 @@ __global__ void __launch_bounds__(kBlock, 4) backplanes_points_param_kernel(cons
         const int64_t idx = first + r * kBlock;
         if (idx >= n) break;
         PlaneSink sink{reinterpret_cast<char *>(out + idx), po};
-        image_point<kSky, kRingAll>(fs, __ldg(x_in + idx), __ldg(y_in + idx), mask, sink);
+        image_point<kSky, kRingAll, kSpinSym>(fs, __ldg(x_in + idx), __ldg(y_in + idx), mask, sink);
     }
 }
 
@@ -373,7 +377,19 @@ cudaError_t launch_backplanes_img(const PMFrame *frames, int n_frames, int nx, i
     count_launches(1);
     return cudaGetLastError();
 }
-// single frame given on the HOST: constants derived here, passed by value
+template <bool kSpinSym>
+static void launch_img_param(const FrameD &fs, dim3 grid, uint32_t nx, uint32_t npx, int per, uint32_t centre,
+                             uint64_t mask, const PlaneOffsets &po, double *out, cudaStream_t st) {
+    if (mask == kDefaultStackMask)
+        backplanes_img_param_kernel<false, kDefaultStackMask, kSpinSym><<<grid, kBlock, 0, st>>>(fs, nx, npx, per, centre,
+                                                                                                mask, po, out);
+    else if (mask & kSkyMask)
+        backplanes_img_param_kernel<true, 0, kSpinSym><<<grid, kBlock, 0, st>>>(fs, nx, npx, per, centre, mask, po, out);
+    else
+        backplanes_img_param_kernel<false, 0, kSpinSym><<<grid, kBlock, 0, st>>>(fs, nx, npx, per, centre, mask, po, out);
+}
+// single frame given on the HOST: constants derived here, passed by value; the frame's spin_sym flag
+// picks the instantiation, so each kernel carries one path's code and registers only
 cudaError_t launch_backplanes_img_host(const PMFrame *frame_host, int nx, int ny, uint64_t mask, double *out,
                                        int sm_count, cudaStream_t st) {
     const int64_t npx = (int64_t)nx * ny;
@@ -394,17 +410,23 @@ cudaError_t launch_backplanes_img_host(const PMFrame *frame_host, int nx, int ny
     static const bool linear = tune_int("PM_IMG_ORDER", 1) == 0;
     if (linear) ct = 0;
     const uint32_t centre = (uint32_t)(ct < 0 ? 0 : (ct >= n_tiles ? n_tiles - 1 : ct));
-    if (mask == kDefaultStackMask)
-        backplanes_img_param_kernel<false, kDefaultStackMask><<<grid, kBlock, 0, st>>>(
-            fs, (uint32_t)nx, (uint32_t)npx, per, centre, mask, po, out);
-    else if (mask & kSkyMask)
-        backplanes_img_param_kernel<true, 0><<<grid, kBlock, 0, st>>>(fs, (uint32_t)nx, (uint32_t)npx, per, centre, mask,
-                                                                       po, out);
+    if (fs.spin_sym)
+        launch_img_param<true>(fs, grid, (uint32_t)nx, (uint32_t)npx, per, centre, mask, po, out, st);
     else
-        backplanes_img_param_kernel<false, 0><<<grid, kBlock, 0, st>>>(fs, (uint32_t)nx, (uint32_t)npx, per, centre, mask,
-                                                                        po, out);
+        launch_img_param<false>(fs, grid, (uint32_t)nx, (uint32_t)npx, per, centre, mask, po, out, st);
     count_launches(1);
     return cudaGetLastError();
+}
+template <bool kSpinSym>
+static void launch_points_param(const FrameD &fs, unsigned grid, const double *x, const double *y, int64_t n,
+                                uint64_t mask, uint32_t flags, const PlaneOffsets &po, double *out, cudaStream_t st) {
+    // the ring planes are sky planes: without a sky plane PM_FLAG_RING_ALL has nothing to change
+    if (!(mask & kSkyMask))
+        backplanes_points_param_kernel<false, false, kSpinSym><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
+    else if (flags & PM_FLAG_RING_ALL)
+        backplanes_points_param_kernel<true, true, kSpinSym><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
+    else
+        backplanes_points_param_kernel<true, false, kSpinSym><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
 }
 // n arbitrary image positions of ONE frame given on the HOST (constants derived here, as above)
 cudaError_t launch_backplanes_points_host(const PMFrame *frame_host, const double *x, const double *y, int64_t n,
@@ -413,13 +435,10 @@ cudaError_t launch_backplanes_points_host(const PMFrame *frame_host, const doubl
     load_frame_host(fs, frame_host);
     const PlaneOffsets po = make_plane_offsets(mask, n);
     const unsigned grid = chunks_for(n);
-    // the ring planes are sky planes: without a sky plane PM_FLAG_RING_ALL has nothing to change
-    if (!(mask & kSkyMask))
-        backplanes_points_param_kernel<false, false><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
-    else if (flags & PM_FLAG_RING_ALL)
-        backplanes_points_param_kernel<true, true><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
+    if (fs.spin_sym)
+        launch_points_param<true>(fs, grid, x, y, n, mask, flags, po, out, st);
     else
-        backplanes_points_param_kernel<true, false><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
+        launch_points_param<false>(fs, grid, x, y, n, mask, flags, po, out, st);
     count_launches(1);
     return cudaGetLastError();
 }

@@ -84,7 +84,7 @@ struct FrameD {
     double As[6];      // xy -> (-ax, ay) in radians: A scaled by rpd / 3600 (first row negated)
     double inv_kmpa;   // 1 / km_per_arcsec
     int biaxial;       // intercept ellipsoid == recpgr spheroid -> closed-form geodetic
-    int pad_;
+    int spin_sym;      // spheroid spinning about its symmetry axis: the image planes are taken in the t_ref frame
 };
 
 constexpr int kDeriveItems = 13;
@@ -160,6 +160,15 @@ PM_HD void derive_frame_item(FrameD &s, int item) {
         s.k[0] = wn > 0.0 ? ex_div(f.omega[0], wn) : 0.0;
         s.k[1] = wn > 0.0 ? ex_div(f.omega[1], wn) : 0.0;
         s.k[2] = wn > 0.0 ? ex_div(f.omega[2], wn) : 0.0;
+        // A spin about the z axis commutes with the scaling of a spheroid with radii[0] == radii[1], so the
+        // intercept and the illumination angles can be solved in the t_ref frame (image_pixel<kSpinSym>).
+        // What that neglects is the spin axis' tilt off z: a displacement of at most |omega_perp| dt (a - c)
+        // of the surface, with |dt| <= 2 a / clight over the disc.  Allowed up to 1e-9 km, far below the
+        // ~4e-7 km that one ulp of the epoch et - lt moves the target (DESIGN.md section 5); 0 for a sphere.
+        const double wperp = ex_sqrt(ex_add(ex_mul(f.omega[0], f.omega[0]), ex_mul(f.omega[1], f.omega[1])));
+        const double flat = fabs(ex_add(f.radii[0], -f.radii[2]));
+        const double shift = ex_mul(ex_mul(wperp, ex_div(ex_mul(2.0, f.radii[0]), f.clight)), flat);
+        s.spin_sym = (f.radii[0] == f.radii[1]) && (shift <= 1.0e-9);
     } else if (item == 1) {
         const double a = f.radii[0], b = f.radii[1], c = f.radii[2];
         s.inv_r[0] = ex_div(1.0, a);
@@ -180,7 +189,6 @@ PM_HD void derive_frame_item(FrameD &s, int item) {
         s.omf = omf;
         s.inv_omf2 = ex_div(1.0, ex_mul(omf, omf));
         s.biaxial = (f.radii[0] == f.radii[1]) && (f.re == f.radii[0]) && (fabs(rp - f.radii[2]) <= 4e-16 * f.radii[2]);
-        s.pad_ = 0;
     }
 }
 
@@ -313,15 +321,10 @@ struct RayHit {
     double t;     // ray parameter of the intercept, t = a - h with the half-chord h = sqrt((1 - |pp|^2) ixx)
     double cos2;  // 1 - |pp|^2: squared half-chord in the unit-sphere space, -> 0 at tangency
 };
-// y: the ray's origin in the scaled (unit-sphere) space, ym2 = |y|^2 (surfpt below, or per frame)
-PM_HD bool surfpt_y(const FrameD &fs, V3 y, double ym2, V3 u, V3 &p, RayHit &hit) {
-    // scaled space (unit sphere); the direction x is deliberately NOT normalised: the
-    // three dot products are independent and a single reciprocal serves both the
-    // projection and the half-chord
-    const V3 x = mul3(u, fs.inv_r);
-    const double xx = dot(x, x), yx = dot(y, x);
-    if (!(xx > 0.0)) return false;
-    const double ixx = fast_rcp(xx);
+// y: the ray's origin in the scaled (unit-sphere) space, ym2 = |y|^2 (surfpt below, or per frame);
+// x = u / radii: the ray's direction in that space, ixx = 1 / |x|^2
+PM_HD bool surfpt_yx(const FrameD &fs, V3 y, double ym2, V3 x, double ixx, V3 &p, RayHit &hit) {
+    const double yx = dot(y, x);
     const double a = -(yx * ixx);
     const V3 pp = axpy(a, x, y);  // component of y perpendicular to the ray
     const double pm2 = dot(pp, pp);
@@ -344,6 +347,15 @@ PM_HD bool surfpt_y(const FrameD &fs, V3 y, double ym2, V3 u, V3 &p, RayHit &hit
     p = mul3(axpy(h, x, pp), fs.f.radii);
     return true;
 }
+PM_HD bool surfpt_y(const FrameD &fs, V3 y, double ym2, V3 u, V3 &p, RayHit &hit) {
+    // scaled space (unit sphere); the direction x is deliberately NOT normalised: the
+    // three dot products are independent and a single reciprocal serves both the
+    // projection and the half-chord
+    const V3 x = mul3(u, fs.inv_r);
+    const double xx = dot(x, x);
+    if (!(xx > 0.0)) return false;
+    return surfpt_yx(fs, y, ym2, x, fast_rcp(xx), p, hit);
+}
 PM_HD bool surfpt(const FrameD &fs, V3 o, V3 u, V3 &p, RayHit &hit) {
     const V3 y = mul3(o, fs.inv_r);
     return surfpt_y(fs, y, dot(y, y), u, p, hit);
@@ -355,6 +367,8 @@ struct Intercept {
     V3 p;        // surface point (body-fixed)
     V3 u;        // unit ray observer -> point in the body frame at the intercept epoch: the line of sight
                  // itself (exact), not (p - o) / L, which carries p's error magnified by r / L for a near observer
+                 // (general path only)
+    V3 p0;       // the surface point in the body frame at t_ref (spin-symmetric path only)
     Rot r;       // spin over dt
     double dt;   // intercept epoch - t_ref
     double L;    // observer -> point range (km)
@@ -365,13 +379,19 @@ struct Intercept {
 // epoch: CSPICE's loop as written - full intercepts until the FP64 epoch et - lt stops
 // changing (at most 10 passes in total).  dt (in: epoch offset of the next pass) and p come
 // back for the converged pass.  Kept out of line so the common path keeps its registers.
+// kSpinSym (FrameD::spin_sym): every pass is solved in the body frame at t_ref, so p is the point in that frame.
+template <bool kSpinSym>
 PM_HD_NOINLINE bool sincpt_converge(const FrameD &fs, V3 u0, double &dt, V3 &p, double &range) {
     const PMFrame &f = fs.f;
     for (int it = 0; it < 8; it++) {
-        const Rot r = make_rot(fs, dt);
-        const V3 o = spin_fwd(fs, r, -target_pos_b(fs, dt));
+        V3 o = -target_pos_b(fs, dt), u = u0;
+        if (!kSpinSym) {
+            const Rot r = make_rot(fs, dt);
+            o = spin_fwd(fs, r, o);
+            u = spin_fwd(fs, r, u0);
+        }
         RayHit hit;
-        if (!surfpt(fs, o, spin_fwd(fs, r, u0), p, hit)) return false;
+        if (!surfpt(fs, o, u, p, hit)) return false;
         range = hit.t;
         const double t = dt + f.t_ref;
         const double t_new = f.et - hit.t * fs.inv_c;  // u0 is a unit vector: the ray parameter is the range
@@ -396,16 +416,32 @@ PM_HD_NOINLINE bool sincpt_converge(const FrameD &fs, V3 u0, double &dt, V3 &p, 
 //   Grazing rays (cos^2 of the scaled-space emission <= kGrazingCos2, i.e. emission > ~86.9 deg) are the
 //   exception: there the light time is too far from linear in the epoch for the two-point fixed point,
 //   so those pixels run CSPICE's loop as written (until et - lt is stable).
+//
+// kSpinSym (FrameD::spin_sym): the body is a spheroid spinning about its symmetry axis.  Spinning the
+// observer and the ray together about that axis leaves the ray / ellipsoid solve unchanged, so every pass
+// is solved in the body frame at t_ref - observer -target_pos_b(dt), ray u0 - and only the final point is
+// spun to its epoch.  Pass 2 then shares pass 1's direction x and 1 / |x|^2, and it.p0 holds the point at
+// t_ref; it.u is not set.
+template <bool kSpinSym = false>
 PM_HD bool sincpt(const FrameD &fs, V3 u0, Intercept &it) {
     const PMFrame &f = fs.f;
     V3 p1, p2;
     RayHit h1, h2;
-    if (!surfpt_y(fs, ld3(fs.y0), fs.y0m2, u0, p1, h1)) return false;  // observer at t_ref: -P0b
+    const V3 x = mul3(u0, fs.inv_r);
+    const double xx = dot(x, x);
+    if (!(xx > 0.0)) return false;
+    const double ixx = fast_rcp(xx);
+    if (!surfpt_yx(fs, ld3(fs.y0), fs.y0m2, x, ixx, p1, h1)) return false;  // observer at t_ref: -P0b
     const double lt1 = h1.t * fs.inv_c;  // u0 is a unit vector: the ray parameter is the range
 
     const double dt1 = (f.et - lt1) - f.t_ref;
-    const Rot r1 = make_rot(fs, dt1);
-    if (!surfpt(fs, spin_fwd(fs, r1, -target_pos_b(fs, dt1)), spin_fwd(fs, r1, u0), p2, h2)) return false;
+    if (kSpinSym) {
+        const V3 y2 = mul3(-target_pos_b(fs, dt1), fs.inv_r);
+        if (!surfpt_yx(fs, y2, dot(y2, y2), x, ixx, p2, h2)) return false;
+    } else {
+        const Rot r1 = make_rot(fs, dt1);
+        if (!surfpt(fs, spin_fwd(fs, r1, -target_pos_b(fs, dt1)), spin_fwd(fs, r1, u0), p2, h2)) return false;
+    }
     const double lt2 = h2.t * fs.inv_c;
 
     // epochs as CSPICE forms them: et - lt rounded to a double (granularity ulp(et) ~ 3e-8 s,
@@ -427,20 +463,31 @@ PM_HD bool sincpt(const FrameD &fs, V3 u0, Intercept &it) {
         dt = fma(lam, dt1, dt1) + f.t_ref;  // the fixed point, rounded as et - lt is
         dt -= f.t_ref;
         const V3 pps = axpy(lam, h2.pp - h1.pp, h2.pp);
-        const double hs = fast_sqrt_lite(fmax(1.0 - dot(pps, pps), 0.0) * fma(lam, h2.ixx - h1.ixx, h2.ixx));
+        const double ixxs = kSpinSym ? ixx : fma(lam, h2.ixx - h1.ixx, h2.ixx);
+        const double hs = fast_sqrt_lite(fmax(1.0 - dot(pps, pps), 0.0) * ixxs);
         L = fma(lam, h2.a - h1.a, h2.a) - hs;
         it.r = make_rot(fs, dt);
-        it.u = spin_fwd(fs, it.r, u0);
-        p = axpy(-hs, it.u, mul3(pps, fs.f.radii));
+        if (kSpinSym) {
+            it.p0 = axpy(-hs, u0, mul3(pps, fs.f.radii));
+            p = spin_fwd(fs, it.r, it.p0);
+        } else {
+            it.u = spin_fwd(fs, it.r, u0);
+            p = axpy(-hs, it.u, mul3(pps, fs.f.radii));
+        }
     } else {
         double dt_c = dt, L_c;  // address-taken copies: keep dt and p themselves in registers
         V3 p_c;
-        if (!sincpt_converge(fs, u0, dt_c, p_c, L_c)) return false;
+        if (!sincpt_converge<kSpinSym>(fs, u0, dt_c, p_c, L_c)) return false;
         dt = dt_c;
-        p = p_c;
         L = L_c;
         it.r = make_rot(fs, dt);
-        it.u = spin_fwd(fs, it.r, u0);
+        if (kSpinSym) {
+            it.p0 = p_c;
+            p = spin_fwd(fs, it.r, p_c);
+        } else {
+            p = p_c;
+            it.u = spin_fwd(fs, it.r, u0);
+        }
     }
     it.p = p;
     it.dt = dt;
@@ -620,13 +667,12 @@ PM_HD void illum_angles(V3 n, V3 s, V3 e, bool want_az, Illum &out) {
     }
 }
 
-// Illumination geometry of body-fixed point p at epoch offset dt (spin r), given the
-// point -> observer vector e (body frame at the epoch).  Solves the Sun -> point light
-// time from the frame's seed lts0.  VS is the Sun's barycentric velocity (~0.013 km/s):
-// the contraction factor of the iteration is VS / c ~ 4e-8 and the seed is off by
-// <= R / c, so ONE refinement leaves a Sun-direction error below 1e-18 rad.
-PM_HD void illum_at(const FrameD &fs, V3 p, V3 p0 /* spin_bwd(p) */, V3 e, Rot r, double dt, bool want_az,
-                    Illum &out) {
+// Point -> Sun vector of the point p0 (body frame at t_ref) at epoch offset dt, in the body
+// frame at t_ref.  Solves the Sun -> point light time from the frame's seed lts0.  VS is the
+// Sun's barycentric velocity (~0.013 km/s): the contraction factor of the iteration is
+// VS / c ~ 4e-8 and the seed is off by <= R / c, so ONE refinement leaves a Sun-direction
+// error below 1e-18 rad.
+PM_HD V3 sun_vec0(const FrameD &fs, V3 p0, double dt) {
     const PMFrame &f = fs.f;
     const double h = 0.5 * dt * dt;
     // target-centre displacement since t_ref + point offset, body frame at t_ref
@@ -634,10 +680,15 @@ PM_HD void illum_at(const FrameD &fs, V3 p, V3 p0 /* spin_bwd(p) */, V3 e, Rot r
                        fs.S0b[1] - fma(fs.ATb[1], h, fma(fs.VTb[1], dt, p0.y)),
                        fs.S0b[2] - fma(fs.ATb[2], h, fma(fs.VTb[2], dt, p0.z)));
     const V3 VSb = ld3(fs.VSb);
-    V3 sv = axpy(dt, VSb, base);
+    const V3 sv = axpy(dt, VSb, base);
     const double lts = fast_sqrt_pos(dot(sv, sv)) * fs.inv_c;  // the Sun is never at the point
-    sv = axpy(dt - (lts - f.lts0), VSb, base);
-    const V3 s_b = spin_fwd(fs, r, sv);
+    return axpy(dt - (lts - f.lts0), VSb, base);
+}
+// Illumination geometry of body-fixed point p at epoch offset dt (spin r), given the
+// point -> observer vector e (body frame at the epoch).
+PM_HD void illum_at(const FrameD &fs, V3 p, V3 p0 /* spin_bwd(p) */, V3 e, Rot r, double dt, bool want_az,
+                    Illum &out) {
+    const V3 s_b = spin_fwd(fs, r, sun_vec0(fs, p0, dt));
     const V3 n = mul3(p, fs.nw);  // spice.surfnm direction
     illum_angles(n, s_b, e, want_az, out);
 }
@@ -793,7 +844,10 @@ constexpr uint64_t kSkyMask = bit(PM_RA) | bit(PM_DEC) | kKmMask | kLimbMask | k
 // becomes a handful of large basic blocks the scheduler can interleave freely.
 // kRingAll = true keeps ring-plane points hidden behind the body
 // (Body.ring_plane_coordinates(only_visible=False), body.py:2577-2615); the backplanes hide them.
-template <bool kSky, uint64_t kFixedMask = 0, bool kRingAll = false, class Sink>
+// kSpinSym = true is the path for frames with FrameD::spin_sym (the launchers pick it from the flag):
+// the intercept, the illumination angles and the radial velocity are taken in the body frame at t_ref,
+// where they equal the epoch frame's up to the bound of spin_sym, and only LON / LAT spin the point.
+template <bool kSky, uint64_t kFixedMask = 0, bool kRingAll = false, bool kSpinSym = false, class Sink>
 PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, Sink &out) {
     const PMFrame &f = fs.f;
     const double nan = NAN;
@@ -834,7 +888,7 @@ PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, S
     bool on_disc = false;
     Intercept it;
     const V3 u0 = mxv(fs.G, v);  // unit ray, body frame at t_ref
-    if (try_disc) on_disc = sincpt(fs, u0, it);
+    if (try_disc) on_disc = sincpt<kSpinSym>(fs, u0, it);
 
     double v_dist = nan;
     if (on_disc) {
@@ -863,11 +917,14 @@ PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, S
         }
         if (mask & (kIllumMask | kStateMask | kRingMask)) {
             // spkcpt's converged light time is the intercept's own: |X| = |p - o|
-            const V3 kxp = cross(ld3(fs.k), p);  // shared by the inverse spin and omega x p
-            const V3 p0 = spin_bwd_c(fs, it.r, p, kxp);
+            const V3 kxp = cross(ld3(fs.k), kSpinSym ? it.p0 : p);  // shared by the inverse spin and omega x p
+            const V3 p0 = kSpinSym ? it.p0 : spin_bwd_c(fs, it.r, p, kxp);
             if (mask & kIllumMask) {  // _get_illumination_gie_img (body_xy.py:3661-3665)
                 Illum il;
-                illum_at(fs, p, p0, -it.u, it.r, it.dt, (mask & bit(PM_AZIMUTH)) != 0, il);
+                if (kSpinSym)  // the angles of (n, s, e) all spun back to t_ref
+                    illum_angles(mul3(p0, fs.nw), sun_vec0(fs, p0, it.dt), -u0, (mask & bit(PM_AZIMUTH)) != 0, il);
+                else
+                    illum_at(fs, p, p0, -it.u, it.r, it.dt, (mask & bit(PM_AZIMUTH)) != 0, il);
                 if (mask & bit(PM_PHASE)) out.put(PM_PHASE, il.phase * kDpr);
                 if (mask & bit(PM_INCIDENCE)) out.put(PM_INCIDENCE, il.incdnc * kDpr);
                 if (mask & bit(PM_EMISSION)) out.put(PM_EMISSION, il.emissn * kDpr);
@@ -877,9 +934,10 @@ PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, S
             if (mask & bit(PM_DISTANCE)) out.put(PM_DISTANCE, v_dist);
             if (mask & (bit(PM_RADIAL_VELOCITY) | bit(PM_DOPPLER))) {
                 // get_radial_velocity_img (body_xy.py:3898-3913): project on the line of sight - the pixel's
-                // own ray (u0 in the frame of t_ref, it.u at the intercept epoch)
+                // own ray (u0 in the frame of t_ref, it.u at the intercept epoch; the spin about k leaves
+                // (k x p) . u unchanged, so the spin-symmetric path takes both at t_ref)
                 const V3 vt = axpy(it.dt, ld3(fs.ATb), ld3(fs.VTb));
-                const double a = fma(fs.wn, dot(kxp, it.u), dot(vt, u0));
+                const double a = fma(fs.wn, dot(kxp, kSpinSym ? u0 : it.u), dot(vt, u0));
                 const double b = dot(ld3(fs.VOb), u0);
                 const double rv = radial_velocity(fs, a, b);
                 if (mask & bit(PM_RADIAL_VELOCITY)) out.put(PM_RADIAL_VELOCITY, rv);
@@ -915,10 +973,10 @@ PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, S
 // fractional pixel, or one outside the image.  A non-finite x or y never reaches image_pixel -
 // a NaN ray would drive sincpt's light-time iteration, which runs until the epoch stops
 // changing - so it writes NaN to every plane, with PIXEL-X / PIXEL-Y echoing the input.
-template <bool kSky, bool kRingAll, class Sink>
+template <bool kSky, bool kRingAll, bool kSpinSym = false, class Sink>
 PM_HD void image_point(const FrameD &fs, double x, double y, uint64_t mask_in, Sink &out) {
     if (fabs(x) < INFINITY && fabs(y) < INFINITY) {
-        image_pixel<kSky, 0, kRingAll>(fs, x, y, mask_in, out);
+        image_pixel<kSky, 0, kRingAll, kSpinSym>(fs, x, y, mask_in, out);
         return;
     }
 #pragma unroll 1

@@ -11,7 +11,7 @@ CSRC="$ROOT/planetmapper_b200/csrc"
 OUT="$ROOT/variants"; mkdir -p "$OUT/obj_$NAME"
 make -C "$CSRC" -j8 >/dev/null
 OBJS=""
-for o in backplane_kernels proj_kernels gather_kernels smooth_kernels stage_kernels host_ephem capi; do
+for o in backplane_kernels proj_kernels gather_kernels smooth_kernels stage_kernels host_ephem regrid_kernels capi; do
   if echo "$UNITS" | grep -q "$o.cu"; then
     /usr/local/cuda/bin/nvcc -O3 -std=c++17 -lineinfo -gencode arch=compute_100a,code=sm_100a -Xcompiler -fPIC -Xptxas -v \
        $( [ "$o" = backplane_kernels ] && echo -fmad=false ) -DPM_TUNING $FLAGS -c "$CSRC/$o.cu" -o "$OUT/obj_$NAME/$o.o" 2> "$OUT/obj_$NAME/$o.ptxas.log"
