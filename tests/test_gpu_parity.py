@@ -526,7 +526,9 @@ def test_full_grid_gather_properties(L, bc_hst):
     for mode in (L.INTERP_LINEAR, L.INTERP_QUADRATIC, L.INTERP_CUBIC):
         out = L.gather(L.spline_prepare(cube, mode), xm, ym, mode, propagate_nan=True)
         if mode == L.INTERP_CUBIC:
-            # narrow map (row length 40 < 64): 4 x 8 cell blocks per warp, ragged edges, odd row count
+            # sub-maps of 1799 x 40 and 1799 x 37 cells are below 20 cells per image pixel, so they run the scalar
+            # kernel: this compares the 1-D DMMA path of the full grid with it (the 4 x 8 cell blocks of narrow
+            # maps are tested in test_gpu_cubic_gather.py)
             xs, ys = xm[:1799, 1000:1040].contiguous(), ym[:1799, 1000:1040].contiguous()
             sub = L.gather(L.spline_prepare(cube, mode), xs, ys, mode, propagate_nan=True)
             assert torch.equal(torch.nan_to_num(sub, nan=-7.0), torch.nan_to_num(out[:, :1799, 1000:1040], nan=-7.0))
