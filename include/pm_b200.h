@@ -237,6 +237,26 @@ int pm_transform(const PMFrame *frame, int src, int dst, const double *a, const 
                  int64_t *n_missed, void *stream);
 
 /*
+ * Time series: the three point transforms above for n_frames frames in ONE launch (what a fresh
+ * BodyXY per epoch and one xy2lonlat / lonlat2xy / _transform call each do in the reference).
+ * `frames`: n_frames (1 .. 65535) PMFrame structs in DEVICE memory, one per epoch, each packed as the
+ * single-frame call of that epoch would use it (e.g. the altitude-adjusted frame for a lon / lat
+ * destination with alt != 0).  Points: frame f reads a[f * point_stride + i], i < n; point_stride = 0
+ * shares one set of n points between all frames, point_stride >= n gives every frame its own row.
+ * Outputs: [n_frames][n].  n_missed: DEVICE int64[n_frames] (may be NULL), frame f's missed rays in
+ * entry f.  aux13: DEVICE [n_frames][13], row f = pm_transform's aux13_host for frame f, or NULL for
+ * every frame's defaults.  alt must be finite; flags as for the single-frame calls.
+ * Row f of every output equals the single-frame call on frame f bit for bit.
+ */
+int pm_xy2lonlat_batch(const PMFrame *frames, int n_frames, const double *x, const double *y, int64_t n,
+                       int64_t point_stride, double *lon, double *lat, int64_t *n_missed, void *stream);
+int pm_lonlat2xy_batch(const PMFrame *frames, int n_frames, const double *lon, const double *lat, int64_t n,
+                       int64_t point_stride, double alt, uint32_t flags, double *x, double *y, void *stream);
+int pm_transform_batch(const PMFrame *frames, int n_frames, int src, int dst, const double *a, const double *b,
+                       int64_t n, int64_t point_stride, double alt, uint32_t flags, const double *aux13,
+                       double *out_a, double *out_b, int64_t *n_missed, void *stream);
+
+/*
  * Inverse map projections, replacing pyproj.Transformer.transform(...,
  * direction='INVERSE') at body_xy.py:3126 for the three named non-rectangular
  * projections.  params = {a (r_eq), b (r_polar), lon_0, lat_0 (deg), lon_sign}.

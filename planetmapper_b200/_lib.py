@@ -46,6 +46,7 @@ EXPORTED_SYMBOLS = [
     'pm_fits_data_unit_bytes', 'pm_fits_stage', 'pm_backplanes_map_batch', 'pm_gather_paired',
     'pm_host_ssb_state', 'pm_host_orientation', 'pm_backplanes_img_host', 'pm_transform', 'pm_fp64_probe', 'pm_proj_forward',
     'pm_backplanes_points_host', 'pm_regrid_work_bytes', 'pm_regrid_fit', 'pm_gather_regrid',
+    'pm_xy2lonlat_batch', 'pm_lonlat2xy_batch', 'pm_transform_batch',
 ]
 
 
@@ -85,6 +86,12 @@ def load_library() -> ctypes.CDLL:
     lib.pm_xy2lonlat.argtypes = [c_p, c_p, c_p, c_i64, c_p, c_p, c_p, c_p]
     lib.pm_lonlat2xy.argtypes = [c_p, c_p, c_p, c_i64, c_u32, c_p, c_p, c_p]
     lib.pm_lonlat2xy_alt.argtypes = [c_p, c_p, c_p, c_i64, ctypes.c_double, c_u32, c_p, c_p, c_p]
+    lib.pm_xy2lonlat_batch.argtypes = [c_p, c_i, c_p, c_p, c_i64, c_i64, c_p, c_p, c_p, c_p]
+    lib.pm_lonlat2xy_batch.argtypes = [c_p, c_i, c_p, c_p, c_i64, c_i64, ctypes.c_double, c_u32, c_p, c_p, c_p]
+    lib.pm_transform_batch.argtypes = [c_p, c_i, c_i, c_i, c_p, c_p, c_i64, c_i64, ctypes.c_double, c_u32, c_p, c_p,
+                                       c_p, c_p, c_p]
+    for fn in ('pm_xy2lonlat_batch', 'pm_lonlat2xy_batch', 'pm_transform_batch'):
+        getattr(lib, fn).restype = c_i
     lib.pm_proj_inverse.argtypes = [c_i, c_p, c_p, c_p, c_i64, c_p, c_p, c_p]
     lib.pm_proj_forward.argtypes = [c_i, c_p, c_p, c_p, c_i64, c_p, c_p, c_p]
     lib.pm_proj_forward.restype = c_i
@@ -439,6 +446,93 @@ def transform(frame_dev, src: str, dst: str, a_dev, b_dev, *, alt: float = 0.0, 
                           aux.ctypes.data_as(ctypes.c_void_p) if aux is not None else None, oa.data_ptr(),
                           ob.data_ptr(), missed.data_ptr(), _stream_ptr(torch))
     _check(rc, 'pm_transform')
+    return oa, ob, missed
+
+
+# ---- time series: one launch for the points of every frame (pm_*_batch) --------------------------
+MAX_BATCH_FRAMES = 65535   # blockIdx.y of the batched kernels; longer series take one launch per block
+
+
+def _batch_layout(frames_dev, a_dev, b_dev, per_frame: bool):
+    """(n_frames, points per frame, point stride, output shape) of a batched point launch: ``a_dev`` / ``b_dev``
+    are contiguous float64 CUDA tensors, (n_frames,) + point shape when ``per_frame``, else the point shape."""
+    torch = _torch()
+    assert frames_dev.is_cuda and frames_dev.dim() == 2 and frames_dev.shape[1] == 92 and frames_dev.is_contiguous()
+    assert a_dev.shape == b_dev.shape and a_dev.is_contiguous() and b_dev.is_contiguous()
+    assert a_dev.dtype == torch.float64 and b_dev.dtype == torch.float64
+    n_frames = int(frames_dev.shape[0])
+    if per_frame:
+        if a_dev.dim() < 1 or a_dev.shape[0] != n_frames:
+            raise ValueError(f'per-frame points need a leading axis of {n_frames} frames')
+        shape = tuple(a_dev.shape[1:])
+        n = a_dev[0].numel() if n_frames else 0
+        return n_frames, n, n, (n_frames,) + shape
+    shape = tuple(a_dev.shape)
+    return n_frames, a_dev.numel(), 0, (n_frames,) + shape
+
+
+def _blocks(n_frames: int):
+    for first in range(0, n_frames, MAX_BATCH_FRAMES):
+        yield first, min(MAX_BATCH_FRAMES, n_frames - first)
+
+
+def xy2lonlat_batch(frames_dev, x_dev, y_dev, *, per_frame: bool = False):
+    """pm_xy2lonlat_batch: lon / lat (n_frames,) + point shape of every frame of ``frames_dev`` (n_frames, 92), and
+    the (n_frames,) int64 counts of missed rays."""
+    torch = _torch()
+    lib = load_library()
+    n_frames, n, stride, shape = _batch_layout(frames_dev, x_dev, y_dev, per_frame)
+    lon = torch.empty(shape, dtype=torch.float64, device=frames_dev.device)
+    lat = torch.empty_like(lon)
+    missed = torch.zeros(n_frames, dtype=torch.int64, device=frames_dev.device)
+    for f, m in _blocks(n_frames):
+        rc = lib.pm_xy2lonlat_batch(frames_dev[f].data_ptr(), m, x_dev.data_ptr() + 8 * f * stride,
+                                    y_dev.data_ptr() + 8 * f * stride, n, stride, lon.data_ptr() + 8 * f * n,
+                                    lat.data_ptr() + 8 * f * n, missed[f].data_ptr(), _stream_ptr(torch))
+        _check(rc, 'pm_xy2lonlat_batch')
+    return lon, lat, missed
+
+
+def lonlat2xy_batch(frames_dev, lon_dev, lat_dev, *, per_frame: bool = False, not_visible_nan: bool = True,
+                    alt: float = 0.0, planetocentric: bool = False):
+    """pm_lonlat2xy_batch: x / y (n_frames,) + point shape of every frame of ``frames_dev``."""
+    torch = _torch()
+    lib = load_library()
+    n_frames, n, stride, shape = _batch_layout(frames_dev, lon_dev, lat_dev, per_frame)
+    x = torch.empty(shape, dtype=torch.float64, device=frames_dev.device)
+    y = torch.empty_like(x)
+    flags = (FLAG_NOT_VISIBLE_NAN if not_visible_nan else 0) | (FLAG_PLANETOCENTRIC if planetocentric else 0)
+    for f, m in _blocks(n_frames):
+        rc = lib.pm_lonlat2xy_batch(frames_dev[f].data_ptr(), m, lon_dev.data_ptr() + 8 * f * stride,
+                                    lat_dev.data_ptr() + 8 * f * stride, n, stride, float(alt), flags,
+                                    x.data_ptr() + 8 * f * n, y.data_ptr() + 8 * f * n, _stream_ptr(torch))
+        _check(rc, 'pm_lonlat2xy_batch')
+    return x, y
+
+
+def transform_batch(frames_dev, src: str, dst: str, a_dev, b_dev, *, per_frame: bool = False, alt: float = 0.0,
+                    not_visible_nan: bool = False, planetocentric: bool = False, aux13_dev=None):
+    """pm_transform_batch: :func:`transform` for every frame of ``frames_dev``; returns (out_a, out_b) shaped
+    (n_frames,) + point shape and the (n_frames,) int64 miss counts.  ``aux13_dev``: (n_frames, 13) CUDA table,
+    row f = frame f's ``aux13``, or None for every frame's defaults."""
+    torch = _torch()
+    lib = load_library()
+    n_frames, n, stride, shape = _batch_layout(frames_dev, a_dev, b_dev, per_frame)
+    if aux13_dev is not None:
+        assert aux13_dev.is_cuda and aux13_dev.dtype == torch.float64 and aux13_dev.is_contiguous()
+        if tuple(aux13_dev.shape) != (n_frames, 13):
+            raise ValueError(f'aux13 must have shape ({n_frames}, 13)')
+    oa = torch.empty(shape, dtype=torch.float64, device=frames_dev.device)
+    ob = torch.empty_like(oa)
+    missed = torch.zeros(n_frames, dtype=torch.int64, device=frames_dev.device)
+    flags = (FLAG_NOT_VISIBLE_NAN if not_visible_nan else 0) | (FLAG_PLANETOCENTRIC if planetocentric else 0)
+    for f, m in _blocks(n_frames):
+        rc = lib.pm_transform_batch(frames_dev[f].data_ptr(), m, COORD[src], COORD[dst],
+                                    a_dev.data_ptr() + 8 * f * stride, b_dev.data_ptr() + 8 * f * stride, n, stride,
+                                    float(alt), flags, aux13_dev[f].data_ptr() if aux13_dev is not None else None,
+                                    oa.data_ptr() + 8 * f * n, ob.data_ptr() + 8 * f * n, missed[f].data_ptr(),
+                                    _stream_ptr(torch))
+        _check(rc, 'pm_transform_batch')
     return oa, ob, missed
 
 

@@ -182,15 +182,23 @@ __global__ void __launch_bounds__(kBlock, 4) backplanes_map_param_kernel(const _
     map_tile<kFixedMask>(fs, lon_in, lat_in, n, mask, po, out);
 }
 
+// ---------------------------------------------------------------------------------
+// Vectorised point transforms.  The per-point loops are shared by the single-frame kernels and their
+// time-series counterparts (grid (chunks, n_frames), frame blockIdx.y staged by the CTA, as in
+// backplanes_img_kernel): every point of frame f goes through the same device functions with the same
+// staged constants, so row f of a batched launch equals the single-frame launch on frame f bit for bit.
+// ---------------------------------------------------------------------------------
+// Warp-reduced count of missed rays, one atomic per warp that missed
+__device__ __forceinline__ void add_missed(unsigned long long missed, unsigned long long *__restrict__ n_missed) {
+    for (int o = 16; o > 0; o >>= 1) missed += __shfl_down_sync(0xffffffffu, missed, o);
+    if ((threadIdx.x & 31) == 0 && missed) atomicAdd(n_missed, missed);
+}
+
 // BodyXY._xy2lonlat (body_xy.py:482-496) -> Body._obsvec_norm2lonlat (body.py:1058-1081)
-__global__ void __launch_bounds__(kBlock, 4) xy2lonlat_kernel(const PMFrame *__restrict__ frame,
-                                                              const double *__restrict__ xs,
-                                                              const double *__restrict__ ys, int64_t n,
-                                                              double *__restrict__ lon_out,
-                                                              double *__restrict__ lat_out,
-                                                              unsigned long long *__restrict__ n_missed) {
-    __shared__ FrameD fs;
-    load_frame(fs, frame);
+__device__ __forceinline__ unsigned long long xy2lonlat_tile(const FrameD &fs, const double *__restrict__ xs,
+                                                             const double *__restrict__ ys, int64_t n,
+                                                             double *__restrict__ lon_out,
+                                                             double *__restrict__ lat_out) {
     unsigned long long missed = 0;
     const int64_t first = (int64_t)blockIdx.x * (kBlock * kPerThread) + threadIdx.x;
 #pragma unroll 1
@@ -205,21 +213,40 @@ __global__ void __launch_bounds__(kBlock, 4) xy2lonlat_kernel(const PMFrame *__r
         lon_out[idx] = lon;
         lat_out[idx] = lat;
     }
-    if (n_missed) {
-        for (int o = 16; o > 0; o >>= 1) missed += __shfl_down_sync(0xffffffffu, missed, o);
-        if ((threadIdx.x & 31) == 0 && missed) atomicAdd(n_missed, missed);
-    }
+    return missed;
+}
+__global__ void __launch_bounds__(kBlock, 4) xy2lonlat_kernel(const PMFrame *__restrict__ frame,
+                                                              const double *__restrict__ xs,
+                                                              const double *__restrict__ ys, int64_t n,
+                                                              double *__restrict__ lon_out,
+                                                              double *__restrict__ lat_out,
+                                                              unsigned long long *__restrict__ n_missed) {
+    __shared__ FrameD fs;
+    load_frame(fs, frame);
+    const unsigned long long missed = xy2lonlat_tile(fs, xs, ys, n, lon_out, lat_out);
+    if (n_missed) add_missed(missed, n_missed);
+}
+// Time series (pm_xy2lonlat_batch): frame f = blockIdx.y reads its points point_stride doubles after frame
+// f - 1's (0: one set shared by every frame), writes row f of the [n_frames][n] outputs, counts into n_missed[f].
+// Three CTAs per SM: at four the ray / ellipsoid solve needs more than 128 registers and spills.
+__global__ void __launch_bounds__(kBlock, 3) xy2lonlat_batch_kernel(const PMFrame *__restrict__ frames,
+                                                                    const double *__restrict__ xs,
+                                                                    const double *__restrict__ ys, int64_t n,
+                                                                    int64_t point_stride,
+                                                                    double *__restrict__ lon_out,
+                                                                    double *__restrict__ lat_out,
+                                                                    unsigned long long *__restrict__ n_missed) {
+    __shared__ FrameD fs;
+    load_frame(fs, frames + blockIdx.y);
+    const int64_t in = (int64_t)blockIdx.y * point_stride, out = (int64_t)blockIdx.y * n;
+    const unsigned long long missed = xy2lonlat_tile(fs, xs + in, ys + in, n, lon_out + out, lat_out + out);
+    if (n_missed) add_missed(missed, n_missed + blockIdx.y);
 }
 
 // BodyXY._lonlat2xy (body_xy.py:544-560) -> Body._lonlat2obsvec (body.py:1039-1056)
-__global__ void __launch_bounds__(kBlock, 4) lonlat2xy_kernel(const PMFrame *__restrict__ frame,
-                                                              const double *__restrict__ lons,
-                                                              const double *__restrict__ lats, int64_t n,
-                                                              double alt, uint32_t flags,
-                                                              double *__restrict__ x_out,
-                                                              double *__restrict__ y_out) {
-    __shared__ FrameD fs;
-    load_frame(fs, frame);
+__device__ __forceinline__ void lonlat2xy_tile(const FrameD &fs, const double *__restrict__ lons,
+                                               const double *__restrict__ lats, int64_t n, double alt, uint32_t flags,
+                                               double *__restrict__ x_out, double *__restrict__ y_out) {
     const int64_t first = (int64_t)blockIdx.x * (kBlock * kPerThread) + threadIdx.x;
 #pragma unroll 1
     for (int r = 0; r < kPerThread; r++) {
@@ -234,33 +261,44 @@ __global__ void __launch_bounds__(kBlock, 4) lonlat2xy_kernel(const PMFrame *__r
         y_out[idx] = y;
     }
 }
-
-// Generic point transform (pm_transform): any pair of the xy / angular / km / RA-Dec / lon-lat systems
-__global__ void __launch_bounds__(kBlock, 4) transform_kernel(const PMFrame *__restrict__ frame,
-                                                              const __grid_constant__ TransformAux aux, int use_aux,
-                                                              int src, int dst, const double *__restrict__ a_in,
-                                                              const double *__restrict__ b_in, int64_t n, double alt,
-                                                              uint32_t flags, double *__restrict__ a_out,
-                                                              double *__restrict__ b_out,
-                                                              unsigned long long *__restrict__ n_missed) {
+__global__ void __launch_bounds__(kBlock, 4) lonlat2xy_kernel(const PMFrame *__restrict__ frame,
+                                                              const double *__restrict__ lons,
+                                                              const double *__restrict__ lats, int64_t n,
+                                                              double alt, uint32_t flags,
+                                                              double *__restrict__ x_out,
+                                                              double *__restrict__ y_out) {
     __shared__ FrameD fs;
-    __shared__ TransformAux ax;
     load_frame(fs, frame);
-    if (threadIdx.x < 13) {
-        double v;
-        if (use_aux) {
-            v = threadIdx.x < 9 ? aux.Mc[threadIdx.x] : aux.km2ang[threadIdx.x - 9];
-        } else if (threadIdx.x < 9) {
-            v = fs.f.M[threadIdx.x];
-        } else {  // inverse of the frame's angular -> km matrix
-            const double *m = fs.f.ang2km;
-            const double det = fma(m[0], m[3], -m[1] * m[2]);
-            const int k = threadIdx.x - 9;
-            v = (k == 0 ? m[3] : k == 1 ? -m[1] : k == 2 ? -m[2] : m[0]) / det;
-        }
-        (threadIdx.x < 9 ? ax.Mc[threadIdx.x] : ax.km2ang[threadIdx.x - 9]) = v;
-    }
-    __syncthreads();
+    lonlat2xy_tile(fs, lons, lats, n, alt, flags, x_out, y_out);
+}
+// Time series (pm_lonlat2xy_batch): layout as xy2lonlat_batch_kernel
+__global__ void __launch_bounds__(kBlock, 4) lonlat2xy_batch_kernel(const PMFrame *__restrict__ frames,
+                                                                    const double *__restrict__ lons,
+                                                                    const double *__restrict__ lats, int64_t n,
+                                                                    int64_t point_stride, double alt, uint32_t flags,
+                                                                    double *__restrict__ x_out,
+                                                                    double *__restrict__ y_out) {
+    __shared__ FrameD fs;
+    load_frame(fs, frames + blockIdx.y);
+    const int64_t in = (int64_t)blockIdx.y * point_stride, out = (int64_t)blockIdx.y * n;
+    lonlat2xy_tile(fs, lons + in, lats + in, n, alt, flags, x_out + out, y_out + out);
+}
+
+// Generic point transform (pm_transform): any pair of the xy / angular / km / RA-Dec / lon-lat systems.
+// Element k < 13 of the frame's default TransformAux: its obsvec -> angular matrix, then the inverse of its
+// angular -> km matrix
+__device__ __forceinline__ double default_aux(const FrameD &fs, int k) {
+    if (k < 9) return fs.f.M[k];
+    const double *m = fs.f.ang2km;
+    const double det = fma(m[0], m[3], -m[1] * m[2]);
+    k -= 9;
+    return (k == 0 ? m[3] : k == 1 ? -m[1] : k == 2 ? -m[2] : m[0]) / det;
+}
+__device__ __forceinline__ unsigned long long transform_tile(const FrameD &fs, const TransformAux &ax, int src, int dst,
+                                                             const double *__restrict__ a_in,
+                                                             const double *__restrict__ b_in, int64_t n, double alt,
+                                                             uint32_t flags, double *__restrict__ a_out,
+                                                             double *__restrict__ b_out) {
     unsigned long long missed = 0;
     const int64_t first = (int64_t)blockIdx.x * (kBlock * kPerThread) + threadIdx.x;
 #pragma unroll 1
@@ -272,10 +310,49 @@ __global__ void __launch_bounds__(kBlock, 4) transform_kernel(const PMFrame *__r
         a_out[idx] = oa;
         b_out[idx] = ob;
     }
-    if (n_missed) {
-        for (int o = 16; o > 0; o >>= 1) missed += __shfl_down_sync(0xffffffffu, missed, o);
-        if ((threadIdx.x & 31) == 0 && missed) atomicAdd(n_missed, missed);
+    return missed;
+}
+__global__ void __launch_bounds__(kBlock, 4) transform_kernel(const PMFrame *__restrict__ frame,
+                                                              const __grid_constant__ TransformAux aux, int use_aux,
+                                                              int src, int dst, const double *__restrict__ a_in,
+                                                              const double *__restrict__ b_in, int64_t n, double alt,
+                                                              uint32_t flags, double *__restrict__ a_out,
+                                                              double *__restrict__ b_out,
+                                                              unsigned long long *__restrict__ n_missed) {
+    __shared__ FrameD fs;
+    __shared__ TransformAux ax;
+    load_frame(fs, frame);
+    if (threadIdx.x < 13) {
+        const double v = !use_aux ? default_aux(fs, threadIdx.x)
+                                  : threadIdx.x < 9 ? aux.Mc[threadIdx.x] : aux.km2ang[threadIdx.x - 9];
+        (threadIdx.x < 9 ? ax.Mc[threadIdx.x] : ax.km2ang[threadIdx.x - 9]) = v;
     }
+    __syncthreads();
+    const unsigned long long missed = transform_tile(fs, ax, src, dst, a_in, b_in, n, alt, flags, a_out, b_out);
+    if (n_missed) add_missed(missed, n_missed);
+}
+// Time series (pm_transform_batch): layout as xy2lonlat_batch_kernel; aux13 = [n_frames][13] DEVICE table of
+// the frames' TransformAux (row f for frame f), or NULL for every frame's default
+__global__ void __launch_bounds__(kBlock, 4) transform_batch_kernel(const PMFrame *__restrict__ frames,
+                                                                    const double *__restrict__ aux13, int src,
+                                                                    int dst, const double *__restrict__ a_in,
+                                                                    const double *__restrict__ b_in, int64_t n,
+                                                                    int64_t point_stride, double alt, uint32_t flags,
+                                                                    double *__restrict__ a_out,
+                                                                    double *__restrict__ b_out,
+                                                                    unsigned long long *__restrict__ n_missed) {
+    __shared__ FrameD fs;
+    __shared__ TransformAux ax;
+    load_frame(fs, frames + blockIdx.y);
+    if (threadIdx.x < 13) {
+        const double v = aux13 ? aux13[(int64_t)blockIdx.y * 13 + threadIdx.x] : default_aux(fs, threadIdx.x);
+        (threadIdx.x < 9 ? ax.Mc[threadIdx.x] : ax.km2ang[threadIdx.x - 9]) = v;
+    }
+    __syncthreads();
+    const int64_t in = (int64_t)blockIdx.y * point_stride, out = (int64_t)blockIdx.y * n;
+    const unsigned long long missed =
+        transform_tile(fs, ax, src, dst, a_in + in, b_in + in, n, alt, flags, a_out + out, b_out + out);
+    if (n_missed) add_missed(missed, n_missed + blockIdx.y);
 }
 
 // FP64 FMA throughput probes (roofline denominators for the compute-bound kernels): 8 independent
@@ -491,6 +568,31 @@ cudaError_t launch_transform(const PMFrame *frame, int src, int dst, const doubl
     }
     transform_kernel<<<chunks_for(n), kBlock, 0, st>>>(frame, aux, aux13_host != nullptr, src, dst, a, b, n, alt,
                                                        flags, out_a, out_b, n_missed);
+    count_launches(1);
+    return cudaGetLastError();
+}
+cudaError_t launch_xy2lonlat_batch(const PMFrame *frames, int n_frames, const double *x, const double *y, int64_t n,
+                                   int64_t point_stride, double *lon, double *lat, unsigned long long *n_missed,
+                                   cudaStream_t st) {
+    xy2lonlat_batch_kernel<<<dim3(chunks_for(n), (unsigned)n_frames), kBlock, 0, st>>>(frames, x, y, n, point_stride,
+                                                                                       lon, lat, n_missed);
+    count_launches(1);
+    return cudaGetLastError();
+}
+cudaError_t launch_lonlat2xy_batch(const PMFrame *frames, int n_frames, const double *lon, const double *lat,
+                                   int64_t n, int64_t point_stride, double alt, uint32_t flags, double *x, double *y,
+                                   cudaStream_t st) {
+    lonlat2xy_batch_kernel<<<dim3(chunks_for(n), (unsigned)n_frames), kBlock, 0, st>>>(frames, lon, lat, n,
+                                                                                       point_stride, alt, flags, x, y);
+    count_launches(1);
+    return cudaGetLastError();
+}
+cudaError_t launch_transform_batch(const PMFrame *frames, int n_frames, int src, int dst, const double *a,
+                                   const double *b, int64_t n, int64_t point_stride, double alt, uint32_t flags,
+                                   const double *aux13, double *out_a, double *out_b, unsigned long long *n_missed,
+                                   cudaStream_t st) {
+    transform_batch_kernel<<<dim3(chunks_for(n), (unsigned)n_frames), kBlock, 0, st>>>(
+        frames, aux13, src, dst, a, b, n, point_stride, alt, flags, out_a, out_b, n_missed);
     count_launches(1);
     return cudaGetLastError();
 }

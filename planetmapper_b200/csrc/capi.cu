@@ -1,6 +1,7 @@
 // capi.cu - the extern "C" boundary of libpm_b200.so (see include/pm_b200.h).
 // Argument checking, device discovery and launch only: no arithmetic lives here.
 #include <atomic>
+#include <cstdint>
 #include <cstdio>
 
 #include "pm_kernels.h"
@@ -163,6 +164,50 @@ int pm_transform(const PMFrame *frame, int src, int dst, const double *a, const 
     if (sm_count() <= 0) return PM_ERR_NO_DEVICE;
     return check(launch_transform(frame, src, dst, a, b, n, alt, flags, aux13_host, out_a, out_b,
                                   (unsigned long long *)n_missed, (cudaStream_t)stream));
+}
+
+// The time-series entry points check every argument before touching the device
+static bool batch_ok(const PMFrame *frames, int n_frames, int64_t n, int64_t point_stride) {
+    return frames && n_frames > 0 && n_frames <= 65535 && n >= 0 && (point_stride == 0 || point_stride >= n) &&
+           point_stride <= INT64_MAX / 65535;
+}
+static bool finite_alt(double alt) { return alt - alt == 0.0; }
+static bool coords_ok(int src, int dst) {
+    return src >= PM_COORD_XY && src <= PM_COORD_LONLAT && dst >= PM_COORD_XY && dst <= PM_COORD_CENTRIC;
+}
+
+int pm_xy2lonlat_batch(const PMFrame *frames, int n_frames, const double *x, const double *y, int64_t n,
+                       int64_t point_stride, double *lon, double *lat, int64_t *n_missed, void *stream) {
+    if (!batch_ok(frames, n_frames, n, point_stride)) return PM_ERR_BAD_ARG;
+    if (n == 0) return PM_OK;
+    if (!x || !y || !lon || !lat) return PM_ERR_BAD_ARG;
+    if (sm_count() <= 0) return PM_ERR_NO_DEVICE;
+    return check(launch_xy2lonlat_batch(frames, n_frames, x, y, n, point_stride, lon, lat,
+                                        (unsigned long long *)n_missed, (cudaStream_t)stream));
+}
+
+int pm_lonlat2xy_batch(const PMFrame *frames, int n_frames, const double *lon, const double *lat, int64_t n,
+                       int64_t point_stride, double alt, uint32_t flags, double *x, double *y, void *stream) {
+    if (!batch_ok(frames, n_frames, n, point_stride) || !finite_alt(alt)) return PM_ERR_BAD_ARG;
+    if (flags & ~(PM_FLAG_NOT_VISIBLE_NAN | PM_FLAG_PLANETOCENTRIC)) return PM_ERR_BAD_ARG;
+    if (n == 0) return PM_OK;
+    if (!lon || !lat || !x || !y) return PM_ERR_BAD_ARG;
+    if (sm_count() <= 0) return PM_ERR_NO_DEVICE;
+    return check(launch_lonlat2xy_batch(frames, n_frames, lon, lat, n, point_stride, alt, flags, x, y,
+                                        (cudaStream_t)stream));
+}
+
+int pm_transform_batch(const PMFrame *frames, int n_frames, int src, int dst, const double *a, const double *b,
+                       int64_t n, int64_t point_stride, double alt, uint32_t flags, const double *aux13,
+                       double *out_a, double *out_b, int64_t *n_missed, void *stream) {
+    if (!batch_ok(frames, n_frames, n, point_stride) || !finite_alt(alt) || !coords_ok(src, dst)) return PM_ERR_BAD_ARG;
+    if (flags & ~(PM_FLAG_NOT_VISIBLE_NAN | PM_FLAG_PLANETOCENTRIC)) return PM_ERR_BAD_ARG;
+    if (src == dst && src != PM_COORD_LONLAT) return PM_ERR_UNSUPPORTED;
+    if (n == 0) return PM_OK;
+    if (!a || !b || !out_a || !out_b) return PM_ERR_BAD_ARG;
+    if (sm_count() <= 0) return PM_ERR_NO_DEVICE;
+    return check(launch_transform_batch(frames, n_frames, src, dst, a, b, n, point_stride, alt, flags, aux13, out_a,
+                                        out_b, (unsigned long long *)n_missed, (cudaStream_t)stream));
 }
 
 int pm_proj_inverse(int kind, const double *params5_host, const double *xx, const double *yy, int64_t n,

@@ -43,6 +43,18 @@ cudaError_t launch_lonlat2xy(const PMFrame *frame, const double *lon, const doub
 cudaError_t launch_transform(const PMFrame *frame, int src, int dst, const double *a, const double *b, int64_t n,
                              double alt, uint32_t flags, const double *aux13_host, double *out_a, double *out_b,
                              unsigned long long *n_missed, cudaStream_t st);
+// time-series forms of the three above: frame blockIdx.y, points point_stride doubles apart per frame (0 = shared),
+// outputs [n_frames][n], n_missed[n_frames]; aux13: DEVICE [n_frames][13] or NULL
+cudaError_t launch_xy2lonlat_batch(const PMFrame *frames, int n_frames, const double *x, const double *y, int64_t n,
+                                   int64_t point_stride, double *lon, double *lat, unsigned long long *n_missed,
+                                   cudaStream_t st);
+cudaError_t launch_lonlat2xy_batch(const PMFrame *frames, int n_frames, const double *lon, const double *lat,
+                                   int64_t n, int64_t point_stride, double alt, uint32_t flags, double *x, double *y,
+                                   cudaStream_t st);
+cudaError_t launch_transform_batch(const PMFrame *frames, int n_frames, int src, int dst, const double *a,
+                                   const double *b, int64_t n, int64_t point_stride, double alt, uint32_t flags,
+                                   const double *aux13, double *out_a, double *out_b, unsigned long long *n_missed,
+                                   cudaStream_t st);
 cudaError_t launch_fp64_probe(double *scratch, int kind, int iters, int sm_count, cudaStream_t st);
 cudaError_t launch_math_probe(int kind, const double *a, const double *b, int64_t n, double *out,
                               cudaStream_t st);

@@ -15,6 +15,7 @@ provider, and never threads.
 from __future__ import annotations
 
 import atexit
+import math
 import os
 import pickle
 import struct
@@ -27,12 +28,16 @@ from . import frame as F
 from .shard import shard_range
 
 
-def _block(provider, target, observer, ets, disc) -> np.ndarray:
+def _block(provider, target, observer, ets, disc):
+    """Frames (len(ets), 92) and km -> angular matrices (len(ets), 2, 2) of a block of epochs.  A disc value is a
+    scalar shared by every epoch or an array holding one value per epoch of the block."""
     out = np.empty((len(ets), F.PMFRAME_NDOUBLES))
+    k2a = np.empty((len(ets), 2, 2))
     for i, et in enumerate(ets):
         bc = F.build_body_constants(provider, target, None, observer, et=float(et), with_subsol=False)
-        out[i] = F.pack_frame(bc, **disc)
-    return out
+        out[i] = F.pack_frame(bc, **{k: v[i] if isinstance(v, np.ndarray) else v for k, v in disc.items()})
+        k2a[i] = F.km2angular_matrix(bc)
+    return out, k2a
 
 
 # ---- worker processes ---------------------------------------------------------------------
@@ -126,34 +131,57 @@ def default_workers() -> int:
     return max(1, cores // ranks)
 
 
-def build_series_frames(target, ets, observer='EARTH', *, nx: int, ny: int, x0: float, y0: float,
-                        r0: float, rotation_radians: float = 0.0, alt: float = 0.0,
-                        workers: int | None = None, provider=None, kepler: bool = False) -> np.ndarray:
-    """PMFrame constants, shape (len(ets), 92), for ``target`` seen from ``observer`` at the
-    ephemeris times ``ets`` with one set of disc parameters.
+def _disc_value(name: str, value, n: int):
+    """A disc parameter as given (a scalar, shared by every epoch) or as a float64 array of one value per epoch."""
+    arr = np.asarray(value, dtype=np.float64)
+    if arr.ndim == 0:
+        if not np.isfinite(arr):
+            raise ValueError(f'{name} must be finite')
+        return value
+    if arr.shape != (n,):
+        raise ValueError(f'{name} must be a scalar or hold one value per epoch ({n}), not shape {arr.shape}')
+    if not np.all(np.isfinite(arr)):
+        raise ValueError(f'{name} must be finite at every epoch')
+    return np.ascontiguousarray(arr)
 
+
+def build_series_frames(target, ets, observer='EARTH', *, nx: int, ny: int, x0, y0, r0,
+                        rotation_radians=0.0, alt: float = 0.0, workers: int | None = None, provider=None,
+                        kepler: bool = False, with_km2angular: bool = False):
+    """PMFrame constants, shape (len(ets), 92), for ``target`` seen from ``observer`` at the
+    ephemeris times ``ets``.
+
+    ``x0``, ``y0``, ``r0`` and ``rotation_radians`` are each a scalar shared by every epoch or an array of
+    ``len(ets)`` values, one per epoch (pointing drift, ``r0`` following the distance at a fixed plate scale):
+    frame f is ``pack_frame(constants_f, x0=x0[f], ...)``.  ``nx``, ``ny`` and ``alt`` are shared.
     ``workers`` host processes (default: :func:`default_workers`) each take one contiguous
     block of epochs; ``workers <= 1``, a short series, or an explicit in-process ``provider``
     runs serially in this process.  The result does not depend on ``workers``.  ``kepler=True`` answers
     the ephemeris of bodies without SPK coverage from the analytic orbits of ``minispice/kepler.py``
-    (synthetic positions: Europa of BASELINE config C5).
+    (synthetic positions: Europa of BASELINE config C5).  ``with_km2angular=True`` returns
+    ``(frames, km2angular)``, the second the (len(ets), 2, 2) km -> angular matrices of the epochs
+    (Body._get_km2angular_matrix), which :func:`transform` needs for km -> angular in a custom angular frame.
     """
     import planetmapper_b200 as pm
 
     ets = np.asarray(ets, dtype=np.float64).reshape(-1)
-    disc = dict(nx=nx, ny=ny, x0=x0, y0=y0, r0=r0, rotation_radians=rotation_radians, alt=alt)
+    disc = dict(nx=nx, ny=ny, alt=alt)
+    for name, value in (('x0', x0), ('y0', y0), ('r0', r0), ('rotation_radians', rotation_radians)):
+        disc[name] = _disc_value(name, value, len(ets))
     workers = default_workers() if workers is None else int(workers)
     workers = min(workers, max(1, len(ets) // 16))   # a block under ~16 epochs does not pay for the hand-off
     if pm.provider_is_custom():   # an in-process provider cannot be rebuilt inside a worker
         workers = 1
     if provider is not None or workers <= 1:
         prov = provider if provider is not None else pm.get_default_provider()
-        return _block(_with_kepler(prov) if kepler else prov, target, observer, ets, disc)
+        frames, k2a = _block(_with_kepler(prov) if kepler else prov, target, observer, ets, disc)
+        return (frames, k2a) if with_km2angular else frames
     procs = _workers(workers)
     try:
         for w, proc in enumerate(procs):
-            block = ets[slice(*shard_range(len(ets), w, workers))]
-            _send(proc.stdin, (pm._KERNEL_PATH, str(target), str(observer), block, disc, bool(kepler)))
+            part = slice(*shard_range(len(ets), w, workers))
+            block_disc = {k: v[part] if isinstance(v, np.ndarray) else v for k, v in disc.items()}
+            _send(proc.stdin, (pm._KERNEL_PATH, str(target), str(observer), ets[part], block_disc, bool(kepler)))
         replies = [_recv(proc.stdout) for proc in procs]   # every reply is drained before any error is raised
     except BaseException:
         shutdown_pool()   # a dead or half-read worker must not serve the next call
@@ -161,7 +189,10 @@ def build_series_frames(target, ets, observer='EARTH', *, nx: int, ny: int, x0: 
     failed = [payload for status, payload in replies if status != 'ok']
     if failed:
         raise RuntimeError(f'series worker failed: {failed[0]}')
-    return np.concatenate([payload for _, payload in replies], axis=0)
+    frames = np.concatenate([payload[0] for _, payload in replies], axis=0)
+    if with_km2angular:
+        return frames, np.concatenate([payload[1] for _, payload in replies], axis=0)
+    return frames
 
 
 def iter_backplane_batches(frames: np.ndarray, nx: int, ny: int, names, batch: int = 32):
@@ -222,6 +253,133 @@ def map_series(frames: np.ndarray, imgs, nx: int, ny: int, lons, lats, *, interp
         src = cube if mode == L.INTERP_NEAREST else L.spline_prepare(cube, 1)
         L.gather_paired(src, xy[:n, 0], xy[:n, 1], mode, propagate_nan=propagate_nan, out=out[first:first + n])
     return out
+
+
+# ---- point transforms over the epochs of a series -------------------------------------------------
+_SOURCES = ('xy', 'angular', 'km', 'radec', 'lonlat')
+
+
+def frames_at_alt(frames: np.ndarray, alt: float) -> np.ndarray:
+    """The frames of a series (built with ``alt=0``) with the target's radii raised by ``alt`` km: per epoch the
+    radii, ``re``, ``f`` and ``r_eq`` that ``pack_frame(..., alt=alt)`` writes, with the same operations
+    (BodyXY._frame_dev(alt), the reference's _AdjustedSurfaceAltitude).  ``r_cut2``, the image kernels'
+    early-out radius, keeps its value: no point transform reads it."""
+    out = np.array(frames, dtype=np.float64, copy=True)
+    o = F.PMFRAME_OFFSETS
+    radii = out[:, o['radii'][0]:o['radii'][0] + 3] + float(alt)
+    re, rp = radii[:, 0].copy(), radii[:, 2].copy()
+    out[:, o['radii'][0]:o['radii'][0] + 3] = radii
+    out[:, o['re'][0]] = re
+    out[:, o['f'][0]] = (re - rp) / re
+    out[:, o['r_eq'][0]] = re
+    return out
+
+
+def _angular_table(frames, origin_ra, origin_dec, coordinate_rotation, km2angular) -> np.ndarray:
+    """(n_frames, 13) rows of BodyXY._angular_aux, one per epoch: the obsvec -> angular matrix centred on
+    (origin_ra, origin_dec), each defaulting to THAT epoch's target RA / Dec (from its P0, as
+    build_body_constants derives them), then the epoch's km -> angular matrix (NaN when not given: only a
+    km source reads it)."""
+    o = F.PMFRAME_OFFSETS['P0'][0]
+    table = np.full((len(frames), 13), np.nan)
+    for f in range(len(frames)):
+        _, ra, dec = F._recrad(frames[f, o:o + 3])
+        m = F.obsvec2angular_matrix(math.degrees(ra) if origin_ra is None else float(origin_ra),
+                                    math.degrees(dec) if origin_dec is None else float(origin_dec),
+                                    float(coordinate_rotation))
+        table[f, :9] = m.ravel()
+        if km2angular is not None:
+            table[f, 9:] = km2angular[f].ravel()
+    return table
+
+
+def transform(frames, src: str, dst: str, a, b, *, alt: float = 0.0, not_visible_nan: bool = False,
+              not_found_nan: bool = True, planetocentric: bool = False, origin_ra=None, origin_dec=None,
+              coordinate_rotation: float = 0.0, per_frame: bool = False, km2angular=None):
+    """Points (a, b) of coordinate system ``src`` in system ``dst`` at every epoch of a series, in one launch:
+    row f is what ``BodyXY`` with frame f's epoch and disc parameters returns from the matching method
+    (``xy2lonlat``, ``lonlat2xy``, ``xy2radec``, ``km2angular``, ...), bit for bit.
+
+    ``frames``: (n_frames, 92) from :func:`build_series_frames` (``alt=0``).  ``src``: 'xy', 'angular', 'km',
+    'radec' or 'lonlat'; ``dst`` also 'centric' (planetocentric lon / lat, graphic2centric_lonlat);
+    'lonlat' -> 'lonlat' with ``planetocentric=True`` is centric2graphic_lonlat.  ``a`` / ``b`` broadcast like
+    the BodyXY methods' inputs and are shared by every epoch; with ``per_frame=True`` their leading axis is the
+    epoch (e.g. a tracked pixel per frame).  ``alt``, ``not_visible_nan``, ``not_found_nan``, ``planetocentric``
+    and the angular-frame arguments mean what they mean for the BodyXY method; ``origin_ra`` / ``origin_dec``
+    default to each epoch's own target RA / Dec.  km -> angular in a custom angular frame also needs
+    ``km2angular``, the (n_frames, 2, 2) matrices of ``build_series_frames(..., with_km2angular=True)``.
+    ``not_found_nan=False`` raises NotFoundError, naming the first epoch, when a ray misses the target.
+
+    Returns two float64 CUDA tensors shaped (n_frames,) + point shape.
+    """
+    from . import _lib as L
+    from .body_xy import BodyXY, NotFoundError
+
+    frames = np.ascontiguousarray(frames, dtype=np.float64)
+    if frames.ndim != 2 or frames.shape[1] != F.PMFRAME_NDOUBLES or len(frames) == 0:
+        raise ValueError(f'frames must have shape (n_frames, {F.PMFRAME_NDOUBLES}) with n_frames >= 1')
+    n_frames = len(frames)
+    if src not in _SOURCES or dst not in L.COORD:
+        raise ValueError(f'unknown coordinate pair {src!r} -> {dst!r}')
+    if src == dst and src != 'lonlat':
+        raise ValueError(f'{src!r} -> {dst!r} is not a transform')
+    custom_angular = not (origin_ra is None and origin_dec is None and coordinate_rotation == 0.0)
+    if custom_angular and 'angular' not in (src, dst):
+        raise ValueError('origin_ra / origin_dec / coordinate_rotation only apply to the angular system')
+    if custom_angular and src == 'km':
+        if km2angular is None:
+            raise ValueError('km -> angular in a custom angular frame needs the epochs\' km2angular matrices '
+                             '(build_series_frames(..., with_km2angular=True))')
+        km2angular = np.asarray(km2angular, dtype=np.float64)
+        if km2angular.shape != (n_frames, 2, 2):
+            raise ValueError(f'km2angular must have shape ({n_frames}, 2, 2)')
+    aa, bb = np.broadcast_arrays(np.asarray(a, dtype=float), np.asarray(b, dtype=float))
+    if per_frame and (aa.ndim == 0 or aa.shape[0] != n_frames):
+        raise ValueError(f'per_frame points need a leading axis of {n_frames} epochs, not shape {aa.shape}')
+    shape = (n_frames,) + (aa.shape[1:] if per_frame else aa.shape)
+
+    # each public method's own host rules (BodyXY.xy2lonlat / lonlat2xy / _transform)
+    alt = float(alt)
+    xy2lonlat = src == 'xy' and dst == 'lonlat'
+    if xy2lonlat or (not math.isfinite(alt) and dst in ('lonlat', 'centric')):
+        BodyXY._check_alt(alt)
+    if not math.isfinite(alt):   # Body._lonlat2targvec_radians: non-finite alt -> NaN
+        torch = L._torch()
+        nan = torch.full(shape, float('nan'), dtype=torch.float64, device='cuda')
+        return nan, nan.clone()
+    fd = L.to_device(frames)
+    a_dev, b_dev = L.to_device(aa), L.to_device(bb)   # scalars arrive as one point: outputs are reshaped below
+    if xy2lonlat and not planetocentric:
+        fa = L.to_device(frames_at_alt(frames, alt)) if alt != 0.0 else fd
+        lon, lat, missed = L.xy2lonlat_batch(fa, a_dev, b_dev, per_frame=per_frame)
+        if not not_found_nan:
+            n = int(np.prod(shape[1:]))   # BodyXY.xy2lonlat: a missed ray, or NaN at a finite input
+            finite_in = (a_dev.isfinite() & b_dev.isfinite()).reshape(n_frames if per_frame else 1, n)
+            bad = (missed > 0) | (finite_in & lon.reshape(n_frames, n).isnan()).any(dim=1)
+            _raise_first_epoch(bad, NotFoundError)
+        return lon.reshape(shape), lat.reshape(shape)
+    if src == 'lonlat' and dst == 'xy':
+        x, y = L.lonlat2xy_batch(fd, a_dev, b_dev, per_frame=per_frame, not_visible_nan=not_visible_nan, alt=alt,
+                                 planetocentric=planetocentric)
+        return x.reshape(shape), y.reshape(shape)
+    # a lon / lat destination intersects the ellipsoid raised by alt (_AdjustedSurfaceAltitude)
+    if dst in ('lonlat', 'centric') and src != 'lonlat' and alt != 0.0:
+        fd = L.to_device(frames_at_alt(frames, alt))
+    aux = None
+    if custom_angular:
+        aux = L.to_device(_angular_table(frames, origin_ra, origin_dec, coordinate_rotation, km2angular))
+    oa, ob, missed = L.transform_batch(fd, src, dst, a_dev, b_dev, per_frame=per_frame, alt=alt,
+                                       not_visible_nan=not_visible_nan, planetocentric=planetocentric, aux13_dev=aux)
+    if not not_found_nan:
+        _raise_first_epoch(missed > 0, NotFoundError)
+    return oa.reshape(shape), ob.reshape(shape)
+
+
+def _raise_first_epoch(bad, error) -> None:
+    """``error`` naming the first epoch flagged in the (n_frames,) bool CUDA tensor ``bad``."""
+    bad = bad.cpu().numpy()
+    if bad.any():
+        raise error(f'ray does not intercept the target body (epoch {int(np.argmax(bad))})')
 
 
 if __name__ == '__main__':
