@@ -186,6 +186,17 @@ int pm_backplanes_map_host(const PMFrame *frame_host, const double *lon, const d
  *                            (xmaps + l * map_stride): nearest (src = the cube as is) or linear
  *                            (src / nanbits / plane_bits = pm_spline_prepare(degree 1) outputs);
  *                            out: [n_planes][n_cells].  Same arithmetic per cell as pm_gather.
+ *   pm_gather_grouped        map_img / get_mapped_data of one image or cube per epoch: map g (xmaps +
+ *                            g * map_stride, g < n_maps <= 65535) serves planes [g * plane_stride,
+ *                            g * plane_stride + planes_per_map) of an n_planes cube, with every mode of
+ *                            pm_gather (nearest: `src` = the raw cube; spline modes: pm_spline_prepare's
+ *                            three buffers for the whole cube).  out: [n_maps][planes_per_map][n_cells].
+ *                            Group g equals pm_gather of its planes through map g bit for bit, except a
+ *                            cubic group of one plane on a map of >= 20 cells per image pixel, whose sums
+ *                            differ from pm_gather's DMMA order in the last bits.  A plane_stride that is a
+ *                            multiple of 4 (groups start on a plane quad) is the fast layout for
+ *                            planes_per_map > 1; pm_gather_paired is planes_per_map = plane_stride = 1.
+ *                            Empty input (n_maps, planes_per_map or n_cells 0) is valid with NULL pointers.
  */
 int pm_backplanes_map_batch(const PMFrame *frames, int n_frames, const double *lon, const double *lat,
                             int64_t n_cells, uint64_t plane_mask, double *out, void *stream);
@@ -193,6 +204,10 @@ int pm_gather_paired(const double *src, const uint32_t *nanbits, const uint32_t 
                      int n_planes, int ny, int nx, const double *xmaps, const double *ymaps,
                      int64_t map_stride, int64_t n_cells, int mode, uint32_t flags, double *out,
                      void *stream);
+int pm_gather_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits,
+                      int n_planes, int ny, int nx, int n_maps, int planes_per_map, int plane_stride,
+                      const double *xmaps, const double *ymaps, int64_t map_stride, int64_t n_cells,
+                      int mode, uint32_t flags, double *out, void *stream);
 
 /*
  * Vectorised point transforms: replace SpiceBase._maybe_transform_as_arrays

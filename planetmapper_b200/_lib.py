@@ -46,7 +46,7 @@ EXPORTED_SYMBOLS = [
     'pm_fits_data_unit_bytes', 'pm_fits_stage', 'pm_backplanes_map_batch', 'pm_gather_paired',
     'pm_host_ssb_state', 'pm_host_orientation', 'pm_backplanes_img_host', 'pm_transform', 'pm_fp64_probe', 'pm_proj_forward',
     'pm_backplanes_points_host', 'pm_regrid_work_bytes', 'pm_regrid_fit', 'pm_gather_regrid',
-    'pm_xy2lonlat_batch', 'pm_lonlat2xy_batch', 'pm_transform_batch',
+    'pm_xy2lonlat_batch', 'pm_lonlat2xy_batch', 'pm_transform_batch', 'pm_gather_grouped',
 ]
 
 
@@ -131,6 +131,9 @@ def load_library() -> ctypes.CDLL:
     lib.pm_backplanes_map_batch.restype = c_i
     lib.pm_gather_paired.argtypes = [c_p, c_p, c_p, c_i, c_i, c_i, c_p, c_p, c_i64, c_i64, c_i, c_u32, c_p, c_p]
     lib.pm_gather_paired.restype = c_i
+    lib.pm_gather_grouped.argtypes = [c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p, c_p, c_i64, c_i64, c_i, c_u32,
+                                      c_p, c_p]
+    lib.pm_gather_grouped.restype = c_i
     lib.pm_host_ssb_state.argtypes = [c_p, c_i, c_p, c_i, ctypes.c_double, c_p]
     lib.pm_host_ssb_state.restype = c_i
     lib.pm_host_orientation.argtypes = [c_p, ctypes.c_double, c_p, c_p]
@@ -392,6 +395,40 @@ def gather_paired(src, xmaps, ymaps, mode: int, propagate_nan: bool = True, out=
                                 spline.plane_bits.data_ptr() if spline is not None else None, n, ny, nx,
                                 xmaps.data_ptr(), ymaps.data_ptr(), xmaps.stride(0) if n else n_cells, n_cells, mode,
                                 flags, out.data_ptr(), _stream_ptr(torch)), 'pm_gather_paired')
+    return out
+
+
+def gather_grouped(src, xmaps, ymaps, mode: int, planes_per_map: int, plane_stride=None, propagate_nan: bool = True,
+                   out=None):
+    """Map g of ``xmaps`` / ``ymaps`` ((n_maps,) + map shape, possibly strided along axis 0) applied to the planes
+    [g * plane_stride, g * plane_stride + planes_per_map) of ``src`` (a time series of cubes: one cube and one disc
+    position per epoch).  ``src``: the CUDA cube (n, ny, nx) for nearest, the :class:`Spline` of the whole cube,
+    prepared with ``mode``, for the spline modes.  ``plane_stride`` defaults to ``planes_per_map``.  Returns
+    (n_maps, planes_per_map) + map shape."""
+    torch = _torch()
+    lib = load_library()
+    spline = src if isinstance(src, Spline) else None
+    if (mode == INTERP_NEAREST) == (spline is not None) or (spline is not None and spline.degree != mode):
+        raise ValueError('gather_grouped: nearest takes the cube, a spline mode the Spline prepared with that mode')
+    if spline is None and not src.is_contiguous():
+        raise ValueError('gather_grouped: the cube must be contiguous')
+    n, ny, nx = (spline.n_planes, spline.ny, spline.nx) if spline is not None else tuple(src.shape)
+    if xmaps.shape != ymaps.shape or xmaps.stride(0) != ymaps.stride(0):
+        raise ValueError('one x / y map per group, laid out alike')
+    n_maps = xmaps.shape[0]
+    n_cells = xmaps[0].numel() if n_maps else 0
+    if n_maps and not (xmaps[0].is_contiguous() and ymaps[0].is_contiguous()):
+        raise ValueError('each map must be contiguous')
+    plane_stride = planes_per_map if plane_stride is None else plane_stride
+    if out is None:
+        out = torch.empty((n_maps, planes_per_map) + tuple(xmaps.shape[1:]), dtype=torch.float64, device=xmaps.device)
+    flags = FLAG_PROPAGATE_NAN if propagate_nan else 0
+    data = spline.coef if spline is not None else src
+    _check(lib.pm_gather_grouped(data.data_ptr(), spline.nanbits.data_ptr() if spline is not None else None,
+                                 spline.plane_bits.data_ptr() if spline is not None else None, n, ny, nx, n_maps,
+                                 planes_per_map, plane_stride, xmaps.data_ptr(), ymaps.data_ptr(),
+                                 xmaps.stride(0) if n_maps else n_cells, n_cells, mode, flags, out.data_ptr(),
+                                 _stream_ptr(torch)), 'pm_gather_grouped')
     return out
 
 

@@ -123,8 +123,38 @@ int pm_gather_paired(const double *src, const uint32_t *nanbits, const uint32_t 
     if (!src || !xmaps || !ymaps || !out) return PM_ERR_BAD_ARG;
     if (mode == PM_INTERP_LINEAR && (!nanbits || !plane_bits || nx < 2 || ny < 2)) return PM_ERR_BAD_ARG;
     if (n_planes > 65535) return PM_ERR_BAD_ARG;
-    return check(launch_gather_paired(src, nanbits, plane_bits, n_planes, ny, nx, xmaps, ymaps, map_stride, n_cells,
-                                      mode, flags, out, (cudaStream_t)stream));
+    return check(launch_gather_grouped(src, nanbits, plane_bits, n_planes, ny, nx, n_planes, 1, 1, xmaps, ymaps,
+                                       map_stride, n_cells, mode, flags, out, 0, (cudaStream_t)stream));
+}
+
+int pm_gather_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes, int ny,
+                      int nx, int n_maps, int planes_per_map, int plane_stride, const double *xmaps,
+                      const double *ymaps, int64_t map_stride, int64_t n_cells, int mode, uint32_t flags, double *out,
+                      void *stream) {
+    if (n_planes < 0 || ny <= 0 || nx <= 0 || n_maps < 0 || n_maps > 65535 || planes_per_map < 0 ||
+        plane_stride < planes_per_map || n_cells < 0 || map_stride < n_cells)
+        return PM_ERR_BAD_ARG;
+    const bool empty = n_maps == 0 || planes_per_map == 0 || n_cells == 0;  // valid, with null pointers
+    if (!empty && (int64_t)(n_maps - 1) * plane_stride + planes_per_map > n_planes) return PM_ERR_BAD_ARG;
+    if (!empty && map_stride > INT64_MAX / n_maps) return PM_ERR_BAD_ARG;
+    int ky = mode, kx = mode;
+    if (mode & PM_INTERP_MIXED) {
+        ky = (mode >> 4) & 0xF;
+        kx = mode & 0xF;
+        if ((mode & ~0x1FF) || ky < 1 || ky > 3 || kx < 1 || kx > 3) return PM_ERR_UNSUPPORTED;
+    } else if (mode < PM_INTERP_NEAREST || mode > PM_INTERP_CUBIC) {
+        return PM_ERR_UNSUPPORTED;
+    }
+    if (mode != PM_INTERP_NEAREST && (nx <= kx || ny <= ky)) return PM_ERR_BAD_ARG;
+    if (empty) return PM_OK;
+    if (!src || !xmaps || !ymaps || !out) return PM_ERR_BAD_ARG;
+    if (mode != PM_INTERP_NEAREST && (!nanbits || !plane_bits)) return PM_ERR_BAD_ARG;
+    if (planes_per_map > 65535 * 128) return PM_ERR_BAD_ARG;
+    int sms = sm_count();
+    if (sms <= 0) return PM_ERR_NO_DEVICE;
+    return check(launch_gather_grouped(src, nanbits, plane_bits, n_planes, ny, nx, n_maps, planes_per_map,
+                                       plane_stride, xmaps, ymaps, map_stride, n_cells, mode, flags, out, sms,
+                                       (cudaStream_t)stream));
 }
 
 int pm_xy2lonlat(const PMFrame *frame, const double *x, const double *y, int64_t n, double *lon, double *lat,

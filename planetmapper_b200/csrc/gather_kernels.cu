@@ -77,14 +77,11 @@ __host__ __device__ __forceinline__ int bspline3_weights(double x, int n, double
 // ---------------------------------------------------------------------------------
 // nearest neighbour: reads the raw cube [n_planes][ny][nx]
 // ---------------------------------------------------------------------------------
-__global__ void __launch_bounds__(kGatherBlock)
-    gather_nearest_kernel(const double *__restrict__ cube, int ny, int nx, int plane_begin, int plane_count,
-                          const double *__restrict__ xmap, const double *__restrict__ ymap, int64_t n_cells,
-                          double *__restrict__ out, int planes_per_group) {
-    const int64_t cell = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (cell >= n_cells) return;
-    const int l0 = blockIdx.y * planes_per_group;
-    const int l1 = min(l0 + planes_per_group, plane_count);
+// Planes plane_begin + [l0, l1) at map cell `cell` into out[l][cell]
+__device__ __forceinline__ void nearest_cell_planes(const double *__restrict__ cube, int ny, int nx, int plane_begin,
+                                                    int l0, int l1, const double *__restrict__ xmap,
+                                                    const double *__restrict__ ymap, int64_t cell, int64_t n_cells,
+                                                    double *__restrict__ out) {
     const int64_t plane_px = (int64_t)ny * nx;
     const double x = __ldg(xmap + cell), y = __ldg(ymap + cell);
     const double nan = NAN;
@@ -121,6 +118,16 @@ __global__ void __launch_bounds__(kGatherBlock)
         src += plane_px;
         dst += n_cells;
     }
+}
+__global__ void __launch_bounds__(kGatherBlock)
+    gather_nearest_kernel(const double *__restrict__ cube, int ny, int nx, int plane_begin, int plane_count,
+                          const double *__restrict__ xmap, const double *__restrict__ ymap, int64_t n_cells,
+                          double *__restrict__ out, int planes_per_group) {
+    const int64_t cell = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (cell >= n_cells) return;
+    const int l0 = blockIdx.y * planes_per_group;
+    const int l1 = min(l0 + planes_per_group, plane_count);
+    nearest_cell_planes(cube, ny, nx, plane_begin, l0, l1, xmap, ymap, cell, n_cells, out);
 }
 
 // ---------------------------------------------------------------------------------
@@ -203,21 +210,15 @@ __device__ __forceinline__ void setup_cell(CellState<KY, KX> &c, double x, doubl
     }
 }
 
-// One cell per thread, KY x KX footprint (KY = row degree + 1, KX = column degree + 1)
-template <int KY, int KX, int kMinBlocks>
-__global__ void __launch_bounds__(kGatherBlock, kMinBlocks)
-    gather_spline_kernel(const double *__restrict__ coefq, const uint32_t *__restrict__ nanbits,
-                         const uint32_t *__restrict__ plane_bits, int n_words, int ny, int nx, int plane_begin,
-                         int plane_count, const double *__restrict__ xmap, const double *__restrict__ ymap,
-                         int64_t n_cells, uint32_t flags, double *__restrict__ out, int planes_per_group) {
-    const int64_t cell = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (cell >= n_cells) return;
-    const int l0 = blockIdx.y * planes_per_group;  // relative to plane_begin, multiple of 4
-    const int l1 = min(l0 + planes_per_group, plane_count);
+// Planes plane_begin + [l0, l1) of one prepared cell, a plane quad at a time (plane_begin + l0 a multiple
+// of 4), into out[l][cell]
+template <int KY, int KX>
+__device__ __forceinline__ void spline_cell_quads(CellState<KY, KX> &cs, const double *__restrict__ coefq,
+                                                  const uint32_t *__restrict__ nanbits,
+                                                  const uint32_t *__restrict__ plane_bits, int n_words, int ny,
+                                                  int nx, int plane_begin, int l0, int l1, bool propagate,
+                                                  int64_t cell, int64_t n_cells, double *__restrict__ out) {
     const double nan = NAN;
-    const bool propagate = (flags & PM_FLAG_PROPAGATE_NAN) != 0;
-    CellState<KY, KX> cs;
-    setup_cell<KY, KX>(cs, __ldg(xmap + cell), __ldg(ymap + cell), ny, nx, propagate);
     const int64_t quad_stride = (int64_t)ny * nx * 4;  // doubles per plane quad
     const int64_t row_stride = (int64_t)nx * 4;
     const double *src = coefq + (int64_t)((plane_begin + l0) >> 2) * quad_stride + cs.origin;
@@ -257,6 +258,49 @@ __global__ void __launch_bounds__(kGatherBlock, kMinBlocks)
         src += quad_stride;
         dst += 4 * n_cells;
     }
+}
+
+// Plane gl (any index) of one prepared cell, read from its lane of the plane quad: per plane the same loads,
+// FMAs (rows outer) and NaN words as spline_cell_quads, so the two agree bit for bit
+template <int KY, int KX>
+__device__ __forceinline__ double spline_cell_plane(const CellState<KY, KX> &cs, const double *__restrict__ coefq,
+                                                    const uint32_t *__restrict__ nanbits,
+                                                    const uint32_t *__restrict__ plane_bits, int n_words, int ny,
+                                                    int nx, int gl, bool propagate) {
+    if (!cs.valid) return NAN;
+    const int word = gl >> 5;
+    uint32_t bad = __ldg(plane_bits + word);
+    if (propagate && __ldg(plane_bits + n_words + word)) {
+#pragma unroll
+        for (int k = 0; k < 4; k++) bad |= __ldg(nanbits + (int64_t)cs.nb[k] * n_words + word);
+    }
+    if ((bad >> (gl & 31)) & 1u) return NAN;
+    const int64_t row_stride = (int64_t)nx * 4;
+    const double *p = coefq + (int64_t)(gl >> 2) * ny * row_stride + cs.origin + (gl & 3);
+    double acc = 0.0;
+#pragma unroll
+    for (int a = 0; a < KY; a++)
+#pragma unroll
+        for (int b = 0; b < KX; b++) acc = fma(__ldg(p + a * row_stride + b * 4), cs.w[a * KX + b], acc);
+    return acc;
+}
+
+// One cell per thread, KY x KX footprint (KY = row degree + 1, KX = column degree + 1)
+template <int KY, int KX, int kMinBlocks>
+__global__ void __launch_bounds__(kGatherBlock, kMinBlocks)
+    gather_spline_kernel(const double *__restrict__ coefq, const uint32_t *__restrict__ nanbits,
+                         const uint32_t *__restrict__ plane_bits, int n_words, int ny, int nx, int plane_begin,
+                         int plane_count, const double *__restrict__ xmap, const double *__restrict__ ymap,
+                         int64_t n_cells, uint32_t flags, double *__restrict__ out, int planes_per_group) {
+    const int64_t cell = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (cell >= n_cells) return;
+    const int l0 = blockIdx.y * planes_per_group;  // relative to plane_begin, multiple of 4
+    const int l1 = min(l0 + planes_per_group, plane_count);
+    const bool propagate = (flags & PM_FLAG_PROPAGATE_NAN) != 0;
+    CellState<KY, KX> cs;
+    setup_cell<KY, KX>(cs, __ldg(xmap + cell), __ldg(ymap + cell), ny, nx, propagate);
+    spline_cell_quads<KY, KX>(cs, coefq, nanbits, plane_bits, n_words, ny, nx, plane_begin, l0, l1, propagate, cell,
+                              n_cells, out);
 }
 
 // ---------------------------------------------------------------------------------
@@ -755,69 +799,61 @@ __global__ void __launch_bounds__(kCubicBlock, PM_CUBIC_CTAS)
 }
 
 // ---------------------------------------------------------------------------------
-// Paired gather for a time series: plane l of the cube is mapped with its own x / y map
-// (pm_gather_paired).  One thread per (plane, cell); per cell the same arithmetic, in the same
-// order, as gather_nearest_kernel / gather_spline_kernel<2, 2>, so results are bit-identical to
-// n_planes single-plane pm_gather calls.  Each voxel reads one (nearest) or four (linear) cube
-// values that neighbouring threads share through L1 / L2; the store is coalesced.
+// Grouped gather for a time series (pm_gather_grouped): map g of n_maps serves the planes
+// [g * plane_stride, g * plane_stride + planes_per_map) of the cube; out [n_maps][planes_per_map][n_cells].
+// Grid (cell blocks, map, plane group).  Per cell the weights and NaN-test pixels are set up once for the
+// map and reused for every plane of the group, and every voxel takes the arithmetic of gather_nearest_kernel /
+// gather_spline_kernel, so a group equals pm_gather of the same planes through the same map bit for bit.
+// kQuads: groups start on a plane quad (plane_stride a multiple of 4) and are read a quad per 32-byte load;
+// otherwise every plane is read from its lane of the quad (one image per epoch packed four to a quad:
+// planes_per_map = plane_stride = 1, which is pm_gather_paired).
 // ---------------------------------------------------------------------------------
-template <bool kLinear>
 __global__ void __launch_bounds__(kGatherBlock)
-    gather_paired_kernel(const double *__restrict__ src, const uint32_t *__restrict__ nanbits,
-                         const uint32_t *__restrict__ plane_bits, int n_words, int ny, int nx,
-                         const double *__restrict__ xmaps, const double *__restrict__ ymaps, int64_t map_stride,
-                         int64_t n_cells, uint32_t flags, double *__restrict__ out) {
+    gather_grouped_nearest_kernel(const double *__restrict__ cube, int ny, int nx, int planes_per_map,
+                                  int plane_stride, const double *__restrict__ xmaps, const double *__restrict__ ymaps,
+                                  int64_t map_stride, int64_t n_cells, double *__restrict__ out, int planes_per_group) {
     const int64_t cell = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (cell >= n_cells) return;
-    const int l = blockIdx.y;
-    const double x = __ldg(xmaps + (int64_t)l * map_stride + cell), y = __ldg(ymaps + (int64_t)l * map_stride + cell);
-    double v = NAN;
-    if (!kLinear) {
-        if (!isnan(x)) {
-            long xi = (long)rint(x), yi = isnan(y) ? -999 : (long)rint(y);
-            if (xi < 0) xi += nx;
-            if (yi < 0) yi += ny;
-            if (xi >= 0 && xi < nx && yi >= 0 && yi < ny) v = __ldg(src + ((int64_t)l * ny + yi) * nx + xi);
-        }
-    } else {
-        const bool propagate = (flags & PM_FLAG_PROPAGATE_NAN) != 0;
-        CellState<2, 2> cs;
-        setup_cell<2, 2>(cs, x, y, ny, nx, propagate);
-        if (cs.valid) {
-            const int word = l >> 5;
-            uint32_t bad = __ldg(plane_bits + word);
-            if (propagate && __ldg(plane_bits + n_words + word)) {
-#pragma unroll
-                for (int k = 0; k < 4; k++) bad |= __ldg(nanbits + (int64_t)cs.nb[k] * n_words + word);
-            }
-            if (!((bad >> (l & 31)) & 1u)) {
-                const int64_t row_stride = (int64_t)nx * 4;
-                const double *p = src + (int64_t)(l >> 2) * ny * row_stride + cs.origin + (l & 3);
-                double acc = 0.0;
-#pragma unroll
-                for (int a = 0; a < 2; a++)
-#pragma unroll
-                    for (int b = 0; b < 2; b++) acc = fma(__ldg(p + a * row_stride + b * 4), cs.w[a * 2 + b], acc);
-                v = acc;
-            }
-        }
-    }
-    __stcs(out + (int64_t)l * n_cells + cell, v);
+    const int g = blockIdx.y;
+    const int l0 = blockIdx.z * planes_per_group;
+    const int l1 = min(l0 + planes_per_group, planes_per_map);
+    nearest_cell_planes(cube, ny, nx, g * plane_stride, l0, l1, xmaps + (int64_t)g * map_stride,
+                        ymaps + (int64_t)g * map_stride, cell, n_cells, out + (int64_t)g * planes_per_map * n_cells);
 }
 
-cudaError_t launch_gather_paired(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes,
-                                 int ny, int nx, const double *xmaps, const double *ymaps, int64_t map_stride,
-                                 int64_t n_cells, int mode, uint32_t flags, double *out, cudaStream_t st) {
-    const dim3 grid((unsigned)((n_cells + kGatherBlock - 1) / kGatherBlock), (unsigned)n_planes);
-    const int n_words = (n_planes + 31) / 32;
-    if (mode == PM_INTERP_LINEAR)
-        gather_paired_kernel<true><<<grid, kGatherBlock, 0, st>>>(src, nanbits, plane_bits, n_words, ny, nx, xmaps, ymaps,
-                                                                   map_stride, n_cells, flags, out);
-    else
-        gather_paired_kernel<false><<<grid, kGatherBlock, 0, st>>>(src, nanbits, plane_bits, n_words, ny, nx, xmaps,
-                                                                    ymaps, map_stride, n_cells, flags, out);
-    count_launches(1);
-    return cudaGetLastError();
+template <int KY, int KX, bool kQuads, int kMinBlocks>
+__global__ void __launch_bounds__(kGatherBlock, kMinBlocks)
+    gather_grouped_kernel(const double *__restrict__ coefq, const uint32_t *__restrict__ nanbits,
+                          const uint32_t *__restrict__ plane_bits, int n_words, int ny, int nx, int planes_per_map,
+                          int plane_stride, const double *__restrict__ xmaps, const double *__restrict__ ymaps,
+                          int64_t map_stride, int64_t n_cells, uint32_t flags, double *__restrict__ out,
+                          int planes_per_group) {
+    const int64_t cell = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (cell >= n_cells) return;
+    const int g = blockIdx.y;
+    const int l0 = blockIdx.z * planes_per_group;  // multiple of 4
+    const int l1 = min(l0 + planes_per_group, planes_per_map);
+    const bool propagate = (flags & PM_FLAG_PROPAGATE_NAN) != 0;
+    const int64_t m = (int64_t)g * map_stride + cell;
+    CellState<KY, KX> cs;
+    setup_cell<KY, KX>(cs, __ldg(xmaps + m), __ldg(ymaps + m), ny, nx, propagate);
+    out += (int64_t)g * planes_per_map * n_cells;
+    if (kQuads) {
+        spline_cell_quads<KY, KX>(cs, coefq, nanbits, plane_bits, n_words, ny, nx, g * plane_stride, l0, l1,
+                                  propagate, cell, n_cells, out);
+    } else {
+        double *dst = out + (int64_t)l0 * n_cells + cell;
+        for (int l = l0; l < l1; l++, dst += n_cells)
+            __stcs(dst, spline_cell_plane<KY, KX>(cs, coefq, nanbits, plane_bits, n_words, ny, nx,
+                                                  g * plane_stride + l, propagate));
+    }
+}
+
+// launch_gather's switch to the DMMA kernel for cubic: many map cells per image pixel share a footprint.
+// Measured crossover with the one-cell-per-thread kernel (tools/probe_density.py): ~16 map cells per image
+// pixel - at 15.8 the scalar kernel is 10 % faster, at 63 the DMMA kernel 1.5x, at 400 (BASELINE C4) 2x
+static bool dense_map(int64_t n_cells, int ny, int nx) {
+    return n_cells >= (int64_t)20 * nx * ny && nx < 16384 && ny < 16384;
 }
 
 cudaError_t launch_gather(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes,
@@ -848,10 +884,8 @@ cudaError_t launch_gather(const double *src, const uint32_t *nanbits, const uint
                                                                     plane_begin, plane_count, xmap, ymap, n_cells, \
                                                                     flags, out, ppg)
     static const int v = tune_int("PM_CUBIC_VARIANT", -1);
-    // dense maps (many cells per image pixel share a footprint): warp-tiled DMMA kernel.  Measured crossover
-    // with the one-cell-per-thread kernel (tools/probe_density.py): ~16 map cells per image pixel - at 15.8 the
-    // scalar kernel is 10 % faster, at 63 the DMMA kernel 1.5x, at 400 (BASELINE C4) 2x
-    const bool dense = n_cells >= (int64_t)20 * nx * ny && nx < 16384 && ny < 16384;
+    // dense maps (many cells per image pixel share a footprint): warp-tiled DMMA kernel
+    const bool dense = dense_map(n_cells, ny, nx);
     if (ky == 3 && kx == 3 && v != 0 && (dense || v > 0)) {
         // larger plane groups: the per-warp setup (map loads, weights, footprint classes) is heavier here
         // than in the scalar kernel
@@ -888,6 +922,70 @@ cudaError_t launch_gather(const double *src, const uint32_t *nanbits, const uint
         }
     }
 #undef PM_SPLINE
+    count_launches(1);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_gather_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes,
+                                  int ny, int nx, int n_maps, int planes_per_map, int plane_stride, const double *xmaps,
+                                  const double *ymaps, int64_t map_stride, int64_t n_cells, int mode, uint32_t flags,
+                                  double *out, int sm_count, cudaStream_t st) {
+    if (n_maps == 0 || planes_per_map == 0 || n_cells == 0) return cudaSuccess;
+    int ppg = 128;  // planes per CTA, as launch_gather
+    if (planes_per_map < ppg) ppg = (planes_per_map + 3) / 4 * 4;
+    const dim3 grid((unsigned)((n_cells + kGatherBlock - 1) / kGatherBlock), (unsigned)n_maps,
+                    (unsigned)((planes_per_map + ppg - 1) / ppg));
+    if (mode == PM_INTERP_NEAREST) {
+        gather_grouped_nearest_kernel<<<grid, kGatherBlock, 0, st>>>(src, ny, nx, planes_per_map, plane_stride, xmaps,
+                                                                     ymaps, map_stride, n_cells, out, ppg);
+        count_launches(1);
+        return cudaGetLastError();
+    }
+    int ky = mode, kx = mode;
+    if (mode & PM_INTERP_MIXED) {
+        ky = (mode >> 4) & 0xF;
+        kx = mode & 0xF;
+    }
+    if (ky < 1 || ky > 3 || kx < 1 || kx > 3) return cudaErrorInvalidValue;
+    const bool quads = planes_per_map > 1 && plane_stride % 4 == 0;
+    if (ky == 3 && kx == 3 && quads && dense_map(n_cells, ny, nx)) {
+        // a cube per map on a dense map: pm_gather's own DMMA launch per map, so each group is its result bit
+        // for bit (plane_begin = g * plane_stride is a multiple of 4)
+        for (int g = 0; g < n_maps; g++) {
+            const cudaError_t e = launch_gather(src, nanbits, plane_bits, n_planes, ny, nx, g * plane_stride,
+                                                planes_per_map, xmaps + (int64_t)g * map_stride,
+                                                ymaps + (int64_t)g * map_stride, n_cells, 0, mode, flags,
+                                                out + (int64_t)g * planes_per_map * n_cells, sm_count, st);
+            if (e != cudaSuccess) return e;
+        }
+        return cudaSuccess;
+    }
+    const int n_words = (n_planes + 31) / 32;
+    // CTAs per SM (quad form, plane-by-plane form): the most at which each instantiation compiles without spills
+    // (ptxas -v); the quad form carries the group indexing on top of gather_spline_kernel's state
+#define PM_GROUPED(KY, KX, MBQ, MB)                                                                                    \
+    do {                                                                                                            \
+        if (quads)                                                                                                  \
+            gather_grouped_kernel<KY, KX, true, MBQ><<<grid, kGatherBlock, 0, st>>>(                                 \
+                src, nanbits, plane_bits, n_words, ny, nx, planes_per_map, plane_stride, xmaps, ymaps, map_stride,  \
+                n_cells, flags, out, ppg);                                                                          \
+        else                                                                                                        \
+            gather_grouped_kernel<KY, KX, false, MB><<<grid, kGatherBlock, 0, st>>>(                                \
+                src, nanbits, plane_bits, n_words, ny, nx, planes_per_map, plane_stride, xmaps, ymaps, map_stride,  \
+                n_cells, flags, out, ppg);                                                                          \
+    } while (0)
+    switch (ky * 4 + kx) {
+        case 1 * 4 + 1: PM_GROUPED(2, 2, 4, 6); break;
+        case 1 * 4 + 2: PM_GROUPED(2, 3, 3, 3); break;
+        case 1 * 4 + 3: PM_GROUPED(2, 4, 2, 3); break;
+        case 2 * 4 + 1: PM_GROUPED(3, 2, 2, 3); break;
+        case 2 * 4 + 2: PM_GROUPED(3, 3, 2, 3); break;
+        case 2 * 4 + 3: PM_GROUPED(3, 4, 2, 2); break;
+        case 3 * 4 + 1: PM_GROUPED(4, 2, 2, 3); break;
+        case 3 * 4 + 2: PM_GROUPED(4, 3, 2, 2); break;
+        default: PM_GROUPED(4, 4, 2, 2); break;
+    }
+#undef PM_GROUPED
     count_launches(1);
     return cudaGetLastError();
 }

@@ -70,9 +70,12 @@ cudaError_t launch_gather(const double *src, const uint32_t *nanbits, const uint
                           int64_t n_cells, int64_t cells_per_row, int mode, uint32_t flags, double *out, int sm_count,
                           cudaStream_t st);
 
-cudaError_t launch_gather_paired(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes,
-                                 int ny, int nx, const double *xmaps, const double *ymaps, int64_t map_stride,
-                                 int64_t n_cells, int mode, uint32_t flags, double *out, cudaStream_t st);
+// time series: map g serves planes [g * plane_stride, g * plane_stride + planes_per_map); pm_gather_paired is
+// planes_per_map = plane_stride = 1
+cudaError_t launch_gather_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes,
+                                  int ny, int nx, int n_maps, int planes_per_map, int plane_stride, const double *xmaps,
+                                  const double *ymaps, int64_t map_stride, int64_t n_cells, int mode, uint32_t flags,
+                                  double *out, int sm_count, cudaStream_t st);
 
 int64_t spline_coef_bytes(int n_planes, int ny, int nx);
 int64_t spline_nanbits_bytes(int n_planes, int ny, int nx);

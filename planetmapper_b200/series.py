@@ -227,7 +227,8 @@ def map_series(frames: np.ndarray, imgs, nx: int, ny: int, lons, lats, *, interp
 
     ``imgs``: (n_frames, ny, nx) array or CUDA tensor; ``lons`` / ``lats``: the map grid (degrees,
     e.g. from ``generate_map_coordinates``); ``interpolation``: 'nearest' or 'linear'.  Returns a CUDA
-    tensor (n_frames,) + grid shape (``out`` if given).
+    tensor (n_frames,) + grid shape (``out`` if given).  :func:`iter_mapped_series` maps with every
+    interpolating spline degree, and a cube per epoch.
     """
     from . import _lib as L
 
@@ -253,6 +254,106 @@ def map_series(frames: np.ndarray, imgs, nx: int, ny: int, lons, lats, *, interp
         src = cube if mode == L.INTERP_NEAREST else L.spline_prepare(cube, 1)
         L.gather_paired(src, xy[:n, 0], xy[:n, 1], mode, propagate_nan=propagate_nan, out=out[first:first + n])
     return out
+
+
+SERIES_MEMORY_SHARE = 0.4   # of the free device memory, for a batch's cubes, prepared operand, maps and output
+
+
+def iter_mapped_series(frames: np.ndarray, cubes, nx: int, ny: int, lons, lats, *, interpolation='linear',
+                       spline_smoothing: float = 0, propagate_nan: bool = True, batch: int | None = None):
+    """``Observation(data=cube_f, ...).get_mapped_data(interpolation)`` (``BodyXY.map_img`` for an image) for every
+    epoch f of a series, each with frame f's own geometry and disc, in batches of epochs.
+
+    ``cubes``: (n_frames, nλ, ny, nx) or (n_frames, ny, nx) (one image per epoch), a numpy array or a CUDA
+    tensor; host input is uploaded one batch at a time.  ``lons`` / ``lats``: the map grid shared by every epoch
+    (degrees, e.g. from ``generate_map_coordinates``).  ``interpolation``: everything map_img accepts without
+    smoothing ('nearest', 'linear', 'quadratic', 'cubic', a degree 1..3 or a (k_rows, k_cols) pair), with
+    map_img's errors; 'smooth' and ``spline_smoothing != 0`` raise NotImplementedError.
+
+    Yields ``(first, mapped)``: ``mapped`` is a CUDA tensor (n, nλ) + grid shape ((n,) + grid shape for 3-D
+    input) holding epochs first .. first + n, equal to the single-epoch call bit for bit.  The tensor is REUSED
+    by the next iteration: consume or copy it before advancing.  Per batch: one launch for every epoch's x / y
+    map, one spline preparation of the whole batch and one grouped gather (a cube series of cubic maps with
+    >= 20 map cells per image pixel: pm_gather's dense-map kernel once per epoch).  ``batch`` (epochs per batch)
+    defaults to what keeps a batch within SERIES_MEMORY_SHARE of the free device memory.
+    """
+    from .body_xy import _interpolation_mode
+
+    if interpolation == 'smooth' or spline_smoothing != 0:
+        raise NotImplementedError("iter_mapped_series: 'smooth' and smoothing splines (spline_smoothing != 0) fit "
+                                  'per-epoch grids; map those epochs with Observation.get_mapped_data')
+    mode = _interpolation_mode(interpolation, 0)
+    frames = np.ascontiguousarray(frames, dtype=np.float64)
+    if frames.ndim != 2 or frames.shape[1] != F.PMFRAME_NDOUBLES:
+        raise ValueError(f'frames must have shape (n_frames, {F.PMFRAME_NDOUBLES})')
+    shape = tuple(int(d) for d in cubes.shape)
+    if len(shape) not in (3, 4) or shape[0] != len(frames) or shape[-2:] != (ny, nx) or 0 in shape[1:]:
+        raise ValueError(f'cubes must have shape ({len(frames)}, nλ, {ny}, {nx}) or ({len(frames)}, {ny}, {nx}), '
+                         f'not {shape}')
+    lons, lats = np.asarray(lons, dtype=np.float64), np.asarray(lats, dtype=np.float64)
+    if lons.shape != lats.shape or lons.size == 0:
+        raise ValueError(f'lons and lats must have one shape, not {lons.shape} and {lats.shape}')
+    if batch is not None and int(batch) < 1:
+        raise ValueError('batch must be at least 1')
+    return _mapped_series(frames, cubes, nx, ny, lons, lats, mode, propagate_nan, batch)
+
+
+def _series_stride(n_planes: int, mode: int) -> int:
+    """Planes per epoch in the prepared cube: a spline cube of several planes starts every epoch on a plane quad
+    (the gather reads quads); one image per epoch, or the raw cube of nearest, is packed as given."""
+    from . import _lib as L
+
+    return n_planes if mode == L.INTERP_NEAREST or n_planes == 1 else (n_planes + 3) // 4 * 4
+
+
+def _mapped_series(frames, cubes, nx, ny, lons, lats, mode, propagate_nan, batch):
+    from . import _lib as L
+
+    torch = L._torch()
+    lib = L.load_library()
+    n_frames = len(frames)
+    nl = 1 if cubes.ndim == 3 else int(cubes.shape[1])
+    stride = _series_stride(nl, mode)
+    n_cells = lons.size
+    # the prepare launches put a plane per grid row (<= 65535), the map and gather launches an epoch per grid row
+    limit = 65535 // stride
+    if batch is None:
+        per_frame = 8 * (nl + 2) * n_cells + 8 * stride * ny * nx   # output, x / y maps, uploaded cube
+        if mode != L.INTERP_NEAREST:
+            per_frame += (lib.pm_spline_coef_bytes(stride, ny, nx) + lib.pm_spline_nanbits_bytes(stride, ny, nx) +
+                          lib.pm_spline_work_bytes(stride, ny, nx, mode))
+        free, _total = torch.cuda.mem_get_info()
+        budget = int(SERIES_MEMORY_SHARE * free)
+        if per_frame > budget:
+            raise ValueError(f'one epoch needs {per_frame / 1e9:.1f} GB of device memory and {budget / 1e9:.1f} GB '
+                             'are available to a batch: map that epoch with Observation.iter_mapped_data')
+        batch = budget // per_frame
+    batch = int(max(1, min(batch, n_frames, limit)))
+    fd = L.to_device(frames)
+    lod = L.to_device(lons % 360)
+    lad = L.to_device(lats)
+    xy_mask = L.mask_from_names(['PIXEL-X', 'PIXEL-Y'])
+    xy = torch.empty((batch, 2) + lons.shape, dtype=torch.float64, device=fd.device)
+    out = torch.empty((batch, nl) + lons.shape, dtype=torch.float64, device=fd.device)
+    on_device = isinstance(cubes, torch.Tensor) and cubes.is_cuda and cubes.dtype == torch.float64
+    staged = None
+    if stride != nl or not on_device:
+        # the batch's cubes at `stride` planes per epoch; pad planes are all NaN and are never mapped
+        staged = torch.full((batch, stride, ny, nx), float('nan'), dtype=torch.float64, device=fd.device)
+    for first in range(0, n_frames, batch):
+        n = min(batch, n_frames - first)
+        L.backplanes_map_batch(fd[first:first + n], lod, lad, xy_mask, out=xy[:n])
+        part = cubes[first:first + n]
+        if staged is None:
+            cube = part.reshape(n * nl, ny, nx).contiguous()
+        else:
+            if not isinstance(part, torch.Tensor):
+                part = torch.from_numpy(np.ascontiguousarray(part, dtype=np.float64))
+            staged[:n, :nl].copy_(part.reshape(n, nl, ny, nx))
+            cube = staged[:n].view(n * stride, ny, nx)
+        src = cube if mode == L.INTERP_NEAREST else L.spline_prepare(cube, mode)
+        L.gather_grouped(src, xy[:n, 0], xy[:n, 1], mode, nl, stride, propagate_nan=propagate_nan, out=out[:n])
+        yield first, (out[:n, 0] if cubes.ndim == 3 else out[:n])
 
 
 # ---- point transforms over the epochs of a series -------------------------------------------------
