@@ -197,7 +197,30 @@ int pm_backplanes_map_host(const PMFrame *frame_host, const double *lon, const d
  *                            multiple of 4 (groups start on a plane quad) is the fast layout for
  *                            planes_per_map > 1; pm_gather_paired is planes_per_map = plane_stride = 1.
  *                            Empty input (n_maps, planes_per_map or n_cells 0) is valid with NULL pointers.
+ *   pm_composite_grouped     pm_gather_grouped's voxels folded over the epochs into ONE map of planes_per_map
+ *                            planes, without storing any epoch's map (a composite of many observations of one
+ *                            target: frames over a rotation, the tiles of a mosaic).  Epoch g's maps are
+ *                            n_map_planes planes n_cells apart at maps + g * map_stride: PIXEL-X, PIXEL-Y and,
+ *                            with n_map_planes = 3, EMISSION (pm_backplanes_map_batch's output for those masks).
+ *                            Epoch g contributes voxel v_g where v_g is not NaN and EMISSION_g <= max_emission
+ *                            (pass INFINITY for no cut; a NaN EMISSION never passes).  Per voxel:
+ *                              PM_COMPOSITE_MEAN          value = the contributions summed in epoch order by IEEE
+ *                                                         adds, over their count; tag = the count (NaN, 0: none).
+ *                                                         n_map_planes = 2 needs max_emission = INFINITY.
+ *                              PM_COMPOSITE_MIN_EMISSION  value = the contribution of the smallest EMISSION, ties to
+ *                                                         the lowest epoch; tag = epoch_begin + g of that epoch (NaN,
+ *                                                         -1: none); needs n_map_planes = 3 and `key`.
+ *                            A long series takes one call per batch of epochs, in order, over the same value /
+ *                            key / tag [planes_per_map][n_cells] (int32 tag): `first` (0 / 1) initialises them
+ *                            instead of reading them, `last` (0 / 1) finalises them (the mean's division; `key` is
+ *                            then no longer written), so the result does not depend on how the epochs are split.
+ *                            The other arguments are pm_gather_grouped's.  Every mode is the scalar arithmetic of
+ *                            the grouped kernels: a cubic cube on a map of >= 20 cells per image pixel differs from
+ *                            pm_gather_grouped's DMMA voxels in the last bits.  Empty input (n_maps, planes_per_map
+ *                            or n_cells 0) launches nothing and is valid with NULL pointers.
  */
+#define PM_COMPOSITE_MEAN 0
+#define PM_COMPOSITE_MIN_EMISSION 1
 int pm_backplanes_map_batch(const PMFrame *frames, int n_frames, const double *lon, const double *lat,
                             int64_t n_cells, uint64_t plane_mask, double *out, void *stream);
 int pm_gather_paired(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits,
@@ -208,6 +231,11 @@ int pm_gather_grouped(const double *src, const uint32_t *nanbits, const uint32_t
                       int n_planes, int ny, int nx, int n_maps, int planes_per_map, int plane_stride,
                       const double *xmaps, const double *ymaps, int64_t map_stride, int64_t n_cells,
                       int mode, uint32_t flags, double *out, void *stream);
+int pm_composite_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits,
+                         int n_planes, int ny, int nx, int n_maps, int planes_per_map, int plane_stride,
+                         const double *maps, int n_map_planes, int64_t map_stride, int64_t n_cells,
+                         int mode, uint32_t flags, int method, double max_emission, int epoch_begin,
+                         int first, int last, double *value, double *key, int32_t *tag, void *stream);
 
 /*
  * Vectorised point transforms: replace SpiceBase._maybe_transform_as_arrays

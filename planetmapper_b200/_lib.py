@@ -47,6 +47,7 @@ EXPORTED_SYMBOLS = [
     'pm_host_ssb_state', 'pm_host_orientation', 'pm_backplanes_img_host', 'pm_transform', 'pm_fp64_probe', 'pm_proj_forward',
     'pm_backplanes_points_host', 'pm_regrid_work_bytes', 'pm_regrid_fit', 'pm_gather_regrid',
     'pm_xy2lonlat_batch', 'pm_lonlat2xy_batch', 'pm_transform_batch', 'pm_gather_grouped',
+    'pm_composite_grouped',
 ]
 
 
@@ -134,6 +135,9 @@ def load_library() -> ctypes.CDLL:
     lib.pm_gather_grouped.argtypes = [c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p, c_p, c_i64, c_i64, c_i, c_u32,
                                       c_p, c_p]
     lib.pm_gather_grouped.restype = c_i
+    lib.pm_composite_grouped.argtypes = [c_p, c_p, c_p, c_i, c_i, c_i, c_i, c_i, c_i, c_p, c_i, c_i64, c_i64, c_i,
+                                         c_u32, c_i, ctypes.c_double, c_i, c_i, c_i, c_p, c_p, c_p, c_p]
+    lib.pm_composite_grouped.restype = c_i
     lib.pm_host_ssb_state.argtypes = [c_p, c_i, c_p, c_i, ctypes.c_double, c_p]
     lib.pm_host_ssb_state.restype = c_i
     lib.pm_host_orientation.argtypes = [c_p, ctypes.c_double, c_p, c_p]
@@ -430,6 +434,42 @@ def gather_grouped(src, xmaps, ymaps, mode: int, planes_per_map: int, plane_stri
                                  xmaps.stride(0) if n_maps else n_cells, n_cells, mode, flags, out.data_ptr(),
                                  _stream_ptr(torch)), 'pm_gather_grouped')
     return out
+
+
+COMPOSITE_METHODS = {'mean': 0, 'min_emission': 1}
+
+
+def composite_grouped(src, maps, mode: int, planes_per_map: int, plane_stride: int, method: str, value, tag, *,
+                      key=None, max_emission: float = float('inf'), epoch_begin: int = 0, first: bool = True,
+                      last: bool = True, propagate_nan: bool = True) -> None:
+    """pm_composite_grouped: the voxels :func:`gather_grouped` would produce from ``src`` through epoch g's maps,
+    folded over the epochs into ``value`` / ``tag`` (and ``key`` for 'min_emission'), CUDA tensors
+    (planes_per_map,) + map shape of float64 / int32 / float64.  ``maps``: (n_maps, 2 or 3) + map shape, the
+    PIXEL-X, PIXEL-Y [, EMISSION] planes of :func:`backplanes_map_batch`.  ``first`` / ``last``: this call holds the
+    first / last epochs of the series (initialise / finalise the accumulators); ``epoch_begin``: the series index of
+    map 0."""
+    torch = _torch()
+    lib = load_library()
+    spline = src if isinstance(src, Spline) else None
+    if (mode == INTERP_NEAREST) == (spline is not None) or (spline is not None and spline.degree != mode):
+        raise ValueError('composite_grouped: nearest takes the cube, a spline mode the Spline prepared with that mode')
+    if spline is None and not src.is_contiguous():
+        raise ValueError('composite_grouped: the cube must be contiguous')
+    n, ny, nx = (spline.n_planes, spline.ny, spline.nx) if spline is not None else tuple(src.shape)
+    if not maps[0].is_contiguous() or maps.dtype != torch.float64:
+        raise ValueError("each epoch's maps must be contiguous float64")
+    for t, dt in ((value, torch.float64), (tag, torch.int32), (key, torch.float64)):
+        if t is not None and (t.dtype != dt or not t.is_contiguous() or tuple(t.shape[1:]) != tuple(maps.shape[2:])):
+            raise ValueError('composite_grouped: accumulators must be contiguous (planes,) + map shape')
+    data = spline.coef if spline is not None else src
+    _check(lib.pm_composite_grouped(data.data_ptr(), spline.nanbits.data_ptr() if spline is not None else None,
+                                    spline.plane_bits.data_ptr() if spline is not None else None, n, ny, nx,
+                                    maps.shape[0], planes_per_map, plane_stride, maps.data_ptr(), maps.shape[1],
+                                    maps.stride(0), maps[0, 0].numel(), mode,
+                                    FLAG_PROPAGATE_NAN if propagate_nan else 0, COMPOSITE_METHODS[method],
+                                    float(max_emission), int(epoch_begin), int(first), int(last), value.data_ptr(),
+                                    key.data_ptr() if key is not None else None, tag.data_ptr(), _stream_ptr(torch)),
+           'pm_composite_grouped')
 
 
 def xy2lonlat(frame_dev, x_dev, y_dev):

@@ -1,6 +1,7 @@
 // capi.cu - the extern "C" boundary of libpm_b200.so (see include/pm_b200.h).
 // Argument checking, device discovery and launch only: no arithmetic lives here.
 #include <atomic>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 
@@ -127,14 +128,14 @@ int pm_gather_paired(const double *src, const uint32_t *nanbits, const uint32_t 
                                        map_stride, n_cells, mode, flags, out, 0, (cudaStream_t)stream));
 }
 
-int pm_gather_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes, int ny,
-                      int nx, int n_maps, int planes_per_map, int plane_stride, const double *xmaps,
-                      const double *ymaps, int64_t map_stride, int64_t n_cells, int mode, uint32_t flags, double *out,
-                      void *stream) {
+// The sizes, layout and mode of a grouped launch (pm_gather_grouped, pm_composite_grouped): PM_OK or the error.
+// `map_len`: the doubles of one epoch's maps, which map_stride must cover; `empty`: nothing to compute
+static int grouped_layout(int n_planes, int ny, int nx, int n_maps, int planes_per_map, int plane_stride,
+                          int64_t map_stride, int64_t map_len, int64_t n_cells, int mode, bool &empty) {
     if (n_planes < 0 || ny <= 0 || nx <= 0 || n_maps < 0 || n_maps > 65535 || planes_per_map < 0 ||
-        plane_stride < planes_per_map || n_cells < 0 || map_stride < n_cells)
+        plane_stride < planes_per_map || n_cells < 0 || map_stride < map_len)
         return PM_ERR_BAD_ARG;
-    const bool empty = n_maps == 0 || planes_per_map == 0 || n_cells == 0;  // valid, with null pointers
+    empty = n_maps == 0 || planes_per_map == 0 || n_cells == 0;  // valid, with null pointers
     if (!empty && (int64_t)(n_maps - 1) * plane_stride + planes_per_map > n_planes) return PM_ERR_BAD_ARG;
     if (!empty && map_stride > INT64_MAX / n_maps) return PM_ERR_BAD_ARG;
     int ky = mode, kx = mode;
@@ -146,6 +147,17 @@ int pm_gather_grouped(const double *src, const uint32_t *nanbits, const uint32_t
         return PM_ERR_UNSUPPORTED;
     }
     if (mode != PM_INTERP_NEAREST && (nx <= kx || ny <= ky)) return PM_ERR_BAD_ARG;
+    return PM_OK;
+}
+
+int pm_gather_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes, int ny,
+                      int nx, int n_maps, int planes_per_map, int plane_stride, const double *xmaps,
+                      const double *ymaps, int64_t map_stride, int64_t n_cells, int mode, uint32_t flags, double *out,
+                      void *stream) {
+    bool empty = true;
+    const int rc = grouped_layout(n_planes, ny, nx, n_maps, planes_per_map, plane_stride, map_stride, n_cells, n_cells,
+                                  mode, empty);
+    if (rc != PM_OK) return rc;
     if (empty) return PM_OK;
     if (!src || !xmaps || !ymaps || !out) return PM_ERR_BAD_ARG;
     if (mode != PM_INTERP_NEAREST && (!nanbits || !plane_bits)) return PM_ERR_BAD_ARG;
@@ -155,6 +167,33 @@ int pm_gather_grouped(const double *src, const uint32_t *nanbits, const uint32_t
     return check(launch_gather_grouped(src, nanbits, plane_bits, n_planes, ny, nx, n_maps, planes_per_map,
                                        plane_stride, xmaps, ymaps, map_stride, n_cells, mode, flags, out, sms,
                                        (cudaStream_t)stream));
+}
+
+int pm_composite_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes, int ny,
+                         int nx, int n_maps, int planes_per_map, int plane_stride, const double *maps, int n_map_planes,
+                         int64_t map_stride, int64_t n_cells, int mode, uint32_t flags, int method,
+                         double max_emission, int epoch_begin, int first, int last, double *value, double *key,
+                         int32_t *tag, void *stream) {
+    if (method != PM_COMPOSITE_MEAN && method != PM_COMPOSITE_MIN_EMISSION) return PM_ERR_UNSUPPORTED;
+    if (n_map_planes != 2 && n_map_planes != 3) return PM_ERR_BAD_ARG;
+    // without an EMISSION plane there is nothing to cut on or to rank by
+    if (n_map_planes == 2 && (method != PM_COMPOSITE_MEAN || max_emission != INFINITY)) return PM_ERR_BAD_ARG;
+    if (max_emission != max_emission || (flags & ~PM_FLAG_PROPAGATE_NAN) || (first & ~1) || (last & ~1) ||
+        epoch_begin < 0 || (int64_t)epoch_begin + n_maps > INT32_MAX)
+        return PM_ERR_BAD_ARG;
+    bool empty = true;
+    const int rc = grouped_layout(n_planes, ny, nx, n_maps, planes_per_map, plane_stride, map_stride,
+                                  (int64_t)n_map_planes * n_cells, n_cells, mode, empty);
+    if (rc != PM_OK) return rc;
+    if (empty) return PM_OK;
+    if (!src || !maps || !value || !tag || (method == PM_COMPOSITE_MIN_EMISSION && !key)) return PM_ERR_BAD_ARG;
+    if (mode != PM_INTERP_NEAREST && (!nanbits || !plane_bits)) return PM_ERR_BAD_ARG;
+    if (planes_per_map > 65535 * 4) return PM_ERR_BAD_ARG;   // plane groups of four along gridDim.y
+    if (sm_count() <= 0) return PM_ERR_NO_DEVICE;
+    return check(launch_composite_grouped(src, nanbits, plane_bits, n_planes, ny, nx, n_maps, planes_per_map,
+                                          plane_stride, maps, n_map_planes, map_stride, n_cells, mode, flags, method,
+                                          max_emission, epoch_begin, first != 0, last != 0, value, key, tag,
+                                          (cudaStream_t)stream));
 }
 
 int pm_xy2lonlat(const PMFrame *frame, const double *x, const double *y, int64_t n, double *lon, double *lat,

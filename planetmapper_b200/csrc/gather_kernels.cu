@@ -77,16 +77,10 @@ __host__ __device__ __forceinline__ int bspline3_weights(double x, int n, double
 // ---------------------------------------------------------------------------------
 // nearest neighbour: reads the raw cube [n_planes][ny][nx]
 // ---------------------------------------------------------------------------------
-// Planes plane_begin + [l0, l1) at map cell `cell` into out[l][cell]
-__device__ __forceinline__ void nearest_cell_planes(const double *__restrict__ cube, int ny, int nx, int plane_begin,
-                                                    int l0, int l1, const double *__restrict__ xmap,
-                                                    const double *__restrict__ ymap, int64_t cell, int64_t n_cells,
-                                                    double *__restrict__ out) {
-    const int64_t plane_px = (int64_t)ny * nx;
-    const double x = __ldg(xmap + cell), y = __ldg(ymap + cell);
-    const double nan = NAN;
+// The pixel a map cell reads (offset inside a plane); false: the cell is NaN in every plane
+__device__ __forceinline__ bool nearest_pixel(double x, double y, int ny, int nx, int64_t &off) {
     bool valid = !isnan(x);  // y is never NaN when x is not (body_xy.py:1646, :1697)
-    int64_t off = 0;
+    off = 0;
     if (valid) {
         // np.round is round-half-to-even == rint (body_xy.py:1642-1643)
         long xi = (long)rint(x), yi = isnan(y) ? -999 : (long)rint(y);
@@ -95,6 +89,18 @@ __device__ __forceinline__ void nearest_cell_planes(const double *__restrict__ c
         valid = xi >= 0 && xi < nx && yi >= 0 && yi < ny;
         off = (int64_t)yi * nx + xi;
     }
+    return valid;
+}
+
+// Planes plane_begin + [l0, l1) at map cell `cell` into out[l][cell]
+__device__ __forceinline__ void nearest_cell_planes(const double *__restrict__ cube, int ny, int nx, int plane_begin,
+                                                    int l0, int l1, const double *__restrict__ xmap,
+                                                    const double *__restrict__ ymap, int64_t cell, int64_t n_cells,
+                                                    double *__restrict__ out) {
+    const int64_t plane_px = (int64_t)ny * nx;
+    const double nan = NAN;
+    int64_t off;
+    const bool valid = nearest_pixel(__ldg(xmap + cell), __ldg(ymap + cell), ny, nx, off);
     const double *src = cube + (int64_t)(plane_begin + l0) * plane_px + off;
     double *dst = out + (int64_t)l0 * n_cells + cell;
     int l = l0;
@@ -210,6 +216,41 @@ __device__ __forceinline__ void setup_cell(CellState<KY, KX> &c, double x, doubl
     }
 }
 
+// NaN bits of a cell's planes 32 * word .. 32 * word + 31: the all-NaN planes, and with propagate_nan the planes
+// where one of the cell's NaN-test pixels was NaN
+template <int KY, int KX>
+__device__ __forceinline__ uint32_t cell_nan_word(const CellState<KY, KX> &cs, const uint32_t *__restrict__ nanbits,
+                                                  const uint32_t *__restrict__ plane_bits, int n_words, int word,
+                                                  bool propagate) {
+    uint32_t bad = __ldg(plane_bits + word);
+    if (cs.valid && propagate && __ldg(plane_bits + n_words + word)) {
+#pragma unroll
+        for (int k = 0; k < 4; k++) bad |= __ldg(nanbits + (int64_t)cs.nb[k] * n_words + word);
+    }
+    return bad;
+}
+
+// The four planes of the plane quad whose footprint starts at `src` (coefficients, rows outer): K*K/4 loads and
+// K*K FMAs per plane
+template <int KY, int KX>
+__device__ __forceinline__ void spline_quad_sums(const CellState<KY, KX> &cs, const double *__restrict__ src,
+                                                 int64_t row_stride, double acc[4]) {
+#pragma unroll
+    for (int j = 0; j < 4; j++) acc[j] = 0.0;
+    if (cs.valid) {
+#pragma unroll
+        for (int a = 0; a < KY; a++) {
+#pragma unroll
+            for (int b = 0; b < KX; b++) {
+                const Quad q = ldg_quad(src + a * row_stride + b * 4);
+                const double ww = cs.w[a * KX + b];
+#pragma unroll
+                for (int j = 0; j < 4; j++) acc[j] = fma(q.v[j], ww, acc[j]);
+            }
+        }
+    }
+}
+
 // Planes plane_begin + [l0, l1) of one prepared cell, a plane quad at a time (plane_begin + l0 a multiple
 // of 4), into out[l][cell]
 template <int KY, int KX>
@@ -229,26 +270,10 @@ __device__ __forceinline__ void spline_cell_quads(CellState<KY, KX> &cs, const d
         const int word = gl >> 5;
         if (word != cur_word) {  // uniform: once per 32 planes
             cur_word = word;
-            uint32_t bad = __ldg(plane_bits + word);
-            if (cs.valid && propagate && __ldg(plane_bits + n_words + word)) {
-#pragma unroll
-                for (int k = 0; k < 4; k++) bad |= __ldg(nanbits + (int64_t)cs.nb[k] * n_words + word);
-            }
-            cs.bad = bad;
+            cs.bad = cell_nan_word<KY, KX>(cs, nanbits, plane_bits, n_words, word, propagate);
         }
-        double acc[4] = {0.0, 0.0, 0.0, 0.0};
-        if (cs.valid) {
-#pragma unroll
-            for (int a = 0; a < KY; a++) {
-#pragma unroll
-                for (int b = 0; b < KX; b++) {
-                    const Quad q = ldg_quad(src + a * row_stride + b * 4);
-                    const double ww = cs.w[a * KX + b];
-#pragma unroll
-                    for (int j = 0; j < 4; j++) acc[j] = fma(q.v[j], ww, acc[j]);
-                }
-            }
-        }
+        double acc[4];
+        spline_quad_sums<KY, KX>(cs, src, row_stride, acc);
         const uint32_t nib = cs.valid ? ((cs.bad >> (gl & 31)) & 0xFu) : 0xFu;
         const int left = l1 - l;
 #pragma unroll
@@ -849,6 +874,166 @@ __global__ void __launch_bounds__(kGatherBlock, kMinBlocks)
     }
 }
 
+// ---------------------------------------------------------------------------------
+// Composite of a mapped series (pm_composite_grouped): the maps and cube of pm_gather_grouped, but instead of
+// storing map g's planes the kernel folds them over the epochs into one (planes_per_map, n_cells) result.  A
+// thread owns one cell and PG planes, loops over the launch's epochs and keeps the PG accumulators in registers:
+// they are read once at the start (or initialised: `first`) and written once at the end (or finalised: `last`).
+// Per epoch the cell's x / y (and EMISSION) are loaded, the cell is set up and every plane is evaluated with
+// gather_grouped_kernel's own functions, so the folded values are the voxels pm_gather_grouped would store.
+//   mean          acc = sum of the non-NaN values in epoch order (__dadd_rn: with FMA contraction on, a plain
+//                 `+` could fuse with the spline's last product), tag = their count; `last`: acc = sum / count,
+//                 NaN for count 0.
+//   min_emission  acc = the non-NaN value of the epoch with the smallest EMISSION, key = that EMISSION, tag =
+//                 its epoch (epoch_begin + g; -1 while none).  Epochs run in increasing order and only a
+//                 strictly smaller EMISSION replaces the pick, so ties keep the lowest epoch.
+// An epoch contributes at a cell only where EMISSION <= max_emission (a NaN EMISSION never does); without an
+// EMISSION plane (n_map_planes = 2, mean, no cut) every epoch does.
+// ---------------------------------------------------------------------------------
+template <int PG, bool kMin>
+struct CompositeAcc {
+    double acc[PG];
+    double key[kMin ? PG : 1];
+    int tag[PG];
+
+    __device__ __forceinline__ void load(const double *__restrict__ value, const double *__restrict__ keys,
+                                         const int *__restrict__ tags, int np, int64_t cell, int64_t n_cells,
+                                         bool first) {
+#pragma unroll
+        for (int p = 0; p < PG; p++) {
+            acc[p] = kMin ? NAN : 0.0;
+            tag[p] = kMin ? -1 : 0;
+            if (kMin) key[p] = NAN;
+            if (!first && p < np) {
+                acc[p] = value[p * n_cells + cell];
+                tag[p] = tags[p * n_cells + cell];
+                if (kMin) key[p] = keys[p * n_cells + cell];
+            }
+        }
+    }
+    __device__ __forceinline__ void fold(int p, double v, double e, int epoch) {
+        if (isnan(v)) return;
+        if (kMin) {
+            if (tag[p] < 0 || e < key[p]) {
+                acc[p] = v;
+                key[p] = e;
+                tag[p] = epoch;
+            }
+        } else {
+            acc[p] = __dadd_rn(acc[p], v);
+            tag[p]++;
+        }
+    }
+    __device__ __forceinline__ void store(double *__restrict__ value, double *__restrict__ keys, int *__restrict__ tags,
+                                          int np, int64_t cell, int64_t n_cells, bool last) const {
+#pragma unroll
+        for (int p = 0; p < PG; p++) {
+            if (p >= np) continue;
+            double a = acc[p];
+            if (!kMin && last) a = tag[p] > 0 ? a / (double)tag[p] : NAN;
+            value[p * n_cells + cell] = a;
+            tags[p * n_cells + cell] = tag[p];
+            if (kMin && !last) keys[p * n_cells + cell] = key[p];
+        }
+    }
+};
+
+struct CompositeArgs {
+    const double *maps;     // epoch g: x at maps + g * map_stride, y at + n_cells, EMISSION at + 2 * n_cells
+    int n_map_planes;       // 2 (x, y) or 3 (x, y, EMISSION)
+    int64_t map_stride;
+    double max_emission;
+    int epoch_begin;
+    bool first, last;
+    double *value, *key;    // [planes_per_map][n_cells]
+    int *tag;
+};
+
+// The epoch's x / y at the cell, and whether the epoch passes the EMISSION cut there
+__device__ __forceinline__ bool composite_epoch(const CompositeArgs &a, int g, int64_t cell, int64_t n_cells,
+                                                double &x, double &y, double &e) {
+    const double *m = a.maps + (int64_t)g * a.map_stride + cell;
+    x = __ldg(m);
+    y = __ldg(m + n_cells);
+    e = a.n_map_planes > 2 ? __ldg(m + 2 * n_cells) : 0.0;
+    return e <= a.max_emission && !isnan(x);
+}
+
+template <int PG, bool kMin>
+__global__ void __launch_bounds__(kGatherBlock)
+    composite_nearest_kernel(const double *__restrict__ cube, int ny, int nx, int n_maps, int planes_per_map,
+                             int plane_stride, int64_t n_cells, const __grid_constant__ CompositeArgs a) {
+    const int64_t cell = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (cell >= n_cells) return;
+    const int l0 = blockIdx.y * PG, np = min(PG, planes_per_map - l0);
+    const int64_t plane_px = (int64_t)ny * nx;
+    CompositeAcc<PG, kMin> s;
+    s.load(a.value + (int64_t)l0 * n_cells, a.key + (int64_t)l0 * n_cells, a.tag + (int64_t)l0 * n_cells, np, cell,
+           n_cells, a.first);
+    for (int g = 0; g < n_maps; g++) {
+        double x, y, e;
+        int64_t off;
+        if (!composite_epoch(a, g, cell, n_cells, x, y, e) || !nearest_pixel(x, y, ny, nx, off)) continue;
+        const double *src = cube + (int64_t)(g * plane_stride + l0) * plane_px + off;
+#pragma unroll
+        for (int p = 0; p < PG; p++)
+            if (p < np) s.fold(p, __ldg(src + p * plane_px), e, a.epoch_begin + g);
+    }
+    s.store(a.value + (int64_t)l0 * n_cells, a.key + (int64_t)l0 * n_cells, a.tag + (int64_t)l0 * n_cells, np, cell,
+            n_cells, a.last);
+}
+
+// kQuads: every epoch's planes start on a plane quad (plane_stride a multiple of 4, PG a multiple of 4) and are
+// read a quad per 32-byte load, as gather_grouped_kernel<kQuads = true>; otherwise plane by plane
+template <int KY, int KX, bool kQuads, int PG, bool kMin, int kMinBlocks>
+__global__ void __launch_bounds__(kGatherBlock, kMinBlocks)
+    composite_grouped_kernel(const double *__restrict__ coefq, const uint32_t *__restrict__ nanbits,
+                             const uint32_t *__restrict__ plane_bits, int n_words, int ny, int nx, int n_maps,
+                             int planes_per_map, int plane_stride, int64_t n_cells, uint32_t flags,
+                             const __grid_constant__ CompositeArgs a) {
+    static_assert(!kQuads || PG % 4 == 0, "a plane group of whole quads");
+    const int64_t cell = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (cell >= n_cells) return;
+    const int l0 = blockIdx.y * PG, np = min(PG, planes_per_map - l0);
+    const bool propagate = (flags & PM_FLAG_PROPAGATE_NAN) != 0;
+    const int64_t row_stride = (int64_t)nx * 4, quad_stride = (int64_t)ny * row_stride;
+    CompositeAcc<PG, kMin> s;
+    s.load(a.value + (int64_t)l0 * n_cells, a.key + (int64_t)l0 * n_cells, a.tag + (int64_t)l0 * n_cells, np, cell,
+           n_cells, a.first);
+    for (int g = 0; g < n_maps; g++) {
+        double x, y, e;
+        if (!composite_epoch(a, g, cell, n_cells, x, y, e)) continue;
+        CellState<KY, KX> cs;
+        setup_cell<KY, KX>(cs, x, y, ny, nx, propagate);
+        if (!cs.valid) continue;   // NaN in every plane
+        const int gb = g * plane_stride + l0;
+        const int epoch = a.epoch_begin + g;
+        if (kQuads) {
+#pragma unroll
+            for (int q = 0; q < PG / 4; q++) {
+                if (4 * q >= np) break;
+                const int gl = gb + 4 * q;   // a multiple of 4: the quad lies in one NaN word
+                const uint32_t nib =
+                    (cell_nan_word<KY, KX>(cs, nanbits, plane_bits, n_words, gl >> 5, propagate) >> (gl & 31)) & 0xFu;
+                double acc[4];
+                spline_quad_sums<KY, KX>(cs, coefq + (int64_t)(gl >> 2) * quad_stride + cs.origin, row_stride, acc);
+#pragma unroll
+                for (int j = 0; j < 4; j++)
+                    if (4 * q + j < np && !((nib >> j) & 1u)) s.fold(4 * q + j, acc[j], e, epoch);
+            }
+        } else {
+#pragma unroll
+            for (int p = 0; p < PG; p++)
+                if (p < np)
+                    s.fold(p, spline_cell_plane<KY, KX>(cs, coefq, nanbits, plane_bits, n_words, ny, nx, gb + p,
+                                                        propagate),
+                           e, epoch);
+        }
+    }
+    s.store(a.value + (int64_t)l0 * n_cells, a.key + (int64_t)l0 * n_cells, a.tag + (int64_t)l0 * n_cells, np, cell,
+            n_cells, a.last);
+}
+
 // launch_gather's switch to the DMMA kernel for cubic: many map cells per image pixel share a footprint.
 // Measured crossover with the one-cell-per-thread kernel (tools/probe_density.py): ~16 map cells per image
 // pixel - at 15.8 the scalar kernel is 10 % faster, at 63 the DMMA kernel 1.5x, at 400 (BASELINE C4) 2x
@@ -986,6 +1171,70 @@ cudaError_t launch_gather_grouped(const double *src, const uint32_t *nanbits, co
         default: PM_GROUPED(4, 4, 2, 2); break;
     }
 #undef PM_GROUPED
+    count_launches(1);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_composite_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits,
+                                     int n_planes, int ny, int nx, int n_maps, int planes_per_map, int plane_stride,
+                                     const double *maps, int n_map_planes, int64_t map_stride, int64_t n_cells,
+                                     int mode, uint32_t flags, int method, double max_emission, int epoch_begin,
+                                     bool first, bool last, double *value, double *key, int32_t *tag,
+                                     cudaStream_t st) {
+    if (n_maps == 0 || planes_per_map == 0 || n_cells == 0) return cudaSuccess;
+    const CompositeArgs a{maps, n_map_planes, map_stride, max_emission, epoch_begin, first, last, value, key, tag};
+    const bool min_e = method == PM_COMPOSITE_MIN_EMISSION;
+    const unsigned cell_blocks = (unsigned)((n_cells + kGatherBlock - 1) / kGatherBlock);
+    auto grid = [&](int pg) { return dim3(cell_blocks, (unsigned)((planes_per_map + pg - 1) / pg)); };
+    if (mode == PM_INTERP_NEAREST) {
+        if (min_e)
+            composite_nearest_kernel<8, true><<<grid(8), kGatherBlock, 0, st>>>(src, ny, nx, n_maps, planes_per_map,
+                                                                                plane_stride, n_cells, a);
+        else
+            composite_nearest_kernel<8, false><<<grid(8), kGatherBlock, 0, st>>>(src, ny, nx, n_maps, planes_per_map,
+                                                                                 plane_stride, n_cells, a);
+        count_launches(1);
+        return cudaGetLastError();
+    }
+    int ky = mode, kx = mode;
+    if (mode & PM_INTERP_MIXED) {
+        ky = (mode >> 4) & 0xF;
+        kx = mode & 0xF;
+    }
+    if (ky < 1 || ky > 3 || kx < 1 || kx > 3) return cudaErrorInvalidValue;
+    // the quad layout of gather_grouped_kernel; a cubic cube on a dense map also takes it (no DMMA form here)
+    const bool quads = planes_per_map > 1 && plane_stride % 4 == 0;
+    const int n_words = (n_planes + 31) / 32;
+    // Planes per thread (quad form, plane-by-plane form) and CTAs per SM: the per-epoch cell setup is shared by a
+    // thread's planes, whose accumulators live in registers for the whole launch; the values are the largest at
+    // which each instantiation compiles without spills (ptxas -v)
+#define PM_COMPOSITE_LAUNCH(KY, KX, Q, PG, MIN, MB)                                                                 \
+    composite_grouped_kernel<KY, KX, Q, PG, MIN, MB><<<grid(PG), kGatherBlock, 0, st>>>(                            \
+        src, nanbits, plane_bits, n_words, ny, nx, n_maps, planes_per_map, plane_stride, n_cells, flags, a)
+#define PM_COMPOSITE(KY, KX, PGQ, MBQ, PG1, MB1)                                                                    \
+    do {                                                                                                            \
+        if (quads && min_e)                                                                                         \
+            PM_COMPOSITE_LAUNCH(KY, KX, true, PGQ, true, MBQ);                                                      \
+        else if (quads)                                                                                             \
+            PM_COMPOSITE_LAUNCH(KY, KX, true, PGQ, false, MBQ);                                                     \
+        else if (min_e)                                                                                             \
+            PM_COMPOSITE_LAUNCH(KY, KX, false, PG1, true, MB1);                                                     \
+        else                                                                                                        \
+            PM_COMPOSITE_LAUNCH(KY, KX, false, PG1, false, MB1);                                                    \
+    } while (0)
+    switch (ky * 4 + kx) {
+        case 1 * 4 + 1: PM_COMPOSITE(2, 2, 4, 4, 4, 4); break;
+        case 1 * 4 + 2: PM_COMPOSITE(2, 3, 4, 3, 4, 3); break;
+        case 1 * 4 + 3: PM_COMPOSITE(2, 4, 4, 3, 4, 3); break;
+        case 2 * 4 + 1: PM_COMPOSITE(3, 2, 4, 3, 4, 3); break;
+        case 2 * 4 + 2: PM_COMPOSITE(3, 3, 4, 2, 4, 3); break;
+        case 2 * 4 + 3: PM_COMPOSITE(3, 4, 4, 3, 4, 3); break;
+        case 3 * 4 + 1: PM_COMPOSITE(4, 2, 4, 3, 4, 3); break;
+        case 3 * 4 + 2: PM_COMPOSITE(4, 3, 4, 2, 4, 3); break;
+        default: PM_COMPOSITE(4, 4, 4, 2, 4, 2); break;
+    }
+#undef PM_COMPOSITE
+#undef PM_COMPOSITE_LAUNCH
     count_launches(1);
     return cudaGetLastError();
 }

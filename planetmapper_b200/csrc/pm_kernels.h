@@ -76,6 +76,14 @@ cudaError_t launch_gather_grouped(const double *src, const uint32_t *nanbits, co
                                   int ny, int nx, int n_maps, int planes_per_map, int plane_stride, const double *xmaps,
                                   const double *ymaps, int64_t map_stride, int64_t n_cells, int mode, uint32_t flags,
                                   double *out, int sm_count, cudaStream_t st);
+// the same maps and planes folded over the epochs into value / key / tag [planes_per_map][n_cells]
+// (pm_composite_grouped); maps: epoch g's n_map_planes planes (x, y[, EMISSION]) at maps + g * map_stride
+cudaError_t launch_composite_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits,
+                                     int n_planes, int ny, int nx, int n_maps, int planes_per_map, int plane_stride,
+                                     const double *maps, int n_map_planes, int64_t map_stride, int64_t n_cells,
+                                     int mode, uint32_t flags, int method, double max_emission, int epoch_begin,
+                                     bool first, bool last, double *value, double *key, int32_t *tag,
+                                     cudaStream_t st);
 
 int64_t spline_coef_bytes(int n_planes, int ny, int nx);
 int64_t spline_nanbits_bytes(int n_planes, int ny, int nx);

@@ -277,10 +277,18 @@ def iter_mapped_series(frames: np.ndarray, cubes, nx: int, ny: int, lons, lats, 
     >= 20 map cells per image pixel: pm_gather's dense-map kernel once per epoch).  ``batch`` (epochs per batch)
     defaults to what keeps a batch within SERIES_MEMORY_SHARE of the free device memory.
     """
+    mode, frames, lons, lats = _series_args('iter_mapped_series', frames, cubes, nx, ny, lons, lats, interpolation,
+                                            spline_smoothing, batch)
+    return _mapped_series(frames, cubes, nx, ny, lons, lats, mode, propagate_nan, batch)
+
+
+def _series_args(fn, frames, cubes, nx, ny, lons, lats, interpolation, spline_smoothing, batch):
+    """The argument rules of the mapped-series functions, checked before any device work: (mode, frames, lons,
+    lats) as the batches need them."""
     from .body_xy import _interpolation_mode
 
     if interpolation == 'smooth' or spline_smoothing != 0:
-        raise NotImplementedError("iter_mapped_series: 'smooth' and smoothing splines (spline_smoothing != 0) fit "
+        raise NotImplementedError(f"{fn}: 'smooth' and smoothing splines (spline_smoothing != 0) fit "
                                   'per-epoch grids; map those epochs with Observation.get_mapped_data')
     mode = _interpolation_mode(interpolation, 0)
     frames = np.ascontiguousarray(frames, dtype=np.float64)
@@ -295,7 +303,7 @@ def iter_mapped_series(frames: np.ndarray, cubes, nx: int, ny: int, lons, lats, 
         raise ValueError(f'lons and lats must have one shape, not {lons.shape} and {lats.shape}')
     if batch is not None and int(batch) < 1:
         raise ValueError('batch must be at least 1')
-    return _mapped_series(frames, cubes, nx, ny, lons, lats, mode, propagate_nan, batch)
+    return mode, frames, lons, lats
 
 
 def _series_stride(n_planes: int, mode: int) -> int:
@@ -306,7 +314,13 @@ def _series_stride(n_planes: int, mode: int) -> int:
     return n_planes if mode == L.INTERP_NEAREST or n_planes == 1 else (n_planes + 3) // 4 * 4
 
 
-def _mapped_series(frames, cubes, nx, ny, lons, lats, mode, propagate_nan, batch):
+def _prepared_batches(frames, cubes, nx, ny, lons, lats, mode, batch, mask, out_planes):
+    """The batches of a mapped series: per batch of n epochs ONE pm_backplanes_map_batch launch with the planes of
+    ``mask`` and the batch's cubes staged at ``_series_stride`` planes per epoch (pad planes all NaN) and prepared
+    once (nearest reads the staged cube as it is).  Yields ``(first, n, maps, src, stride)``: maps (n,
+    popcount(mask)) + grid and the gather source, both REUSED by the next batch.  ``batch`` None: what keeps a
+    batch's cubes, prepared operand, maps and ``out_planes`` output planes per epoch within SERIES_MEMORY_SHARE of
+    the free device memory."""
     from . import _lib as L
 
     torch = L._torch()
@@ -315,10 +329,11 @@ def _mapped_series(frames, cubes, nx, ny, lons, lats, mode, propagate_nan, batch
     nl = 1 if cubes.ndim == 3 else int(cubes.shape[1])
     stride = _series_stride(nl, mode)
     n_cells = lons.size
+    n_maps = L.popcount(mask)
     # the prepare launches put a plane per grid row (<= 65535), the map and gather launches an epoch per grid row
     limit = 65535 // stride
     if batch is None:
-        per_frame = 8 * (nl + 2) * n_cells + 8 * stride * ny * nx   # output, x / y maps, uploaded cube
+        per_frame = 8 * (out_planes + n_maps) * n_cells + 8 * stride * ny * nx   # output, maps, uploaded cube
         if mode != L.INTERP_NEAREST:
             per_frame += (lib.pm_spline_coef_bytes(stride, ny, nx) + lib.pm_spline_nanbits_bytes(stride, ny, nx) +
                           lib.pm_spline_work_bytes(stride, ny, nx, mode))
@@ -332,9 +347,7 @@ def _mapped_series(frames, cubes, nx, ny, lons, lats, mode, propagate_nan, batch
     fd = L.to_device(frames)
     lod = L.to_device(lons % 360)
     lad = L.to_device(lats)
-    xy_mask = L.mask_from_names(['PIXEL-X', 'PIXEL-Y'])
-    xy = torch.empty((batch, 2) + lons.shape, dtype=torch.float64, device=fd.device)
-    out = torch.empty((batch, nl) + lons.shape, dtype=torch.float64, device=fd.device)
+    maps = torch.empty((batch, n_maps) + lons.shape, dtype=torch.float64, device=fd.device)
     on_device = isinstance(cubes, torch.Tensor) and cubes.is_cuda and cubes.dtype == torch.float64
     staged = None
     if stride != nl or not on_device:
@@ -342,7 +355,7 @@ def _mapped_series(frames, cubes, nx, ny, lons, lats, mode, propagate_nan, batch
         staged = torch.full((batch, stride, ny, nx), float('nan'), dtype=torch.float64, device=fd.device)
     for first in range(0, n_frames, batch):
         n = min(batch, n_frames - first)
-        L.backplanes_map_batch(fd[first:first + n], lod, lad, xy_mask, out=xy[:n])
+        L.backplanes_map_batch(fd[first:first + n], lod, lad, mask, out=maps[:n])
         part = cubes[first:first + n]
         if staged is None:
             cube = part.reshape(n * nl, ny, nx).contiguous()
@@ -351,9 +364,75 @@ def _mapped_series(frames, cubes, nx, ny, lons, lats, mode, propagate_nan, batch
                 part = torch.from_numpy(np.ascontiguousarray(part, dtype=np.float64))
             staged[:n, :nl].copy_(part.reshape(n, nl, ny, nx))
             cube = staged[:n].view(n * stride, ny, nx)
-        src = cube if mode == L.INTERP_NEAREST else L.spline_prepare(cube, mode)
-        L.gather_grouped(src, xy[:n, 0], xy[:n, 1], mode, nl, stride, propagate_nan=propagate_nan, out=out[:n])
+        yield first, n, maps[:n], (cube if mode == L.INTERP_NEAREST else L.spline_prepare(cube, mode)), stride
+
+
+def _mapped_series(frames, cubes, nx, ny, lons, lats, mode, propagate_nan, batch):
+    from . import _lib as L
+
+    torch = L._torch()
+    nl = 1 if cubes.ndim == 3 else int(cubes.shape[1])
+    out = None
+    for first, n, xy, src, stride in _prepared_batches(frames, cubes, nx, ny, lons, lats, mode, batch,
+                                                       L.mask_from_names(['PIXEL-X', 'PIXEL-Y']), nl):
+        if out is None:   # the first batch is a full one
+            out = torch.empty((n, nl) + lons.shape, dtype=torch.float64, device=xy.device)
+        L.gather_grouped(src, xy[:, 0], xy[:, 1], mode, nl, stride, propagate_nan=propagate_nan, out=out[:n])
         yield first, (out[:n, 0] if cubes.ndim == 3 else out[:n])
+
+
+def composite_mapped_series(frames: np.ndarray, cubes, nx: int, ny: int, lons, lats, *, interpolation='linear',
+                            spline_smoothing: float = 0, propagate_nan: bool = True, method: str = 'mean',
+                            max_emission=None, batch: int | None = None):
+    """The epochs of a mapped series combined into ONE map on the device: a composite of many observations of one
+    target on a shared lon / lat grid (frames spread over a rotation, the tiles or dithers of a mosaic: one epoch
+    repeated with different discs).  Takes what :func:`iter_mapped_series` takes, with its errors.
+
+    Let v_f be the value :func:`iter_mapped_series` produces for epoch f at a plane and cell, and e_f epoch f's
+    EMISSION angle at that cell (``BodyXY.get_backplane_map('EMISSION')``).  Epoch f contributes there iff v_f is
+    not NaN and, when ``max_emission`` (degrees, 0..180) is given, e_f <= max_emission (a NaN e_f does not).
+
+    ``method='mean'``: the contributions summed in epoch order by IEEE adds, over their count (``np.nanmean`` with
+    that summation order); tag = the count.  ``method='min_emission'``: the contribution of the epoch with the
+    smallest e_f, ties to the lowest epoch; tag = that epoch's index.  The choice is per voxel: a NaN pixel of the
+    best epoch in one plane falls through to the next-best epoch for that plane.  Cells without a contribution
+    are NaN with tag 0 (mean) or -1 (min_emission).
+
+    Returns ``(composite, tag)``: CUDA tensors (nλ,) + grid shape (grid shape for 3-D input), float64 and int32.
+    Per batch of epochs: one map launch (PIXEL-X / PIXEL-Y, plus EMISSION when the method or the cut reads it), the
+    spline preparation of :func:`iter_mapped_series` and ONE pm_composite_grouped launch, which folds every
+    epoch's voxels into accumulators held in registers and never stores the per-epoch maps.  The result does not
+    depend on ``batch``, bit for bit.  Every mode equals the fold of :func:`iter_mapped_series`' output bit for
+    bit, except cubic cubes on maps of >= 20 cells per image pixel, where that function runs the DMMA gather and
+    the values may differ in the last bits.
+    """
+    from . import _lib as L
+
+    mode, frames, lons, lats = _series_args('composite_mapped_series', frames, cubes, nx, ny, lons, lats,
+                                            interpolation, spline_smoothing, batch)
+    if method not in L.COMPOSITE_METHODS:
+        raise ValueError(f"method must be one of {sorted(L.COMPOSITE_METHODS)}, not {method!r}")
+    if max_emission is not None:
+        max_emission = float(max_emission)
+        if not 0.0 <= max_emission <= 180.0:
+            raise ValueError(f'max_emission must be None or an angle in [0, 180] degrees, not {max_emission}')
+    if len(frames) == 0:
+        raise ValueError('composite_mapped_series needs at least one epoch')
+    torch = L._torch()
+    nl = 1 if cubes.ndim == 3 else int(cubes.shape[1])
+    shape = (nl,) + lons.shape
+    value = torch.empty(shape, dtype=torch.float64, device='cuda')
+    tag = torch.empty(shape, dtype=torch.int32, device='cuda')
+    key = torch.empty(shape, dtype=torch.float64, device='cuda') if method == 'min_emission' else None
+    # a plain mean keeps the x / y-only mask (the map kernel's fixed-plane-set instantiation)
+    names = ['PIXEL-X', 'PIXEL-Y'] + (['EMISSION'] if method == 'min_emission' or max_emission is not None else [])
+    cut = float('inf') if max_emission is None else max_emission
+    for first, n, maps, src, stride in _prepared_batches(frames, cubes, nx, ny, lons, lats, mode, batch,
+                                                         L.mask_from_names(names), 0):
+        L.composite_grouped(src, maps, mode, nl, stride, method, value, tag, key=key, max_emission=cut,
+                            epoch_begin=first, first=first == 0, last=first + n == len(frames),
+                            propagate_nan=propagate_nan)
+    return (value[0], tag[0]) if cubes.ndim == 3 else (value, tag)
 
 
 # ---- point transforms over the epochs of a series -------------------------------------------------
