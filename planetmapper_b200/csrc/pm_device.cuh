@@ -85,6 +85,7 @@ struct FrameD {
     double inv_kmpa;   // 1 / km_per_arcsec
     int biaxial;       // intercept ellipsoid == recpgr spheroid -> closed-form geodetic
     int spin_sym;      // spheroid spinning about its symmetry axis: the image planes are taken in the t_ref frame
+    int spin_z;        // spin_sym with the spin axis on z: LON / LAT are taken from the point at t_ref as well
 };
 
 constexpr int kDeriveItems = 13;
@@ -169,6 +170,13 @@ PM_HD void derive_frame_item(FrameD &s, int item) {
         const double flat = fabs(ex_add(f.radii[0], -f.radii[2]));
         const double shift = ex_mul(ex_mul(wperp, ex_div(ex_mul(2.0, f.radii[0]), f.clight)), flat);
         s.spin_sym = (f.radii[0] == f.radii[1]) && (shift <= 1.0e-9);
+        // image_pixel<kSpinSym> then also takes LON / LAT without spinning the point: rho and z of the point at
+        // t_ref, the longitude less omega_z dt.  That neglects the rotation |omega_perp| dt about an axis
+        // perpendicular to z, a displacement of at most |omega_perp| (2 a / clight) a.  Allowed up to 1e-8 km (Jupiter:
+        // 2.5e-9 km, 2e-12 deg), still 40 times below the epoch quantum's 4e-7 km.  A sphere whose spin axis is tilted
+        // off z keeps spin_sym but not this: its points are spun.
+        const double lon_shift = ex_mul(ex_mul(wperp, ex_div(ex_mul(2.0, f.radii[0]), f.clight)), f.radii[0]);
+        s.spin_z = s.spin_sym && (lon_shift <= 1.0e-8);
     } else if (item == 1) {
         const double a = f.radii[0], b = f.radii[1], c = f.radii[2];
         s.inv_r[0] = ex_div(1.0, a);
@@ -364,12 +372,12 @@ PM_HD bool surfpt(const FrameD &fs, V3 o, V3 u, V3 &p, RayHit &hit) {
 // Result of the converged intercept, everything in the body frame at the intercept
 // epoch t_ref + dt unless stated.
 struct Intercept {
-    V3 p;        // surface point (body-fixed)
+    V3 p;        // surface point (body-fixed; general path only)
     V3 u;        // unit ray observer -> point in the body frame at the intercept epoch: the line of sight
                  // itself (exact), not (p - o) / L, which carries p's error magnified by r / L for a near observer
                  // (general path only)
     V3 p0;       // the surface point in the body frame at t_ref (spin-symmetric path only)
-    Rot r;       // spin over dt
+    Rot r;       // spin over dt (general path only)
     double dt;   // intercept epoch - t_ref
     double L;    // observer -> point range (km)
     double lt;   // L / c
@@ -419,13 +427,12 @@ PM_HD_NOINLINE bool sincpt_converge(const FrameD &fs, V3 u0, double &dt, V3 &p, 
 //
 // kSpinSym (FrameD::spin_sym): the body is a spheroid spinning about its symmetry axis.  Spinning the
 // observer and the ray together about that axis leaves the ray / ellipsoid solve unchanged, so every pass
-// is solved in the body frame at t_ref - observer -target_pos_b(dt), ray u0 - and only the final point is
-// spun to its epoch.  Pass 2 then shares pass 1's direction x and 1 / |x|^2, and it.p0 holds the point at
-// t_ref; it.u is not set.
+// is solved in the body frame at t_ref - observer -target_pos_b(dt), ray u0.  Pass 2 then shares pass 1's
+// direction x and 1 / |x|^2, and it.p0 holds the point at t_ref; it.p, it.u and it.r are not set.
 template <bool kSpinSym = false>
 PM_HD bool sincpt(const FrameD &fs, V3 u0, Intercept &it) {
     const PMFrame &f = fs.f;
-    V3 p1, p2;
+    V3 p1, p2, p;
     RayHit h1, h2;
     const V3 x = mul3(u0, fs.inv_r);
     const double xx = dot(x, x);
@@ -447,7 +454,6 @@ PM_HD bool sincpt(const FrameD &fs, V3 u0, Intercept &it) {
     // epochs as CSPICE forms them: et - lt rounded to a double (granularity ulp(et) ~ 3e-8 s,
     // i.e. ~1e-6 km of target motion)
     double dt = (f.et - lt2) - f.t_ref;
-    V3 p;
     double L;
     if (fabs(dt1) > PM_T(kPixC)[kPixDt1Min] && h2.cos2 > PM_T(kPixC)[kPixGrazing]) {
         // The epochs e_0 = t_ref, e_1, e_2 of CSPICE's loop contract geometrically (ratio (e_2 - e_1) /
@@ -466,11 +472,10 @@ PM_HD bool sincpt(const FrameD &fs, V3 u0, Intercept &it) {
         const double ixxs = kSpinSym ? ixx : fma(lam, h2.ixx - h1.ixx, h2.ixx);
         const double hs = fast_sqrt_lite(fmax(1.0 - dot(pps, pps), 0.0) * ixxs);
         L = fma(lam, h2.a - h1.a, h2.a) - hs;
-        it.r = make_rot(fs, dt);
         if (kSpinSym) {
             it.p0 = axpy(-hs, u0, mul3(pps, fs.f.radii));
-            p = spin_fwd(fs, it.r, it.p0);
         } else {
+            it.r = make_rot(fs, dt);
             it.u = spin_fwd(fs, it.r, u0);
             p = axpy(-hs, it.u, mul3(pps, fs.f.radii));
         }
@@ -480,16 +485,15 @@ PM_HD bool sincpt(const FrameD &fs, V3 u0, Intercept &it) {
         if (!sincpt_converge<kSpinSym>(fs, u0, dt_c, p_c, L_c)) return false;
         dt = dt_c;
         L = L_c;
-        it.r = make_rot(fs, dt);
         if (kSpinSym) {
             it.p0 = p_c;
-            p = spin_fwd(fs, it.r, p_c);
         } else {
+            it.r = make_rot(fs, dt);
             p = p_c;
             it.u = spin_fwd(fs, it.r, u0);
         }
     }
-    it.p = p;
+    if (!kSpinSym) it.p = p;
     it.dt = dt;
     it.L = L;
     it.lt = L * fs.inv_c;
@@ -599,10 +603,10 @@ PM_HD double local_solar_time(const PMFrame &f, double lon_deg) {
     double ang = f.lon_sign * (lon_deg * PM_T(kPixC)[kPixRpd]) - f.sun_lon_lst;
     if (f.prograde == 0.0) ang = -ang;
     // fmod(ang, 2 pi) folded into [0, 2 pi): ang - k 2pi is exact for the small k here
-    const double k = floor(ang * PM_T(kMisc)[8]);
-    ang = fma(-k, PM_T(kMisc)[7], ang);
-    if (ang < 0.0) ang += PM_T(kMisc)[7];
-    if (ang >= PM_T(kMisc)[7]) ang -= PM_T(kMisc)[7];
+    const double k = floor(ang * PM_T(kMisc)[7]);
+    ang = fma(-k, PM_T(kMisc)[6], ang);
+    if (ang < 0.0) ang += PM_T(kMisc)[6];
+    if (ang >= PM_T(kMisc)[6]) ang -= PM_T(kMisc)[6];
     double sec = fma(ang, 86400.0 / kTwoPi, 43200.0);
     if (sec >= 86400.0) sec -= 86400.0;
     const int isec = (int)sec;  // floor: sec >= 0
@@ -846,7 +850,8 @@ constexpr uint64_t kSkyMask = bit(PM_RA) | bit(PM_DEC) | kKmMask | kLimbMask | k
 // (Body.ring_plane_coordinates(only_visible=False), body.py:2577-2615); the backplanes hide them.
 // kSpinSym = true is the path for frames with FrameD::spin_sym (the launchers pick it from the flag):
 // the intercept, the illumination angles and the radial velocity are taken in the body frame at t_ref,
-// where they equal the epoch frame's up to the bound of spin_sym, and only LON / LAT spin the point.
+// where they equal the epoch frame's up to the bound of spin_sym, and only LON / LAT spin the point - or,
+// with FrameD::spin_z, shift its longitude.
 template <bool kSky, uint64_t kFixedMask = 0, bool kRingAll = false, bool kSpinSym = false, class Sink>
 PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, Sink &out) {
     const PMFrame &f = fs.f;
@@ -892,12 +897,26 @@ PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, S
 
     double v_dist = nan;
     if (on_disc) {
-        const V3 p = it.p;
         if (mask & (kLonLatMask | kCentricMask)) {
             // _get_lonlat_img (body_xy.py:3284-3288), _get_lonlat_centric_img (:3349): the
             // east longitude and the cylindrical radius are shared by recpgr and reclat
+            V3 p = kSpinSym ? it.p0 : it.p;
+            double lon_e;
+            if (kSpinSym) {
+                // FrameD::spin_z: the spin about z keeps rho and z and turns the longitude by -omega_z dt
+                // (back into atan2's [-pi, pi]); otherwise the point is spun to its epoch
+                double turn = 0.0;
+                if (fs.spin_z)
+                    turn = f.omega[2] * it.dt;
+                else
+                    p = spin_fwd(fs, make_rot(fs, it.dt), p);
+                lon_e = fast_atan2(p.y, p.x) - turn;
+                if (lon_e > PM_T(kMisc)[2]) lon_e -= PM_T(kMisc)[6];
+                if (lon_e < -PM_T(kMisc)[2]) lon_e += PM_T(kMisc)[6];
+            } else {
+                lon_e = fast_atan2(p.y, p.x);
+            }
             const double rho = fast_sqrt_lite(fma(p.x, p.x, p.y * p.y));
-            const double lon_e = fast_atan2(p.y, p.x);
             if (mask & kLonLatMask) {
                 double l = f.lon_sign * lon_e;
                 if (l < 0.0) l += kTwoPi;
@@ -917,14 +936,14 @@ PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, S
         }
         if (mask & (kIllumMask | kStateMask | kRingMask)) {
             // spkcpt's converged light time is the intercept's own: |X| = |p - o|
-            const V3 kxp = cross(ld3(fs.k), kSpinSym ? it.p0 : p);  // shared by the inverse spin and omega x p
-            const V3 p0 = kSpinSym ? it.p0 : spin_bwd_c(fs, it.r, p, kxp);
+            const V3 kxp = cross(ld3(fs.k), kSpinSym ? it.p0 : it.p);  // shared by the inverse spin and omega x p
+            const V3 p0 = kSpinSym ? it.p0 : spin_bwd_c(fs, it.r, it.p, kxp);
             if (mask & kIllumMask) {  // _get_illumination_gie_img (body_xy.py:3661-3665)
                 Illum il;
                 if (kSpinSym)  // the angles of (n, s, e) all spun back to t_ref
                     illum_angles(mul3(p0, fs.nw), sun_vec0(fs, p0, it.dt), -u0, (mask & bit(PM_AZIMUTH)) != 0, il);
                 else
-                    illum_at(fs, p, p0, -it.u, it.r, it.dt, (mask & bit(PM_AZIMUTH)) != 0, il);
+                    illum_at(fs, it.p, p0, -it.u, it.r, it.dt, (mask & bit(PM_AZIMUTH)) != 0, il);
                 if (mask & bit(PM_PHASE)) out.put(PM_PHASE, il.phase * kDpr);
                 if (mask & bit(PM_INCIDENCE)) out.put(PM_INCIDENCE, il.incdnc * kDpr);
                 if (mask & bit(PM_EMISSION)) out.put(PM_EMISSION, il.emissn * kDpr);

@@ -34,10 +34,16 @@
 #define PM_DEV_TABLE(name, n, ...)                        \
     static __constant__ __align__(16) double name##_dev[n] = {__VA_ARGS__}; \
     static const double name##_host[n] = {__VA_ARGS__};
+// tables indexed per lane: global memory read through the read-only cache (a __constant__ operand
+// serialises a warp over its distinct addresses)
+#define PM_LDG_TABLE(name, n, ...)                        \
+    static __device__ __align__(16) double name##_dev[n] = {__VA_ARGS__}; \
+    static const double name##_host[n] = {__VA_ARGS__};
 #else
 #define PM_HD inline
 #define PM_HD_NOINLINE static
 #define PM_DEV_TABLE(name, n, ...) static const double name##_host[n] = {__VA_ARGS__};
+#define PM_LDG_TABLE(name, n, ...) static const double name##_host[n] = {__VA_ARGS__};
 #endif
 
 #ifdef __CUDA_ARCH__
@@ -56,26 +62,21 @@ constexpr double kDpr = 180.0 / kPi;
 constexpr double kRpd = kPi / 180.0;
 
 // minimax fits (mpmath, Chebyshev nodes, 60 digits; tools/fit_coefficients.py):
-//   atan(q) = q + q z A(z),  z = q^2 <= tan(pi/12)^2     |err| < 2e-17
 //   sin(x)  = x + x z S(z),  z = x^2 <= (pi/4)^2          |err| < 2e-17
 //   cos(x)  = 1 - z/2 + z^2 C(z)                           |err| < 5e-19
-PM_DEV_TABLE(kAtanC, 8, -0.33333333333333245175, 0.19999999999842781854, -0.14285714239619743943,
-             0.11111105950225735071, -0.090906243717563017737, 0.076837307398386464706,
-             -0.065219990167523964706, 0.04578335659104139954)
 PM_DEV_TABLE(kSinC, 6, -0.16666666666666664621, 0.008333333333330946103, -0.00019841269836754970194,
              2.7557316100683122624e-6, -2.5051131455447427132e-8, 1.5918101231677278624e-10)
 PM_DEV_TABLE(kCosC, 6, 0.041666666666666665387, -0.0013888888888887395746, 0.000024801587298763433277,
              -2.7557317270560382548e-7, 2.0876146024701932874e-9, -1.1382614869434128293e-11)
-// misc constants read as constant-bank operands: tan(pi/12), pi/4, pi/2, pi, 2/pi,
-// pi/2 split (hi, lo), 2 pi, 1/(2 pi), sqrt(3), pi/6, the zero guard of the square roots
-PM_DEV_TABLE(kMisc, 12, 0.2679491924311227064725537, 0.78539816339744830961566, 1.5707963267948966192313,
-             3.1415926535897932384626, 0.6366197723675813430755351, 1.570796326794896619231322,
-             6.12323399573676588613033e-17, 6.283185307179586476925287, 0.1591549430918953357688838,
-             1.732050807568877293527446, 0.5235987755982988730771072, 1.0e-300)
+// misc constants read as constant-bank operands: pi/4, pi/2, pi, 2/pi, pi/2 split (hi, lo), 2 pi,
+// 1/(2 pi), the zero guard of the square roots
+PM_DEV_TABLE(kMisc, 9, 0.78539816339744830961566, 1.5707963267948966192313, 3.1415926535897932384626,
+             0.6366197723675813430755351, 1.570796326794896619231322, 6.12323399573676588613033e-17,
+             6.283185307179586476925287, 0.1591549430918953357688838, 1.0e-300)
 
 // x + sqrt_guard() keeps an rsqrt seed finite at x == 0 (1e-300, read from the table like the other
 // full-mantissa literals instead of being rebuilt by two 32-bit moves at every use)
-PM_HD double sqrt_guard() { return PM_T(kMisc)[11]; }
+PM_HD double sqrt_guard() { return PM_T(kMisc)[8]; }
 
 // ---- MUFU seeds ----------------------------------------------------------------
 PM_HD double rcp_seed(double b) {
@@ -178,7 +179,7 @@ PM_HD_NOINLINE void sincos_lib(double x, double *s, double *c) {
 }
 // sin, cos for small arguments with a cold fallback for everything else
 PM_HD void sincos_small(double x, double &s, double &c) {
-    if (fabs(x) <= PM_T(kMisc)[1]) {
+    if (fabs(x) <= PM_T(kMisc)[0]) {
         sincos_quarter(x, s, c);
     } else {
         sincos_lib(x, &s, &c);
@@ -201,7 +202,7 @@ PM_HD void sincos_small2(double a, double b, double &sa, double &ca, double &sb,
     if (m <= 0.00390625) {  // 2^-8
         sincos_tiny(a, sa, ca);
         sincos_tiny(b, sb, cb);
-    } else if (m <= PM_T(kMisc)[1]) {
+    } else if (m <= PM_T(kMisc)[0]) {
         sincos_quarter(a, sa, ca);
         sincos_quarter(b, sb, cb);
     } else {
@@ -215,9 +216,9 @@ PM_HD void sincos_full(double x, double &s, double &c) {
         sincos_lib(x, &s, &c);
         return;
     }
-    const double k = rint(x * PM_T(kMisc)[4]);
-    double r = fma(-k, PM_T(kMisc)[5], x);
-    r = fma(-k, PM_T(kMisc)[6], r);
+    const double k = rint(x * PM_T(kMisc)[3]);
+    double r = fma(-k, PM_T(kMisc)[4], x);
+    r = fma(-k, PM_T(kMisc)[5], r);
     double sr, cr;
     sincos_quarter(r, sr, cr);
     const int n = (int)k;
@@ -265,22 +266,297 @@ PM_HD bool sign_bit(double x) {
 #endif
 }
 
-// atan(a / b) for 0 <= a <= b, b > 0: one division; the argument is folded into
-// |q| <= tan(pi/12) by  atan(a/b) = pi/6 + atan((sqrt(3) a - b) / (sqrt(3) b + a)).
-// Branch-free on purpose: independent calls then sit in one basic block and the
-// scheduler interleaves their dependent FMA chains.
+// Table-reduced arctangent (tools/fit_atan_table.py): series, and (t0, atan(t0)) at t0 = k / 256
+// atan(r) = r + r z (c1 + c2 z + c3 z^2), |r| <= 2^-8: relative truncation error 6.02e-21
+PM_DEV_TABLE(kAtanC, 3, -0.3333333333333333, 0.2, -0.14285714285714285)
+// (k / 2^8, atan(k / 2^8)) for k = 0 .. 256
+PM_LDG_TABLE(kAtanT, 514,
+             0.0, 0.0,
+             0.00390625, 0.0039062301319669718,
+             0.0078125, 0.007812341060101111,
+             0.01171875, 0.01171821360239413,
+             0.015625, 0.015623728620476831,
+             0.01953125, 0.019528767041413708,
+             0.0234375, 0.023433209879467586,
+             0.02734375, 0.027336938257824413,
+             0.03125, 0.031239833430268277,
+             0.03515625, 0.03514177680279678,
+             0.0390625, 0.03904264995516699,
+             0.04296875, 0.04294233466236217,
+             0.046875, 0.046840712915969654,
+             0.05078125, 0.05073766694546022,
+             0.0546875, 0.05463307923935948,
+             0.05859375, 0.05852683256630177,
+             0.0625, 0.06241880999595735,
+             0.06640625, 0.06630889491982349,
+             0.0703125, 0.07019697107187052,
+             0.07421875, 0.07408292254903373,
+             0.078125, 0.0779666338315423,
+             0.08203125, 0.08184798980307655,
+             0.0859375, 0.08572687577074481,
+             0.08984375, 0.08960317748487175,
+             0.09375, 0.09347678115858947,
+             0.09765625, 0.09734757348722367,
+             0.1015625, 0.10121544166746667,
+             0.10546875, 0.10508027341632953,
+             0.109375, 0.10894195698986579,
+             0.11328125, 0.11280038120165939,
+             0.1171875, 0.11665543544106935,
+             0.12109375, 0.12050700969122456,
+             0.125, 0.12435499454676144,
+             0.12890625, 0.12819928123129815,
+             0.1328125, 0.13203976161463876,
+             0.13671875, 0.1358763282297013,
+             0.140625, 0.13970887428916365,
+             0.14453125, 0.14353729370182122,
+             0.1484375, 0.14736148108865163,
+             0.15234375, 0.15118133179858007,
+             0.15625, 0.15499674192394097,
+             0.16015625, 0.15880760831563107,
+             0.1640625, 0.16261382859794857,
+             0.16796875, 0.16641530118311493,
+             0.171875, 0.1702119252854744,
+             0.17578125, 0.1740036009353677,
+             0.1796875, 0.17779022899267607,
+             0.18359375, 0.18157171116003218,
+             0.1875, 0.18534794999569476,
+             0.19140625, 0.189118848926084,
+             0.1953125, 0.19288431225797467,
+             0.19921875, 0.196644245190345,
+             0.203125, 0.2003985538258785,
+             0.20703125, 0.20414714518211702,
+             0.2109375, 0.207889927202263,
+             0.21484375, 0.21162680876562978,
+             0.21875, 0.21535769969773805,
+             0.22265625, 0.21908251078005778,
+             0.2265625, 0.22280115375939452,
+             0.23046875, 0.22651354135691962,
+             0.234375, 0.23021958727684372,
+             0.23828125, 0.23391920621473344,
+             0.2421875, 0.23761231386547124,
+             0.24609375, 0.24129882693085883,
+             0.25, 0.24497866312686414,
+             0.25390625, 0.24865174119051325,
+             0.2578125, 0.2523179808864272,
+             0.26171875, 0.25597730301300553,
+             0.265625, 0.2596296294082575,
+             0.26953125, 0.2632748829552824,
+             0.2734375, 0.26691298758740045,
+             0.27734375, 0.2705438682929366,
+             0.28125, 0.2741674511196588,
+             0.28515625, 0.27778366317887326,
+             0.2890625, 0.28139243264917846,
+             0.29296875, 0.2849936887798813,
+             0.296875, 0.2885873618940774,
+             0.30078125, 0.29217338339139876,
+             0.3046875, 0.29575168575043154,
+             0.30859375, 0.29932220253080744,
+             0.3125, 0.3028848683749714,
+             0.31640625, 0.3064396190096301,
+             0.3203125, 0.30998639124688343,
+             0.32421875, 0.3135251229850439,
+             0.328125, 0.31705575320914703,
+             0.33203125, 0.320578221991157,
+             0.3359375, 0.3240924704898717,
+             0.33984375, 0.32759844095053087,
+             0.34375, 0.3310960767041321,
+             0.34765625, 0.334585322166459,
+             0.3515625, 0.33806612283682547,
+             0.35546875, 0.3415384252965417,
+             0.359375, 0.34500217720710513,
+             0.36328125, 0.34845732730812207,
+             0.3671875, 0.3519038254149648,
+             0.37109375, 0.35534162241616835,
+             0.375, 0.35877067027057225,
+             0.37890625, 0.3621909220042122,
+             0.3828125, 0.3656023317069669,
+             0.38671875, 0.3690048545289644,
+             0.390625, 0.3723984466767542,
+             0.39453125, 0.37578306540924894,
+             0.3984375, 0.3791586690334418,
+             0.40234375, 0.38252521689990515,
+             0.40625, 0.38588266939807375,
+             0.41015625, 0.3892309879513207,
+             0.4140625, 0.3925701350118286,
+             0.41796875, 0.3959000740552629,
+             0.421875, 0.39922076957525254,
+             0.42578125, 0.4025321870776825,
+             0.4296875, 0.4058342930748041,
+             0.43359375, 0.4091270550791683,
+             0.4375, 0.4124104415973873,
+             0.44140625, 0.4156844221237294,
+             0.4453125, 0.41894896713355284,
+             0.44921875, 0.4222040480765836,
+             0.453125, 0.42544963737004227,
+             0.45703125, 0.4286857083916258,
+             0.4609375, 0.4319122354723482,
+             0.46484375, 0.43512919388924687,
+             0.46875, 0.43833655985795783,
+             0.47265625, 0.44153431052516673,
+             0.4765625, 0.44472242396093936,
+             0.48046875, 0.4479008791509373,
+             0.484375, 0.4510696559885235,
+             0.48828125, 0.4542287352667625,
+             0.4921875, 0.4573780986703208,
+             0.49609375, 0.4605177287672711,
+             0.5, 0.4636476090008061,
+             0.50390625, 0.4667677236808665,
+             0.5078125, 0.46987805797568694,
+             0.51171875, 0.4729785979032656,
+             0.515625, 0.4760693303227612,
+             0.51953125, 0.47915024292582253,
+             0.5234375, 0.48222132422785374,
+             0.52734375, 0.4852825635592213,
+             0.53125, 0.48833395105640554,
+             0.53515625, 0.4913754776531019,
+             0.5390625, 0.49440713507127537,
+             0.54296875, 0.49742891581217225,
+             0.546875, 0.5004408131472942,
+             0.55078125, 0.5034428211093364,
+             0.5546875, 0.5064349344830967,
+             0.55859375, 0.5094171487963564,
+             0.5625, 0.5123894603107377,
+             0.56640625, 0.5153518660125433,
+             0.5703125, 0.518304363603578,
+             0.57421875, 0.5212469514919582,
+             0.578125, 0.5241796287829132,
+             0.58203125, 0.5271023952695796,
+             0.5859375, 0.5300152514237931,
+             0.58984375, 0.5329181983868821,
+             0.59375, 0.5358112379604637,
+             0.59765625, 0.5386943725972466,
+             0.6015625, 0.541567605391845,
+             0.60546875, 0.5444309400716031,
+             0.609375, 0.5472843809874369,
+             0.61328125, 0.5501279331046931,
+             0.6171875, 0.5529616019940283,
+             0.62109375, 0.5557853938223135,
+             0.625, 0.5585993153435624,
+             0.62890625, 0.5614033738898894,
+             0.6328125, 0.5641975773624976,
+             0.63671875, 0.5669819342227005,
+             0.640625, 0.5697564534829784,
+             0.64453125, 0.5725211446980724,
+             0.6484375, 0.5752760179561178,
+             0.65234375, 0.5780210838698195,
+             0.65625, 0.5807563535676704,
+             0.66015625, 0.5834818386852149,
+             0.6640625, 0.5861975513563606,
+             0.66796875, 0.5889035042047381,
+             0.671875, 0.5915997103351114,
+             0.67578125, 0.5942861833248413,
+             0.6796875, 0.5969629372154015,
+             0.68359375, 0.5996299865039514,
+             0.6875, 0.6022873461349642,
+             0.69140625, 0.604935031491914,
+             0.6953125, 0.6075730583890224,
+             0.69921875, 0.6102014430630652,
+             0.703125, 0.6128202021652414,
+             0.70703125, 0.6154293527531051,
+             0.7109375, 0.6180289122825618,
+             0.71484375, 0.6206188985999295,
+             0.71875, 0.6231993299340659,
+             0.72265625, 0.6257702248885632,
+             0.7265625, 0.6283316024340097,
+             0.73046875, 0.630883481900322,
+             0.734375, 0.6334258829691446,
+             0.73828125, 0.6359588256663214,
+             0.7421875, 0.6384823303544376,
+             0.74609375, 0.6409964177254321,
+             0.75, 0.6435011087932844,
+             0.75390625, 0.6459964248867716,
+             0.7578125, 0.6484823876423006,
+             0.76171875, 0.6509590189968124,
+             0.765625, 0.6534263411807619,
+             0.76953125, 0.6558843767111708,
+             0.7734375, 0.658333148384756,
+             0.77734375, 0.6607726792711327,
+             0.78125, 0.6632029927060933,
+             0.78515625, 0.665624112284961,
+             0.7890625, 0.6680360618560202,
+             0.79296875, 0.6704388655140214,
+             0.796875, 0.6728325475937632,
+             0.80078125, 0.6752171326637499,
+             0.8046875, 0.6775926455199252,
+             0.80859375, 0.6799591111794819,
+             0.8125, 0.6823165548747481,
+             0.81640625, 0.684665002047149,
+             0.8203125, 0.687004478341245,
+             0.82421875, 0.6893350095988459,
+             0.828125, 0.6916566218531999,
+             0.83203125, 0.6939693413232598,
+             0.8359375, 0.6962731944080236,
+             0.83984375, 0.69856820768095,
+             0.84375, 0.7008544078844502,
+             0.84765625, 0.7031318219244538,
+             0.8515625, 0.705400476865049,
+             0.85546875, 0.7076603999231981,
+             0.859375, 0.7099116184635249,
+             0.86328125, 0.7121541599931787,
+             0.8671875, 0.714388052156769,
+             0.87109375, 0.7166133227313746,
+             0.875, 0.7188299996216245,
+             0.87890625, 0.7210381108548516,
+             0.8828125, 0.7232376845763179,
+             0.88671875, 0.7254287490445107,
+             0.890625, 0.7276113326265107,
+             0.89453125, 0.7297854637934291,
+             0.8984375, 0.7319511711159166,
+             0.90234375, 0.7341084832597397,
+             0.90625, 0.7362574289814281,
+             0.91015625, 0.7383980371239895,
+             0.9140625, 0.7405303366126927,
+             0.91796875, 0.7426543564509179,
+             0.921875, 0.7447701257160751,
+             0.92578125, 0.7468776735555875,
+             0.9296875, 0.7489770291829414,
+             0.93359375, 0.7510682218738024,
+             0.9375, 0.7531512809621944,
+             0.94140625, 0.7552262358367449,
+             0.9453125, 0.7572931159369924,
+             0.94921875, 0.759351950749758,
+             0.953125, 0.7614027698055784,
+             0.95703125, 0.7634456026752018,
+             0.9609375, 0.7654804789661445,
+             0.96484375, 0.7675074283193083,
+             0.96875, 0.7695264804056583,
+             0.97265625, 0.7715376649229596,
+             0.9765625, 0.7735410115925735,
+             0.98046875, 0.7755365501563117,
+             0.984375, 0.7775243103733478,
+             0.98828125, 0.7795043220171863,
+             0.9921875, 0.7814766148726883,
+             0.99609375, 0.7834412187331518,
+             1.0, 0.7853981633974483)
+
+PM_HD uint32_t lo_word(double x) {
+#ifdef __CUDA_ARCH__
+    return (uint32_t)__double2loint(x);
+#else
+    uint64_t u;
+    memcpy(&u, &x, 8);
+    return (uint32_t)u;
+#endif
+}
+// atan(a / b) for 0 <= a <= b, b > 0: atan(t0) + atan(r), r = (a - t0 b) / (b + t0 a), one division.
+// k = round(256 a / b) from the reciprocal seed: adding 1.5 * 2^44 (ulp 2^-8) leaves it in the low
+// mantissa word.  A seed ~20 bits short can move k by one, which keeps |r| <= 2^-8, the range of the
+// series.  The clamp keeps a NaN quotient (0 / 0, NaN in) inside the table; the result is NaN anyway.
+// Branch-free on purpose: independent calls then sit in one basic block and the scheduler interleaves
+// their dependent FMA chains.
 PM_HD double atan_ratio(double mn, double mx) {
-    const bool hi = mn > mx * PM_T(kMisc)[0];
-    const double num = hi ? fma(PM_T(kMisc)[9], mn, -mx) : mn;
-    const double den = hi ? fma(PM_T(kMisc)[9], mx, mn) : mx;
-    const double q = fast_div_lite(num, den);
-    const double z = q * q;
-    double p = PM_T(kAtanC)[7];
-#pragma unroll
-    for (int i = 6; i >= 0; i--) p = fma(p, z, PM_T(kAtanC)[i]);
-    double r = fma(q * z, p, q);
-    if (hi) r += PM_T(kMisc)[10];
-    return r;
+    const uint32_t kr = lo_word(fma(mn, rcp_seed(mx), 26388279066624.0));
+    const uint32_t k = kr < 256u ? kr : 256u;
+#ifdef __CUDA_ARCH__
+    const double2 e = __ldg(reinterpret_cast<const double2 *>(kAtanT_dev) + k);
+    const double t0 = e.x, a0 = e.y;
+#else
+    const double t0 = kAtanT_host[2 * k], a0 = kAtanT_host[2 * k + 1];
+#endif
+    const double r = fast_div_lite(fma(-t0, mx, mn), fma(t0, mn, mx));
+    const double z = r * r;
+    const double p = fma(fma(PM_T(kAtanC)[2], z, PM_T(kAtanC)[1]), z, PM_T(kAtanC)[0]);
+    return a0 + fma(r * z, p, r);
 }
 // atan2(y, x), full quadrant, atan2(0, 0) = 0 (the convention recrad / reclat / recgeo
 // apply explicitly).  NaN in -> NaN out.
@@ -289,8 +565,8 @@ PM_HD double fast_atan2(double y, double x) {
     const bool sw = pos_gt(ay, ax);
     const double mx = sw ? ay : ax, mn = sw ? ax : ay;
     double r = atan_ratio(mn, mx);  // 0 / 0 -> NaN, replaced below
-    if (sw) r = PM_T(kMisc)[2] - r;
-    if (sign_bit(x)) r = PM_T(kMisc)[3] - r;
+    if (sw) r = PM_T(kMisc)[1] - r;
+    if (sign_bit(x)) r = PM_T(kMisc)[2] - r;
     r = with_sign_of(r, y);
     return (mx == 0.0) ? 0.0 : r;
 }
@@ -300,8 +576,8 @@ PM_HD double fast_atan2_ypos(double y, double x) {
     const bool sw = pos_gt(abs_bits(y), ax);
     const double mx = sw ? y : ax, mn = sw ? ax : y;
     double r = atan_ratio(mn, mx);
-    if (sw) r = PM_T(kMisc)[2] - r;
-    if (sign_bit(x)) r = PM_T(kMisc)[3] - r;
+    if (sw) r = PM_T(kMisc)[1] - r;
+    if (sign_bit(x)) r = PM_T(kMisc)[2] - r;
     return r;
 }
 // atan2(y, x) for x >= 0 and (x, y) != (0, 0): angle in [-pi/2, pi/2] (latitudes)
@@ -310,7 +586,7 @@ PM_HD double fast_atan2_xpos(double y, double x) {
     const bool sw = pos_gt(ay, abs_bits(x));
     const double mx = sw ? ay : x, mn = sw ? x : ay;
     double r = atan_ratio(mn, mx);
-    if (sw) r = PM_T(kMisc)[2] - r;
+    if (sw) r = PM_T(kMisc)[1] - r;
     return with_sign_of(r, y);
 }
 // acos(x); NaN for |x| > 1 like the libm routine
