@@ -198,6 +198,12 @@ def random_geometry(seed):
     fast and slow rotators), observer anywhere between 1.3 and 1e5 body radii in a random direction with a
     random velocity of up to ~50 km/s relative to the target, random disc position / size / rotation.
     Returns (frame, nx, ny, label)."""
+    bc, disc, alt, label = random_geometry_parts(seed)
+    return img_case(bc, *disc, alt), disc[0], disc[1], label
+
+
+def random_geometry_parts(seed):
+    """random_geometry(seed) before packing: (constants, (nx, ny, x0, y0, r0, rotation in degrees), alt, label)."""
     import planetmapper_b200 as pm
     from planetmapper_b200.minispice.kepler import KeplerOrbitProvider
 
@@ -221,7 +227,7 @@ def random_geometry(seed):
     rot = rng.uniform(0, 360)
     # every fourth geometry on an altitude-adjusted surface (get_backplane_img(..., alt=...), body_xy.py:2586)
     alt = float(rng.uniform(-0.01, 0.05) * rmax) if seed % 4 == 3 else 0.0
-    return (img_case(bc, nx, ny, x0, y0, r0, rot, alt), nx, ny,
+    return (bc, (nx, ny, x0, y0, r0, rot), alt,
             f'seed {seed}: {target} D/r={dist / rmax:.3g} {nx}x{ny} r0={r0:.1f} rot={rot:.0f} alt={alt:.0f}')
 
 

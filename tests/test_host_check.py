@@ -327,24 +327,30 @@ int main(int argc, char **argv) {
 """
 
 
-def build_ld_oracle(bdir):
-    """Compiles the oracle with every `double` turned into an 80-bit `long double` into `bdir` and
-    returns run(frame, nx, ny) -> (26, ny, nx) planes (rounded to double at the very end)."""
+def write_ld_sources(bdir):
+    """Writes the oracle with every `double` turned into an 80-bit `long double` into `bdir`: pm_oracle_ld.c and
+    the headers it includes.  A driver declares what it calls from it (or includes the .c to reach its static
+    routines) with "pm_b200_ld.h", whose PMFrame holds long doubles."""
     import re
 
     root = os.path.dirname(HERE)
-    exe = os.path.join(bdir, 'oracle_ld')
-    src_c = os.path.join(root, 'oracle', 'pm_oracle.c')
 
     def ld(text):
         return re.sub(r'\bdouble\b', 'long double', text)
-    c = ld(open(src_c).read()).replace('#include <math.h>', '#include <tgmath.h>')
+    c = ld(open(os.path.join(root, 'oracle', 'pm_oracle.c')).read()).replace('#include <math.h>', '#include <tgmath.h>')
     c = c.replace('#define PI 3.14159265358979323846264338327950288\n',
                   '#define PI 3.14159265358979323846264338327950288L\n')
     h = ld(open(os.path.join(root, 'oracle', 'pm_oracle.h')).read()).replace('"../include/pm_b200.h"', '"pm_b200_ld.h"')
     open(os.path.join(bdir, 'pm_oracle_ld.c'), 'w').write(c)
     open(os.path.join(bdir, 'pm_oracle.h'), 'w').write(h)
     open(os.path.join(bdir, 'pm_b200_ld.h'), 'w').write(ld(open(os.path.join(root, 'include', 'pm_b200.h')).read()))
+
+
+def build_ld_oracle(bdir):
+    """Compiles the oracle with every `double` turned into an 80-bit `long double` into `bdir` and
+    returns run(frame, nx, ny) -> (26, ny, nx) planes (rounded to double at the very end)."""
+    exe = os.path.join(bdir, 'oracle_ld')
+    write_ld_sources(bdir)
     open(os.path.join(bdir, 'drv.c'), 'w').write(LD_DRV)
     subprocess.run(['gcc', '-O2', '-w', '-fopenmp', '-o', exe, 'drv.c', 'pm_oracle_ld.c', '-lm'], cwd=bdir, check=True,
                    capture_output=True)
