@@ -59,7 +59,7 @@ struct PlaneSink {
 // Image direction: all requested backplanes for every pixel of every frame.
 // ---------------------------------------------------------------------------------
 // Pixels idx, idx + 128, ... of this CTA's tile, every requested plane of each
-template <bool kSky, uint64_t kFixedMask, bool kSpinSym>
+template <bool kSky, uint64_t kFixedMask, int kFrame>
 __device__ __forceinline__ void img_tile(const FrameD &fs, uint32_t tile, uint32_t nx, uint32_t npx, int per_thread,
                                          uint64_t mask, const PlaneOffsets &po, double *__restrict__ out) {
     uint32_t idx = tile * (uint32_t)(kBlock * per_thread) + threadIdx.x;
@@ -67,7 +67,7 @@ __device__ __forceinline__ void img_tile(const FrameD &fs, uint32_t tile, uint32
 #pragma unroll 1
     for (int r = 0; r < per_thread && idx < npx; r++) {
         PlaneSink sink{reinterpret_cast<char *>(out + idx), po};
-        image_pixel<kSky, kFixedMask, false, kSpinSym>(fs, (double)xi, (double)yi, mask, sink);
+        image_pixel<kSky, kFixedMask, false, kFrame>(fs, (double)xi, (double)yi, mask, sink);
         idx += kBlock;
         xi += kBlock;
         while (xi >= nx) {
@@ -78,7 +78,8 @@ __device__ __forceinline__ void img_tile(const FrameD &fs, uint32_t tile, uint32
 }
 
 // Batched launch (time series): frame blockIdx.y is staged in shared memory by the CTA.  The frame's
-// spin_sym flag is uniform over the CTA, so the branch on it does not diverge.
+// spin_sym flag is uniform over the CTA, so the branch on it does not diverge; kFrameSpinSym tests the
+// frame's other flags at run time.
 template <bool kSky, uint64_t kFixedMask>
 __global__ void __launch_bounds__(kBlock, 4) backplanes_img_kernel(const PMFrame *__restrict__ frames, uint32_t nx,
                                                                    uint32_t npx, int per_thread, uint64_t mask,
@@ -88,9 +89,9 @@ __global__ void __launch_bounds__(kBlock, 4) backplanes_img_kernel(const PMFrame
     load_frame(fs, frames + blockIdx.y);
     double *out = out_all + (int64_t)blockIdx.y * __popcll(mask) * npx;
     if (fs.spin_sym)
-        img_tile<kSky, kFixedMask, true>(fs, blockIdx.x, nx, npx, per_thread, mask, po, out);
+        img_tile<kSky, kFixedMask, kFrameSpinSym>(fs, blockIdx.x, nx, npx, per_thread, mask, po, out);
     else
-        img_tile<kSky, kFixedMask, false>(fs, blockIdx.x, nx, npx, per_thread, mask, po, out);
+        img_tile<kSky, kFixedMask, kFrameGeneral>(fs, blockIdx.x, nx, npx, per_thread, mask, po, out);
 }
 
 // Single frame: the finished constants (derived on the host with the same exactly rounded
@@ -108,11 +109,11 @@ __device__ __forceinline__ uint32_t centre_out_tile(uint32_t k, uint32_t n_tiles
     if (j <= min(lo, hi)) return (k & 1u) ? centre + j : centre - j;
     return lo < hi ? k : n_tiles - 1u - k;  // one side exhausted: the rest in order, moving away
 }
-template <bool kSky, uint64_t kFixedMask, bool kSpinSym>
+template <bool kSky, uint64_t kFixedMask, int kFrame>
 __global__ void __launch_bounds__(kBlock, kImgParamCtas) backplanes_img_param_kernel(
     const __grid_constant__ FrameD fs, uint32_t nx, uint32_t npx, int per_thread, uint32_t centre_tile, uint64_t mask,
     const __grid_constant__ PlaneOffsets po, double *__restrict__ out) {
-    img_tile<kSky, kFixedMask, kSpinSym>(fs, centre_out_tile(blockIdx.x, gridDim.x, centre_tile), nx, npx, per_thread,
+    img_tile<kSky, kFixedMask, kFrame>(fs, centre_out_tile(blockIdx.x, gridDim.x, centre_tile), nx, npx, per_thread,
                                          mask, po, out);
 }
 
@@ -120,7 +121,7 @@ __global__ void __launch_bounds__(kBlock, kImgParamCtas) backplanes_img_param_ke
 // Image direction at arbitrary positions (pm_backplanes_points_host): the per-pixel code of the
 // single-frame image kernel on a list of (x, y), tiled like map_tile; output plane stride = n
 // ---------------------------------------------------------------------------------
-template <bool kSky, bool kRingAll, bool kSpinSym>
+template <bool kSky, bool kRingAll, int kFrame>
 __global__ void __launch_bounds__(kBlock, 4) backplanes_points_param_kernel(const __grid_constant__ FrameD fs,
                                                                             const double *__restrict__ x_in,
                                                                             const double *__restrict__ y_in,
@@ -133,7 +134,7 @@ __global__ void __launch_bounds__(kBlock, 4) backplanes_points_param_kernel(cons
         const int64_t idx = first + r * kBlock;
         if (idx >= n) break;
         PlaneSink sink{reinterpret_cast<char *>(out + idx), po};
-        image_point<kSky, kRingAll, kSpinSym>(fs, __ldg(x_in + idx), __ldg(y_in + idx), mask, sink);
+        image_point<kSky, kRingAll, kFrame>(fs, __ldg(x_in + idx), __ldg(y_in + idx), mask, sink);
     }
 }
 
@@ -454,18 +455,18 @@ cudaError_t launch_backplanes_img(const PMFrame *frames, int n_frames, int nx, i
     count_launches(1);
     return cudaGetLastError();
 }
-template <bool kSpinSym>
+template <int kFrame>
 static void launch_img_param(const FrameD &fs, dim3 grid, uint32_t nx, uint32_t npx, int per, uint32_t centre,
                              uint64_t mask, const PlaneOffsets &po, double *out, cudaStream_t st) {
     if (mask == kDefaultStackMask)
-        backplanes_img_param_kernel<false, kDefaultStackMask, kSpinSym><<<grid, kBlock, 0, st>>>(fs, nx, npx, per, centre,
-                                                                                                mask, po, out);
+        backplanes_img_param_kernel<false, kDefaultStackMask, kFrame><<<grid, kBlock, 0, st>>>(fs, nx, npx, per, centre,
+                                                                                              mask, po, out);
     else if (mask & kSkyMask)
-        backplanes_img_param_kernel<true, 0, kSpinSym><<<grid, kBlock, 0, st>>>(fs, nx, npx, per, centre, mask, po, out);
+        backplanes_img_param_kernel<true, 0, kFrame><<<grid, kBlock, 0, st>>>(fs, nx, npx, per, centre, mask, po, out);
     else
-        backplanes_img_param_kernel<false, 0, kSpinSym><<<grid, kBlock, 0, st>>>(fs, nx, npx, per, centre, mask, po, out);
+        backplanes_img_param_kernel<false, 0, kFrame><<<grid, kBlock, 0, st>>>(fs, nx, npx, per, centre, mask, po, out);
 }
-// single frame given on the HOST: constants derived here, passed by value; the frame's spin_sym flag
+// single frame given on the HOST: constants derived here, passed by value; the frame's kind (frame_kind)
 // picks the instantiation, so each kernel carries one path's code and registers only
 cudaError_t launch_backplanes_img_host(const PMFrame *frame_host, int nx, int ny, uint64_t mask, double *out,
                                        int sm_count, cudaStream_t st) {
@@ -487,23 +488,26 @@ cudaError_t launch_backplanes_img_host(const PMFrame *frame_host, int nx, int ny
     static const bool linear = tune_int("PM_IMG_ORDER", 1) == 0;
     if (linear) ct = 0;
     const uint32_t centre = (uint32_t)(ct < 0 ? 0 : (ct >= n_tiles ? n_tiles - 1 : ct));
-    if (fs.spin_sym)
-        launch_img_param<true>(fs, grid, (uint32_t)nx, (uint32_t)npx, per, centre, mask, po, out, st);
+    const int kind = frame_kind(fs);
+    if (kind == kFrameSpinZ)
+        launch_img_param<kFrameSpinZ>(fs, grid, (uint32_t)nx, (uint32_t)npx, per, centre, mask, po, out, st);
+    else if (kind == kFrameSpinSym)
+        launch_img_param<kFrameSpinSym>(fs, grid, (uint32_t)nx, (uint32_t)npx, per, centre, mask, po, out, st);
     else
-        launch_img_param<false>(fs, grid, (uint32_t)nx, (uint32_t)npx, per, centre, mask, po, out, st);
+        launch_img_param<kFrameGeneral>(fs, grid, (uint32_t)nx, (uint32_t)npx, per, centre, mask, po, out, st);
     count_launches(1);
     return cudaGetLastError();
 }
-template <bool kSpinSym>
+template <int kFrame>
 static void launch_points_param(const FrameD &fs, unsigned grid, const double *x, const double *y, int64_t n,
                                 uint64_t mask, uint32_t flags, const PlaneOffsets &po, double *out, cudaStream_t st) {
     // the ring planes are sky planes: without a sky plane PM_FLAG_RING_ALL has nothing to change
     if (!(mask & kSkyMask))
-        backplanes_points_param_kernel<false, false, kSpinSym><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
+        backplanes_points_param_kernel<false, false, kFrame><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
     else if (flags & PM_FLAG_RING_ALL)
-        backplanes_points_param_kernel<true, true, kSpinSym><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
+        backplanes_points_param_kernel<true, true, kFrame><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
     else
-        backplanes_points_param_kernel<true, false, kSpinSym><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
+        backplanes_points_param_kernel<true, false, kFrame><<<grid, kBlock, 0, st>>>(fs, x, y, n, mask, po, out);
 }
 // n arbitrary image positions of ONE frame given on the HOST (constants derived here, as above)
 cudaError_t launch_backplanes_points_host(const PMFrame *frame_host, const double *x, const double *y, int64_t n,
@@ -513,9 +517,9 @@ cudaError_t launch_backplanes_points_host(const PMFrame *frame_host, const doubl
     const PlaneOffsets po = make_plane_offsets(mask, n);
     const unsigned grid = chunks_for(n);
     if (fs.spin_sym)
-        launch_points_param<true>(fs, grid, x, y, n, mask, flags, po, out, st);
+        launch_points_param<kFrameSpinSym>(fs, grid, x, y, n, mask, flags, po, out, st);
     else
-        launch_points_param<false>(fs, grid, x, y, n, mask, flags, po, out, st);
+        launch_points_param<kFrameGeneral>(fs, grid, x, y, n, mask, flags, po, out, st);
     count_launches(1);
     return cudaGetLastError();
 }

@@ -88,6 +88,15 @@ struct FrameD {
     int spin_z;        // spin_sym with the spin axis on z: LON / LAT are taken from the point at t_ref as well
 };
 
+// Which per-pixel path a frame takes (image_pixel's kFrame).  The launchers pick it from the frame's flags
+// (frame_kind); kFrameSpinSym tests spin_z and biaxial at run time, kFrameSpinZ has both set at compile
+// time, so its instantiation carries neither geodetic_general nor the spin of the point.
+enum FrameKind : int {
+    kFrameGeneral = 0,  // any ellipsoid: the observer, the ray and the Sun are spun to every epoch
+    kFrameSpinSym = 1,  // FrameD::spin_sym
+    kFrameSpinZ = 2,    // FrameD::spin_sym, spin_z and biaxial (Jupiter, Saturn, every sphere spinning about z)
+};
+
 constexpr int kDeriveItems = 13;
 
 // Exactly rounded IEEE operations for the derived constants.  The derivation runs in two places -
@@ -229,6 +238,10 @@ inline void load_frame_host(FrameD &s, const PMFrame *g) {
     s.f = *g;
     for (int i = 0; i < kDeriveItems; i++) derive_frame_item(s, i);
 }
+inline int frame_kind(const FrameD &s) {
+    if (!s.spin_sym) return kFrameGeneral;
+    return (s.spin_z && s.biaxial) ? kFrameSpinZ : kFrameSpinSym;
+}
 
 // cos^2 (scaled-space emission) below which sincpt iterates to convergence: emission > ~86.9 deg.
 // Above it the fixed-point step's own error (the light time is not linear in the epoch:
@@ -244,12 +257,10 @@ constexpr double kGrazingCos2 = PM_GRAZING_COS2;
 enum PixC {
     kPixDt1Min = 0,   // sincpt: |dt1| above which the two-pass fixed point is used
     kPixGrazing = 1,  // sincpt: kGrazingCos2
-    kPixInv60 = 2,    // local_solar_time: 1/60, 1/3600
-    kPixInv3600 = 3,
-    kPixRpd = 4,      // local_solar_time: rad per deg
-    kPixBetaMax = 5,  // doppler_factor / radial_velocity: |v| / c bound of the series
+    kPixRpd = 2,      // local_solar_time: rad per deg
+    kPixBetaMax = 3,  // doppler_factor / radial_velocity: |v| / c bound of the series
 };
-PM_DEV_TABLE(kPixC, 6, 1.0e-6, kGrazingCos2, 1.0 / 60.0, 1.0 / 3600.0, kRpd, 1.0e-3)
+PM_DEV_TABLE(kPixC, 4, 1.0e-6, kGrazingCos2, kRpd, 1.0e-3)
 
 // ---------------------------------------------------------------------------------
 // Frame spin: body frame at t_ref  <->  body frame at t_ref + dt
@@ -596,9 +607,33 @@ PM_HD void reclat_angles(V3 v, double &lon, double &lat) {
     lon = fast_atan2(v.y, v.x);
 }
 
+// mn / 60 and sc / 3600 of the local solar time, correctly rounded (the compiler folds each quotient): entries
+// [mn] and [60 + sc].  Per lane indices, so read like the arctangent table, through the read-only cache.
+PM_LDG_TABLE(kLstT, 120,
+             0 / 60.0, 1 / 60.0, 2 / 60.0, 3 / 60.0, 4 / 60.0, 5 / 60.0, 6 / 60.0, 7 / 60.0, 8 / 60.0, 9 / 60.0,
+             10 / 60.0, 11 / 60.0, 12 / 60.0, 13 / 60.0, 14 / 60.0, 15 / 60.0, 16 / 60.0, 17 / 60.0, 18 / 60.0, 19 / 60.0,
+             20 / 60.0, 21 / 60.0, 22 / 60.0, 23 / 60.0, 24 / 60.0, 25 / 60.0, 26 / 60.0, 27 / 60.0, 28 / 60.0, 29 / 60.0,
+             30 / 60.0, 31 / 60.0, 32 / 60.0, 33 / 60.0, 34 / 60.0, 35 / 60.0, 36 / 60.0, 37 / 60.0, 38 / 60.0, 39 / 60.0,
+             40 / 60.0, 41 / 60.0, 42 / 60.0, 43 / 60.0, 44 / 60.0, 45 / 60.0, 46 / 60.0, 47 / 60.0, 48 / 60.0, 49 / 60.0,
+             50 / 60.0, 51 / 60.0, 52 / 60.0, 53 / 60.0, 54 / 60.0, 55 / 60.0, 56 / 60.0, 57 / 60.0, 58 / 60.0, 59 / 60.0,
+             0 / 3600.0, 1 / 3600.0, 2 / 3600.0, 3 / 3600.0, 4 / 3600.0, 5 / 3600.0, 6 / 3600.0, 7 / 3600.0, 8 / 3600.0, 9 / 3600.0,
+             10 / 3600.0, 11 / 3600.0, 12 / 3600.0, 13 / 3600.0, 14 / 3600.0, 15 / 3600.0, 16 / 3600.0, 17 / 3600.0, 18 / 3600.0, 19 / 3600.0,
+             20 / 3600.0, 21 / 3600.0, 22 / 3600.0, 23 / 3600.0, 24 / 3600.0, 25 / 3600.0, 26 / 3600.0, 27 / 3600.0, 28 / 3600.0, 29 / 3600.0,
+             30 / 3600.0, 31 / 3600.0, 32 / 3600.0, 33 / 3600.0, 34 / 3600.0, 35 / 3600.0, 36 / 3600.0, 37 / 3600.0, 38 / 3600.0, 39 / 3600.0,
+             40 / 3600.0, 41 / 3600.0, 42 / 3600.0, 43 / 3600.0, 44 / 3600.0, 45 / 3600.0, 46 / 3600.0, 47 / 3600.0, 48 / 3600.0, 49 / 3600.0,
+             50 / 3600.0, 51 / 3600.0, 52 / 3600.0, 53 / 3600.0, 54 / 3600.0, 55 / 3600.0, 56 / 3600.0, 57 / 3600.0, 58 / 3600.0, 59 / 3600.0)
+PM_HD void lst_fractions(int mn, int sc, double &qm, double &qs) {
+#ifdef __CUDA_ARCH__
+    qm = __ldg(kLstT_dev + mn);
+    qs = __ldg(kLstT_dev + 60 + sc);
+#else
+    qm = kLstT_host[mn];
+    qs = kLstT_host[60 + sc];
+#endif
+}
 // Body.local_solar_time_from_lon (body.py:2364-2398) -> spice.et2lst 'planetographic'
 // lon_deg finite.  Whole seconds are split with integer arithmetic; the two divisions
-// of the reference's `hr + mn / 60 + sc / 3600` are reproduced correctly rounded.
+// of the reference's `hr + mn / 60 + sc / 3600` are read correctly rounded from kLstT.
 PM_HD double local_solar_time(const PMFrame &f, double lon_deg) {
     double ang = f.lon_sign * (lon_deg * PM_T(kPixC)[kPixRpd]) - f.sun_lon_lst;
     if (f.prograde == 0.0) ang = -ang;
@@ -612,12 +647,8 @@ PM_HD double local_solar_time(const PMFrame &f, double lon_deg) {
     const int isec = (int)sec;  // floor: sec >= 0
     const int hr = isec / 3600, rem = isec - hr * 3600;
     const int mn = rem / 60, sc = rem - mn * 60;
-    // correctly rounded mn / 60 and sc / 3600 (Markstein: r = RN(1/b), one FMA correction)
-    const double dm = (double)mn, ds = (double)sc;
-    double qm = dm * PM_T(kPixC)[kPixInv60];
-    qm = fma(fma(-60.0, qm, dm), PM_T(kPixC)[kPixInv60], qm);
-    double qs = ds * PM_T(kPixC)[kPixInv3600];
-    qs = fma(fma(-3600.0, qs, ds), PM_T(kPixC)[kPixInv3600], qs);
+    double qm, qs;
+    lst_fractions(mn, sc, qm, qs);
     return ((double)hr + qm) + qs;
 }
 
@@ -848,13 +879,17 @@ constexpr uint64_t kSkyMask = bit(PM_RA) | bit(PM_DEC) | kKmMask | kLimbMask | k
 // becomes a handful of large basic blocks the scheduler can interleave freely.
 // kRingAll = true keeps ring-plane points hidden behind the body
 // (Body.ring_plane_coordinates(only_visible=False), body.py:2577-2615); the backplanes hide them.
-// kSpinSym = true is the path for frames with FrameD::spin_sym (the launchers pick it from the flag):
-// the intercept, the illumination angles and the radial velocity are taken in the body frame at t_ref,
-// where they equal the epoch frame's up to the bound of spin_sym, and only LON / LAT spin the point - or,
-// with FrameD::spin_z, shift its longitude.
-template <bool kSky, uint64_t kFixedMask = 0, bool kRingAll = false, bool kSpinSym = false, class Sink>
+// kFrame (FrameKind, picked by the launchers with frame_kind) != kFrameGeneral is the path for frames with
+// FrameD::spin_sym: the intercept, the illumination angles and the radial velocity are taken in the body
+// frame at t_ref, where they equal the epoch frame's up to the bound of spin_sym, and only LON / LAT spin the
+// point - or, with FrameD::spin_z, shift its longitude.  kFrameSpinZ fixes spin_z and biaxial; both kinds
+// compute the same bits for a frame that has those flags.
+template <bool kSky, uint64_t kFixedMask = 0, bool kRingAll = false, int kFrame = kFrameGeneral, class Sink>
 PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, Sink &out) {
     const PMFrame &f = fs.f;
+    constexpr bool kSpinSym = kFrame != kFrameGeneral;
+    const bool spin_z = kFrame == kFrameSpinZ || fs.spin_z;
+    const bool biaxial = kFrame == kFrameSpinZ || fs.biaxial;
     const double nan = NAN;
     const uint64_t mask = kFixedMask ? kFixedMask : (kSky ? mask_in : (mask_in & ~kSkyMask));
     if (mask & bit(PM_PIXEL_X)) out.put(PM_PIXEL_X, x);  // BodyXY.get_x_img / get_y_img (body_xy.py:3494-3531)
@@ -906,7 +941,7 @@ PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, S
                 // FrameD::spin_z: the spin about z keeps rho and z and turns the longitude by -omega_z dt
                 // (back into atan2's [-pi, pi]); otherwise the point is spun to its epoch
                 double turn = 0.0;
-                if (fs.spin_z)
+                if (spin_z)
                     turn = f.omega[2] * it.dt;
                 else
                     p = spin_fwd(fs, make_rot(fs, it.dt), p);
@@ -922,7 +957,7 @@ PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, S
                 if (l < 0.0) l += kTwoPi;
                 const double v_lon = l * kDpr;
                 double lat, alt;
-                if (fs.biaxial) {
+                if (biaxial) {
                     lat = fast_atan2_xpos(p.z * fs.inv_omf2, rho);
                 } else {
                     geodetic_general(fs, rho, p.z, lat, alt);
@@ -992,10 +1027,10 @@ PM_HD void image_pixel(const FrameD &fs, double x, double y, uint64_t mask_in, S
 // fractional pixel, or one outside the image.  A non-finite x or y never reaches image_pixel -
 // a NaN ray would drive sincpt's light-time iteration, which runs until the epoch stops
 // changing - so it writes NaN to every plane, with PIXEL-X / PIXEL-Y echoing the input.
-template <bool kSky, bool kRingAll, bool kSpinSym = false, class Sink>
+template <bool kSky, bool kRingAll, int kFrame = kFrameGeneral, class Sink>
 PM_HD void image_point(const FrameD &fs, double x, double y, uint64_t mask_in, Sink &out) {
     if (fabs(x) < INFINITY && fabs(y) < INFINITY) {
-        image_pixel<kSky, 0, kRingAll, kSpinSym>(fs, x, y, mask_in, out);
+        image_pixel<kSky, 0, kRingAll, kFrame>(fs, x, y, mask_in, out);
         return;
     }
 #pragma unroll 1
