@@ -138,16 +138,9 @@ static int grouped_layout(int n_planes, int ny, int nx, int n_maps, int planes_p
     empty = n_maps == 0 || planes_per_map == 0 || n_cells == 0;  // valid, with null pointers
     if (!empty && (int64_t)(n_maps - 1) * plane_stride + planes_per_map > n_planes) return PM_ERR_BAD_ARG;
     if (!empty && map_stride > INT64_MAX / n_maps) return PM_ERR_BAD_ARG;
-    int ky = mode, kx = mode;
-    if (mode & PM_INTERP_MIXED) {
-        ky = (mode >> 4) & 0xF;
-        kx = mode & 0xF;
-        if ((mode & ~0x1FF) || ky < 1 || ky > 3 || kx < 1 || kx > 3) return PM_ERR_UNSUPPORTED;
-    } else if (mode < PM_INTERP_NEAREST || mode > PM_INTERP_CUBIC) {
-        return PM_ERR_UNSUPPORTED;
-    }
-    if (mode != PM_INTERP_NEAREST && (nx <= kx || ny <= ky)) return PM_ERR_BAD_ARG;
-    return PM_OK;
+    int ky, kx;
+    if (interp_degrees(mode, ky, kx) != PM_OK) return PM_ERR_UNSUPPORTED;
+    return nx <= kx || ny <= ky ? PM_ERR_BAD_ARG : PM_OK;
 }
 
 int pm_gather_grouped(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes, int ny,
@@ -309,15 +302,9 @@ int pm_gather(const double *src, const uint32_t *nanbits, const uint32_t *plane_
         return PM_ERR_BAD_ARG;
     const bool empty = n_cells == 0 || plane_count == 0;  // valid, and the empty arrays carry null pointers
     if (!empty && (!src || !xmap || !ymap || !out)) return PM_ERR_BAD_ARG;
-    int ky = mode, kx = mode;
-    if (mode & PM_INTERP_MIXED) {
-        ky = (mode >> 4) & 0xF;
-        kx = mode & 0xF;
-        if ((mode & ~0x1FF) || ky < 1 || ky > 3 || kx < 1 || kx > 3) return PM_ERR_UNSUPPORTED;
-    } else if (mode < PM_INTERP_NEAREST || mode > PM_INTERP_CUBIC) {
-        return PM_ERR_UNSUPPORTED;
-    }
-    if (mode != PM_INTERP_NEAREST && (nx <= kx || ny <= ky)) return PM_ERR_BAD_ARG;
+    int ky, kx;
+    if (interp_degrees(mode, ky, kx) != PM_OK) return PM_ERR_UNSUPPORTED;
+    if (nx <= kx || ny <= ky) return PM_ERR_BAD_ARG;
     if (empty) return PM_OK;
     if (mode != PM_INTERP_NEAREST && (!nanbits || !plane_bits || (plane_begin & 3))) return PM_ERR_BAD_ARG;
     if (plane_count > 65535 * 128) return PM_ERR_BAD_ARG;
@@ -348,13 +335,8 @@ int pm_spline_prepare(const double *cube, int n_planes, int ny, int nx, int degr
                       uint32_t *nanbits, uint32_t *plane_bits, void *work, void *stream) {
     if (!cube || !coef || !nanbits || !plane_bits || !work || n_planes < 0 || ny <= 0 || nx <= 0)
         return PM_ERR_BAD_ARG;
-    int ky = degree, kx = degree;
-    if (degree & PM_INTERP_MIXED) {
-        ky = (degree >> 4) & 0xF;
-        kx = degree & 0xF;
-        if (degree & ~0x1FF) return PM_ERR_UNSUPPORTED;
-    }
-    if (ky < 1 || ky > 3 || kx < 1 || kx > 3) return PM_ERR_UNSUPPORTED;
+    int ky, kx;
+    if (interp_degrees(degree, ky, kx) != PM_OK || ky == 0) return PM_ERR_UNSUPPORTED;   // nearest needs no spline
     if (nx <= kx || ny <= ky) return PM_ERR_BAD_ARG;
     int sms = sm_count();
     if (sms <= 0) return PM_ERR_NO_DEVICE;

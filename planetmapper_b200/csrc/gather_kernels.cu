@@ -310,7 +310,10 @@ __device__ __forceinline__ double spline_cell_plane(const CellState<KY, KX> &cs,
     return acc;
 }
 
-// One cell per thread, KY x KX footprint (KY = row degree + 1, KX = column degree + 1)
+// One cell per thread, KY x KX footprint (KY = row degree + 1, KX = column degree + 1).
+// CTAs per SM, [row degree - 1][column degree - 1]: linear runs five (48 registers instead of 64), measured faster
+// than four (profiles/r1_summary.md)
+constexpr int kSplineCtas[3][3] = {{5, 3, 3}, {3, 3, 2}, {3, 2, 2}};
 template <int KY, int KX, int kMinBlocks>
 __global__ void __launch_bounds__(kGatherBlock, kMinBlocks)
     gather_spline_kernel(const double *__restrict__ coefq, const uint32_t *__restrict__ nanbits,
@@ -846,6 +849,11 @@ __global__ void __launch_bounds__(kGatherBlock)
                         ymaps + (int64_t)g * map_stride, cell, n_cells, out + (int64_t)g * planes_per_map * n_cells);
 }
 
+// CTAs per SM, [row degree - 1][column degree - 1], of the quad form and the plane-by-plane form: the most at which
+// each instantiation compiles without spills (ptxas -v); the quad form carries the group indexing on top of
+// gather_spline_kernel's state
+constexpr int kGroupedQuadCtas[3][3] = {{4, 3, 2}, {2, 2, 2}, {2, 2, 2}};
+constexpr int kGroupedPlaneCtas[3][3] = {{6, 3, 3}, {3, 3, 2}, {3, 2, 2}};
 template <int KY, int KX, bool kQuads, int kMinBlocks>
 __global__ void __launch_bounds__(kGatherBlock, kMinBlocks)
     gather_grouped_kernel(const double *__restrict__ coefq, const uint32_t *__restrict__ nanbits,
@@ -984,7 +992,13 @@ __global__ void __launch_bounds__(kGatherBlock)
 }
 
 // kQuads: every epoch's planes start on a plane quad (plane_stride a multiple of 4, PG a multiple of 4) and are
-// read a quad per 32-byte load, as gather_grouped_kernel<kQuads = true>; otherwise plane by plane
+// read a quad per 32-byte load, as gather_grouped_kernel<kQuads = true>; otherwise plane by plane.
+// Planes per thread, and CTAs per SM [row degree - 1][column degree - 1] of the quad form and the plane-by-plane form:
+// the per-epoch cell setup is shared by a thread's planes, whose accumulators live in registers for the whole
+// launch; the values are the largest at which each instantiation compiles without spills (ptxas -v)
+constexpr int kCompositePlanes = 4;
+constexpr int kCompositeQuadCtas[3][3] = {{4, 3, 3}, {3, 2, 3}, {3, 2, 2}};
+constexpr int kCompositePlaneCtas[3][3] = {{4, 3, 3}, {3, 3, 3}, {3, 3, 2}};
 template <int KY, int KX, bool kQuads, int PG, bool kMin, int kMinBlocks>
 __global__ void __launch_bounds__(kGatherBlock, kMinBlocks)
     composite_grouped_kernel(const double *__restrict__ coefq, const uint32_t *__restrict__ nanbits,
@@ -1041,6 +1055,26 @@ static bool dense_map(int64_t n_cells, int ny, int nx) {
     return n_cells >= (int64_t)20 * nx * ny && nx < 16384 && ny < 16384;
 }
 
+// Calls f(Footprint<KY, KX>{}) with the compile-time footprint of validated spline degrees ky, kx in 1..3
+template <int KY_, int KX_>
+struct Footprint {
+    static constexpr int KY = KY_, KX = KX_;
+};
+template <class F>
+static void with_footprint(int ky, int kx, F &&f) {
+    switch (ky * 4 + kx) {
+        case 1 * 4 + 1: f(Footprint<2, 2>{}); break;
+        case 1 * 4 + 2: f(Footprint<2, 3>{}); break;
+        case 1 * 4 + 3: f(Footprint<2, 4>{}); break;
+        case 2 * 4 + 1: f(Footprint<3, 2>{}); break;
+        case 2 * 4 + 2: f(Footprint<3, 3>{}); break;
+        case 2 * 4 + 3: f(Footprint<3, 4>{}); break;
+        case 3 * 4 + 1: f(Footprint<4, 2>{}); break;
+        case 3 * 4 + 2: f(Footprint<4, 3>{}); break;
+        default: f(Footprint<4, 4>{}); break;
+    }
+}
+
 cudaError_t launch_gather(const double *src, const uint32_t *nanbits, const uint32_t *plane_bits, int n_planes,
                           int ny, int nx, int plane_begin, int plane_count, const double *xmap, const double *ymap,
                           int64_t n_cells, int64_t cells_per_row, int mode, uint32_t flags, double *out, int sm_count,
@@ -1052,22 +1086,14 @@ cudaError_t launch_gather(const double *src, const uint32_t *nanbits, const uint
     // every CTA of the scalar kernels covers kGatherBlock cells (the DMMA kernel sizes its own grid below)
     dim3 grid((unsigned)((n_cells + kGatherBlock - 1) / kGatherBlock), (unsigned)((plane_count + ppg - 1) / ppg));
     const int n_words = (n_planes + 31) / 32;
-    int ky = mode, kx = mode;  // spline degree along image rows (y) / columns (x)
-    if (mode & PM_INTERP_MIXED) {
-        ky = (mode >> 4) & 0xF;
-        kx = mode & 0xF;
-    }
     if (mode == PM_INTERP_NEAREST) {
         gather_nearest_kernel<<<grid, kGatherBlock, 0, st>>>(src, ny, nx, plane_begin, plane_count, xmap, ymap, n_cells,
                                                              out, ppg);
         count_launches(1);
         return cudaGetLastError();
     }
-    if (ky < 1 || ky > 3 || kx < 1 || kx > 3) return cudaErrorInvalidValue;
-#define PM_SPLINE(KY, KX, MB)                                                                                     \
-    gather_spline_kernel<KY, KX, MB><<<grid, kGatherBlock, 0, st>>>(src, nanbits, plane_bits, n_words, ny, nx,    \
-                                                                    plane_begin, plane_count, xmap, ymap, n_cells, \
-                                                                    flags, out, ppg)
+    int ky, kx;  // spline degree along image rows (y) / columns (x)
+    if (interp_degrees(mode, ky, kx) != PM_OK) return cudaErrorInvalidValue;
     static const int v = tune_int("PM_CUBIC_VARIANT", -1);
     // dense maps (many cells per image pixel share a footprint): warp-tiled DMMA kernel
     const bool dense = dense_map(n_cells, ny, nx);
@@ -1094,19 +1120,13 @@ cudaError_t launch_gather(const double *src, const uint32_t *nanbits, const uint
                                                                 row_len, flags, out - (int64_t)lead * n_cells, g2,
                                                                 lead);
     } else {
-        switch (ky * 4 + kx) {
-            case 1 * 4 + 1: PM_SPLINE(2, 2, 5); break;
-            case 1 * 4 + 2: PM_SPLINE(2, 3, 3); break;
-            case 1 * 4 + 3: PM_SPLINE(2, 4, 3); break;
-            case 2 * 4 + 1: PM_SPLINE(3, 2, 3); break;
-            case 2 * 4 + 2: PM_SPLINE(3, 3, 3); break;
-            case 2 * 4 + 3: PM_SPLINE(3, 4, 2); break;
-            case 3 * 4 + 1: PM_SPLINE(4, 2, 3); break;
-            case 3 * 4 + 2: PM_SPLINE(4, 3, 2); break;
-            default: PM_SPLINE(4, 4, 2); break;
-        }
+        with_footprint(ky, kx, [&](auto fp) {
+            constexpr int KY = decltype(fp)::KY, KX = decltype(fp)::KX;
+            gather_spline_kernel<KY, KX, kSplineCtas[KY - 2][KX - 2]><<<grid, kGatherBlock, 0, st>>>(
+                src, nanbits, plane_bits, n_words, ny, nx, plane_begin, plane_count, xmap, ymap, n_cells, flags, out,
+                ppg);
+        });
     }
-#undef PM_SPLINE
     count_launches(1);
     return cudaGetLastError();
 }
@@ -1126,12 +1146,8 @@ cudaError_t launch_gather_grouped(const double *src, const uint32_t *nanbits, co
         count_launches(1);
         return cudaGetLastError();
     }
-    int ky = mode, kx = mode;
-    if (mode & PM_INTERP_MIXED) {
-        ky = (mode >> 4) & 0xF;
-        kx = mode & 0xF;
-    }
-    if (ky < 1 || ky > 3 || kx < 1 || kx > 3) return cudaErrorInvalidValue;
+    int ky, kx;
+    if (interp_degrees(mode, ky, kx) != PM_OK) return cudaErrorInvalidValue;
     const bool quads = planes_per_map > 1 && plane_stride % 4 == 0;
     if (ky == 3 && kx == 3 && quads && dense_map(n_cells, ny, nx)) {
         // a cube per map on a dense map: pm_gather's own DMMA launch per map, so each group is its result bit
@@ -1146,31 +1162,13 @@ cudaError_t launch_gather_grouped(const double *src, const uint32_t *nanbits, co
         return cudaSuccess;
     }
     const int n_words = (n_planes + 31) / 32;
-    // CTAs per SM (quad form, plane-by-plane form): the most at which each instantiation compiles without spills
-    // (ptxas -v); the quad form carries the group indexing on top of gather_spline_kernel's state
-#define PM_GROUPED(KY, KX, MBQ, MB)                                                                                    \
-    do {                                                                                                            \
-        if (quads)                                                                                                  \
-            gather_grouped_kernel<KY, KX, true, MBQ><<<grid, kGatherBlock, 0, st>>>(                                 \
-                src, nanbits, plane_bits, n_words, ny, nx, planes_per_map, plane_stride, xmaps, ymaps, map_stride,  \
-                n_cells, flags, out, ppg);                                                                          \
-        else                                                                                                        \
-            gather_grouped_kernel<KY, KX, false, MB><<<grid, kGatherBlock, 0, st>>>(                                \
-                src, nanbits, plane_bits, n_words, ny, nx, planes_per_map, plane_stride, xmaps, ymaps, map_stride,  \
-                n_cells, flags, out, ppg);                                                                          \
-    } while (0)
-    switch (ky * 4 + kx) {
-        case 1 * 4 + 1: PM_GROUPED(2, 2, 4, 6); break;
-        case 1 * 4 + 2: PM_GROUPED(2, 3, 3, 3); break;
-        case 1 * 4 + 3: PM_GROUPED(2, 4, 2, 3); break;
-        case 2 * 4 + 1: PM_GROUPED(3, 2, 2, 3); break;
-        case 2 * 4 + 2: PM_GROUPED(3, 3, 2, 3); break;
-        case 2 * 4 + 3: PM_GROUPED(3, 4, 2, 2); break;
-        case 3 * 4 + 1: PM_GROUPED(4, 2, 2, 3); break;
-        case 3 * 4 + 2: PM_GROUPED(4, 3, 2, 2); break;
-        default: PM_GROUPED(4, 4, 2, 2); break;
-    }
-#undef PM_GROUPED
+    with_footprint(ky, kx, [&](auto fp) {
+        constexpr int KY = decltype(fp)::KY, KX = decltype(fp)::KX;
+        const auto kernel = quads ? gather_grouped_kernel<KY, KX, true, kGroupedQuadCtas[KY - 2][KX - 2]>
+                                  : gather_grouped_kernel<KY, KX, false, kGroupedPlaneCtas[KY - 2][KX - 2]>;
+        kernel<<<grid, kGatherBlock, 0, st>>>(src, nanbits, plane_bits, n_words, ny, nx, planes_per_map, plane_stride,
+                                              xmaps, ymaps, map_stride, n_cells, flags, out, ppg);
+    });
     count_launches(1);
     return cudaGetLastError();
 }
@@ -1196,45 +1194,21 @@ cudaError_t launch_composite_grouped(const double *src, const uint32_t *nanbits,
         count_launches(1);
         return cudaGetLastError();
     }
-    int ky = mode, kx = mode;
-    if (mode & PM_INTERP_MIXED) {
-        ky = (mode >> 4) & 0xF;
-        kx = mode & 0xF;
-    }
-    if (ky < 1 || ky > 3 || kx < 1 || kx > 3) return cudaErrorInvalidValue;
+    int ky, kx;
+    if (interp_degrees(mode, ky, kx) != PM_OK) return cudaErrorInvalidValue;
     // the quad layout of gather_grouped_kernel; a cubic cube on a dense map also takes it (no DMMA form here)
     const bool quads = planes_per_map > 1 && plane_stride % 4 == 0;
     const int n_words = (n_planes + 31) / 32;
-    // Planes per thread (quad form, plane-by-plane form) and CTAs per SM: the per-epoch cell setup is shared by a
-    // thread's planes, whose accumulators live in registers for the whole launch; the values are the largest at
-    // which each instantiation compiles without spills (ptxas -v)
-#define PM_COMPOSITE_LAUNCH(KY, KX, Q, PG, MIN, MB)                                                                 \
-    composite_grouped_kernel<KY, KX, Q, PG, MIN, MB><<<grid(PG), kGatherBlock, 0, st>>>(                            \
-        src, nanbits, plane_bits, n_words, ny, nx, n_maps, planes_per_map, plane_stride, n_cells, flags, a)
-#define PM_COMPOSITE(KY, KX, PGQ, MBQ, PG1, MB1)                                                                    \
-    do {                                                                                                            \
-        if (quads && min_e)                                                                                         \
-            PM_COMPOSITE_LAUNCH(KY, KX, true, PGQ, true, MBQ);                                                      \
-        else if (quads)                                                                                             \
-            PM_COMPOSITE_LAUNCH(KY, KX, true, PGQ, false, MBQ);                                                     \
-        else if (min_e)                                                                                             \
-            PM_COMPOSITE_LAUNCH(KY, KX, false, PG1, true, MB1);                                                     \
-        else                                                                                                        \
-            PM_COMPOSITE_LAUNCH(KY, KX, false, PG1, false, MB1);                                                    \
-    } while (0)
-    switch (ky * 4 + kx) {
-        case 1 * 4 + 1: PM_COMPOSITE(2, 2, 4, 4, 4, 4); break;
-        case 1 * 4 + 2: PM_COMPOSITE(2, 3, 4, 3, 4, 3); break;
-        case 1 * 4 + 3: PM_COMPOSITE(2, 4, 4, 3, 4, 3); break;
-        case 2 * 4 + 1: PM_COMPOSITE(3, 2, 4, 3, 4, 3); break;
-        case 2 * 4 + 2: PM_COMPOSITE(3, 3, 4, 2, 4, 3); break;
-        case 2 * 4 + 3: PM_COMPOSITE(3, 4, 4, 3, 4, 3); break;
-        case 3 * 4 + 1: PM_COMPOSITE(4, 2, 4, 3, 4, 3); break;
-        case 3 * 4 + 2: PM_COMPOSITE(4, 3, 4, 2, 4, 3); break;
-        default: PM_COMPOSITE(4, 4, 4, 2, 4, 2); break;
-    }
-#undef PM_COMPOSITE
-#undef PM_COMPOSITE_LAUNCH
+    with_footprint(ky, kx, [&](auto fp) {
+        constexpr int KY = decltype(fp)::KY, KX = decltype(fp)::KX, PG = kCompositePlanes;
+        constexpr int mbq = kCompositeQuadCtas[KY - 2][KX - 2], mb = kCompositePlaneCtas[KY - 2][KX - 2];
+        const auto kernel = quads ? (min_e ? composite_grouped_kernel<KY, KX, true, PG, true, mbq>
+                                           : composite_grouped_kernel<KY, KX, true, PG, false, mbq>)
+                                  : (min_e ? composite_grouped_kernel<KY, KX, false, PG, true, mb>
+                                           : composite_grouped_kernel<KY, KX, false, PG, false, mb>);
+        kernel<<<grid(PG), kGatherBlock, 0, st>>>(src, nanbits, plane_bits, n_words, ny, nx, n_maps, planes_per_map,
+                                                  plane_stride, n_cells, flags, a);
+    });
     count_launches(1);
     return cudaGetLastError();
 }
@@ -1706,6 +1680,8 @@ cudaError_t launch_spline_prepare(const double *cube, int n_planes, int ny, int 
                                   uint32_t *nanbits, uint32_t *plane_bits, void *work, int sm_count,
                                   cudaStream_t st) {
     if (n_planes == 0) return cudaSuccess;
+    int deg_y, deg_x;  // rows (image y) / columns (image x)
+    if (interp_degrees(degree, deg_y, deg_x) != PM_OK) return cudaErrorInvalidValue;
     char *w = static_cast<char *>(work);
     PlaneStats *stats = reinterpret_cast<PlaneStats *>(w);
     w += align256((int64_t)n_planes * sizeof(PlaneStats));
@@ -1745,11 +1721,6 @@ cudaError_t launch_spline_prepare(const double *cube, int n_planes, int ny, int 
     }
     fill_isolated_kernel<<<dim3(rblocks, n_planes), 256, 0, st>>>(cube, ny, nx, stats, median, coef);
     count_launches(4);
-    int deg_y = degree, deg_x = degree;  // rows (image y) / columns (image x)
-    if (degree & PM_INTERP_MIXED) {
-        deg_y = (degree >> 4) & 0xF;
-        deg_x = degree & 0xF;
-    }
     {
         double *lu_x = reinterpret_cast<double *>(w);
         w += align256((int64_t)5 * nx * sizeof(double));

@@ -26,6 +26,18 @@ inline int tune_int(const char *name, int dflt) {
 constexpr int tune_int(const char *, int dflt) { return dflt; }
 #endif
 
+// The spline degrees of an interpolation mode along image rows (ky) and columns (kx): 0, 0 for nearest, 1..3 each
+// for PM_INTERP_LINEAR .. PM_INTERP_CUBIC and PM_INTERP_MIXED_MODE(rows, cols).  PM_OK or PM_ERR_UNSUPPORTED.
+inline int interp_degrees(int mode, int &ky, int &kx) {
+    if (mode & PM_INTERP_MIXED) {
+        ky = (mode >> 4) & 0xF;
+        kx = mode & 0xF;
+        return (mode & ~0x1FF) == 0 && ky >= 1 && ky <= 3 && kx >= 1 && kx <= 3 ? PM_OK : PM_ERR_UNSUPPORTED;
+    }
+    ky = kx = mode;
+    return mode >= PM_INTERP_NEAREST && mode <= PM_INTERP_CUBIC ? PM_OK : PM_ERR_UNSUPPORTED;
+}
+
 cudaError_t launch_backplanes_img(const PMFrame *frames, int n_frames, int nx, int ny, uint64_t mask,
                                   double *out, int sm_count, cudaStream_t st);
 cudaError_t launch_backplanes_img_host(const PMFrame *frame_host, int nx, int ny, uint64_t mask, double *out,

@@ -223,12 +223,13 @@ def map_series(frames: np.ndarray, imgs, nx: int, ny: int, lons, lats, *, interp
     """``BodyXY(...).map_img(img_f, ...)`` for every frame f of a series (body_xy.py:1414-1631 once per
     epoch in the reference): frame f's image is mapped onto the lon / lat grid with frame f's own
     disc geometry.  Per batch of frames: ONE launch for all x / y maps (``pm_backplanes_map_batch``),
-    the NaN repair of the batch's images (linear), ONE paired gather.
+    the NaN repair of the batch's images (linear), ONE grouped gather of one image per map.
 
-    ``imgs``: (n_frames, ny, nx) array or CUDA tensor; ``lons`` / ``lats``: the map grid (degrees,
-    e.g. from ``generate_map_coordinates``); ``interpolation``: 'nearest' or 'linear'.  Returns a CUDA
-    tensor (n_frames,) + grid shape (``out`` if given).  :func:`iter_mapped_series` maps with every
-    interpolating spline degree, and a cube per epoch.
+    ``imgs``: (n_frames, ny, nx) array or tensor; a stack that is not a float64 CUDA tensor is uploaded and
+    converted one batch at a time.  ``lons`` / ``lats``: the map grid (degrees, e.g. from
+    ``generate_map_coordinates``); ``interpolation``: 'nearest' or 'linear'.  Returns a CUDA tensor
+    (n_frames,) + grid shape (``out`` if given).  :func:`iter_mapped_series` maps with every interpolating
+    spline degree, and a cube per epoch.
     """
     from . import _lib as L
 
@@ -236,23 +237,18 @@ def map_series(frames: np.ndarray, imgs, nx: int, ny: int, lons, lats, *, interp
     mode = {'nearest': L.INTERP_NEAREST, 'linear': L.INTERP_LINEAR, 1: L.INTERP_LINEAR}.get(interpolation)
     if mode is None:
         raise NotImplementedError("map_series: interpolation must be 'nearest' or 'linear'")
-    fd = L.to_device(np.ascontiguousarray(frames, dtype=np.float64))
+    frames = np.ascontiguousarray(frames, dtype=np.float64)
     if not isinstance(imgs, torch.Tensor):
-        imgs = L.to_device(imgs)
+        imgs = np.asarray(imgs)
     if tuple(imgs.shape) != (len(frames), ny, nx):
         raise ValueError(f'imgs must have shape ({len(frames)}, {ny}, {nx})')
-    lod = L.to_device(np.asarray(lons, dtype=np.float64) % 360)
-    lad = L.to_device(lats)
+    lons, lats = np.asarray(lons, dtype=np.float64), np.asarray(lats, dtype=np.float64)
     if out is None:
-        out = torch.empty((len(frames),) + tuple(lod.shape), dtype=torch.float64, device=fd.device)
-    xy_mask = L.mask_from_names(['PIXEL-X', 'PIXEL-Y'])
-    xy = torch.empty((min(batch, len(frames)), 2) + tuple(lod.shape), dtype=torch.float64, device=fd.device)
-    for first in range(0, len(frames), batch):
-        n = min(batch, len(frames) - first)
-        L.backplanes_map_batch(fd[first:first + n], lod, lad, xy_mask, out=xy[:n])
-        cube = imgs[first:first + n].contiguous()
-        src = cube if mode == L.INTERP_NEAREST else L.spline_prepare(cube, 1)
-        L.gather_paired(src, xy[:n, 0], xy[:n, 1], mode, propagate_nan=propagate_nan, out=out[first:first + n])
+        out = torch.empty((len(frames),) + lons.shape, dtype=torch.float64, device='cuda')
+    for first, n, xy, src, stride in _prepared_batches(frames, imgs, nx, ny, lons, lats, mode, batch,
+                                                       L.mask_from_names(['PIXEL-X', 'PIXEL-Y']), 1):
+        L.gather_grouped(src, xy[:, 0], xy[:, 1], mode, 1, stride, propagate_nan=propagate_nan,
+                         out=out[first:first + n])
     return out
 
 

@@ -249,7 +249,7 @@ def test_series_batches_equal_one_bodyxy_per_epoch():
 
 
 def test_map_series_equals_map_img_per_epoch():
-    """series.map_series (batched x / y maps + paired gather) gives, frame by frame, exactly what
+    """series.map_series (batched x / y maps + grouped gather) gives, frame by frame, exactly what
     BodyXY(...).map_img(img_f) returns for that epoch (body_xy.py:1414-1631)."""
     import planetmapper_b200 as pm
     from planetmapper_b200 import _lib as L
@@ -284,6 +284,15 @@ def test_map_series_equals_map_img_per_epoch():
             assert np.isfinite(got[0]).sum() > 100 and not np.isfinite(got[3]).any()
             if interp == 'nearest':
                 assert launches == 2 * 2   # two batches x (maps + gather), not two launches per frame
+    # a stack that is not a float64 CUDA tensor is converted batch by batch: float32 on the device maps as its
+    # float64 copy, a host tensor as the numpy stack
+    import torch
+    imgs32 = torch.tensor(imgs, dtype=torch.float32, device='cuda')
+    for stack, same in ((imgs32, imgs32.double()), (torch.from_numpy(imgs), imgs)):
+        for interp in ('nearest', 'linear'):
+            got = S.map_series(frames, stack, nx, ny, lons, lats, interpolation=interp, batch=4).cpu().numpy()
+            want = S.map_series(frames, same, nx, ny, lons, lats, interpolation=interp, batch=4).cpu().numpy()
+            assert np.isfinite(got).sum() > 100 and np.array_equal(got, want, equal_nan=True), (stack.dtype, interp)
     with pytest.raises(NotImplementedError):
         S.map_series(frames, imgs, nx, ny, lons, lats, interpolation='cubic')
     # the batched map kernel alone: every plane of every frame equals the single-frame call

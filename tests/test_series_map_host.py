@@ -1,6 +1,6 @@
 """
-Host side of the mapped time series (no GPU): the argument checks of pm_gather_grouped and the argument rules of
-series.iter_mapped_series, both before any device work.
+Host side of the mapped time series (no GPU): the argument checks of pm_gather_grouped, the interpolation modes the
+gather entry points accept, and the argument rules of series.iter_mapped_series, all before any device work.
 """
 import ctypes
 
@@ -48,6 +48,25 @@ def test_grouped_gather_validates_arguments_before_device_work():
     assert g(None, None, None, 0, 5, 6, 0, 4, 4, None, None, 0, 0, L.INTERP_CUBIC, 0, None, None) == 0
     assert g(None, None, None, 12, 5, 6, 3, 0, 4, None, None, 10, 10, L.INTERP_LINEAR, 0, None, None) == 0
     assert g(None, None, None, 12, 5, 6, 3, 4, 4, None, None, 10, 0, L.INTERP_NEAREST, 0, None, None) == 0
+
+
+def test_gather_entry_points_agree_on_every_interpolation_mode():
+    """pm_gather, pm_gather_grouped, pm_composite_grouped and pm_spline_prepare decode the interpolation mode alike:
+    on a 1 x 1 image with no map cells a spline mode is refused for the image size, nearest is empty work (no spline
+    to prepare) and every other code is unsupported; none of these calls reaches the device."""
+    lib = L.load_library()
+    buf = np.zeros(64)
+    p = buf.ctypes.data_as(ctypes.c_void_p)
+    splines = {L.INTERP_LINEAR, L.INTERP_QUADRATIC, L.INTERP_CUBIC}
+    splines |= {L.INTERP_MIXED | (ky << 4) | kx for ky in (1, 2, 3) for kx in (1, 2, 3)}
+    for mode in range(-2, 0x400):
+        want = BAD if mode in splines else 0 if mode == L.INTERP_NEAREST else UNSUPPORTED
+        assert lib.pm_gather(p, p, p, 1, 1, 1, 0, 1, p, p, 0, 0, mode, 0, p, None) == want, mode
+        assert lib.pm_gather_grouped(p, p, p, 1, 1, 1, 1, 1, 1, p, p, 0, 0, mode, 0, p, None) == want, mode
+        assert lib.pm_composite_grouped(p, p, p, 1, 1, 1, 1, 1, 1, p, 2, 0, 0, mode, 0, 0, float('inf'), 0, 1, 1, p,
+                                        None, p, None) == want, mode
+        want = UNSUPPORTED if mode == L.INTERP_NEAREST else want
+        assert lib.pm_spline_prepare(p, 1, 1, 1, mode, p, p, p, p, None) == want, mode
 
 
 def _args(n=3, nl=None, ny=8, nx=9):
